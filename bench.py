@@ -5,6 +5,7 @@ allqueries.fasta, BLOSUM62 -11/-1, database resident, `runpeakbenchmark.sh:26-54
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference ...                       (CPU arm: the oracle port on the host cores)
+  python bench.py ... --dump-outputs DIR                     (also writes the last timed step's top-k lists as .npy)
 
 A *step* = one pass of the hot path over the whole query batch: all 20 queries scanned against the resident database
 (20 sw4_scan calls through the C ABI, each: query H2D -> profile -> score kernels -> top-k -> k results D2H).
@@ -347,6 +348,19 @@ def ref_gpu_leg(local_rank, ours_e2e_gcups, ours_value_gcups):
     return out
 
 
+def dump_outputs(out_dir, merged):
+    """What a caller of the timed path receives, from its last step: the merged top-k (score, global id) lists of the
+    20 queries, as float64 (n_queries, TOP_K) arrays topk_scores.npy and topk_ids.npy (NaN pads a shorter list). The
+    database and the queries are fixed, so two builds run with the same arguments can be compared array for array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, col in (("topk_scores", 0), ("topk_ids", 1)):
+        a = np.full((len(merged), TOP_K), np.nan)
+        for qi, pairs in enumerate(merged):
+            a[qi, :len(pairs)] = [p[col] for p in pairs]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -356,7 +370,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c4", action="store_true", help="skip the C4 strong-scaling leg")
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip timing the reference's own GPU binary")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -403,7 +420,7 @@ def main():
 
     def one_step():
         """One pass of the hot path over the query batch: the 20 queries through sw4_scan_many (host letters in, top-k
-        out). Returns (device-timed seconds of the call, launches, merged top-k of the last query)."""
+        out). Returns (device-timed seconds of the call, launches, merged top-k list of every query)."""
         if single:
             dev_s, launches, results = 0.0, 0, []
             for q in letters:
@@ -415,9 +432,7 @@ def main():
             results, total = eng.scanMany(letters)
             dev_s, launches = total.seconds, total.kernelLaunches
         # the only exchange step: k (score, id) pairs per rank and query (NCCL all_gather), merged on every rank
-        merged = None
-        for r in results:
-            merged = gather_topk(r.scores, r.referenceIds, TOP_K, device=dev)
+        merged = [gather_topk(r.scores, r.referenceIds, TOP_K, device=dev) for r in results]
         return dev_s, launches, merged
 
     def kernel_step():
@@ -443,6 +458,8 @@ def main():
         launches += l
     barrier()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, merged)
     ker_s = 0.0
     for _ in range(args.steps):
         ker_s += kernel_step()
@@ -491,7 +508,7 @@ def main():
                                  "the NCCL gather of the per-rank top-k",
                        "l2_note": "each scan streams 256 MB of database per GPU (> 126 MB L2) and scans alternate 20 different "
                                   "query profiles, so no timed iteration re-reads L2-resident inputs",
-                       "db_upload_s": upload_s, "top1": merged[0] if merged else None},
+                       "db_upload_s": upload_s, "top1": merged[-1][0] if merged and merged[-1] else None},
             "clocks": clocks,
             "e2e": {"value": e2e, "unit": "GCUPS", "h2d_bytes_per_step": total_q + 441 * len(queries),
                     "d2h_bytes_per_step": len(queries) * (2 * TOP_K * 4 + 32)},

@@ -1,6 +1,7 @@
 """Drop-in CLIs. CPU: our makedb reproduces the reference makedb's files byte for byte (golden fixtures written by the
-reference binary). GPU: our `align` and the reference's own `align` (built for sm_100a from /root/reference into
-oracle/_ref/, --dpx and default half2 kernels) print identical TSV results on the same database and queries."""
+reference binary). GPU: our `align` prints the same result files as the reference's own `align` (--dpx and default
+half2 kernels) on the same database and queries: the stored results under tests/golden/align/, and live when the
+reference has been built into oracle/_ref/ (oracle/Makefile)."""
 import os
 import subprocess
 
@@ -54,22 +55,40 @@ def _run_align(binary, args, cwd):
     return r.stdout
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("mat,extra", [("blosum62", []), ("blosum45", []), ("blosum80", ["--gop", "-14", "--gex", "-2"])])
-def test_align_matches_reference_align(tmp_path, mat, extra):
-    if not os.path.exists(REF_ALIGN):
-        pytest.skip("oracle/_ref/align_gapfix not built (needs /root/reference at build time)")
+ALIGN_CASES = [("blosum62", []), ("blosum45", []), ("blosum80", ["--gop", "-14", "--gex", "-2"])]
+
+
+def align_case_inputs(workdir, mat, extra):
+    """Writes the database and queries of test_align_matches_reference_align into `workdir` (with the makedb files of
+    the database under the prefix `db`); returns the `align` arguments the test runs both programs with."""
     _build_cli()
     recs, queries = synth.config_c1(seed=1, n=3000)
     rng = np.random.default_rng(5)
     recs += [(f"long{i}", dbformat.decode(synth.random_residues(rng, int(n)))) for i, n in enumerate([1300, 2000, 4100, 8100, 9000])]
-    dbformat.write_fasta(str(tmp_path / "db.fa"), recs)
-    dbformat.write_fasta(str(tmp_path / "q.fa"), queries[:6] + [queries[19]])
-    subprocess.run([MAKEDB, str(tmp_path / "db.fa"), str(tmp_path / "db")], check=True, stdout=subprocess.DEVNULL)
-    common = ["--query", "q.fa", "--db", "db", "--top", "25", "--tsv", "--mat", mat, "--uploadFull", "--prefetchDBFile"] + extra
+    dbformat.write_fasta(os.path.join(workdir, "db.fa"), recs)
+    dbformat.write_fasta(os.path.join(workdir, "q.fa"), queries[:6] + [queries[19]])
+    subprocess.run([MAKEDB, os.path.join(workdir, "db.fa"), os.path.join(workdir, "db")], check=True, stdout=subprocess.DEVNULL)
+    return ["--query", "q.fa", "--db", "db", "--top", "25", "--tsv", "--mat", mat, "--uploadFull", "--prefetchDBFile"] + extra
+
+
+def pseudodb_case_inputs(workdir):
+    """Writes the queries of test_align_plain_output_and_pseudodb into `workdir`; returns the common `align` arguments."""
+    _build_cli()
+    dbformat.write_fasta(os.path.join(workdir, "q.fa"), synth.load_queries()[:2])
+    return ["--query", "q.fa", "--pseudodb", "5000", "256", "--top", "3"]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("mat,extra", ALIGN_CASES)
+def test_align_matches_reference_align(tmp_path, golden_dir, mat, extra):
+    common = align_case_inputs(str(tmp_path), mat, extra)
     _run_align(ALIGN, common + ["--dpx", "--of", "ours.tsv"], str(tmp_path))
     ours = open(tmp_path / "ours.tsv").read()
     assert ours.count("\n") == 1 + 7 * 25
+    with open(os.path.join(golden_dir, "align", f"{mat}.tsv")) as f:
+        assert ours == f.read()
+    if not os.path.exists(REF_ALIGN):
+        return
     for tag, flags in (("dpx", ["--dpx"]), ("half2", [])):
         _run_align(REF_ALIGN, common + flags + ["--of", f"ref_{tag}.tsv"], str(tmp_path))
         ref = open(tmp_path / f"ref_{tag}.tsv").read()
@@ -77,17 +96,18 @@ def test_align_matches_reference_align(tmp_path, mat, extra):
 
 
 @pytest.mark.gpu
-def test_align_plain_output_and_pseudodb(tmp_path):
-    _build_cli()
-    dbformat.write_fasta(str(tmp_path / "q.fa"), synth.load_queries()[:2])
-    out = _run_align(ALIGN, ["--query", "q.fa", "--pseudodb", "5000", "256", "--top", "3", "--verbose", "--of", "res.txt"], str(tmp_path))
+def test_align_plain_output_and_pseudodb(tmp_path, golden_dir):
+    common = pseudodb_case_inputs(str(tmp_path))
+    out = _run_align(ALIGN, common + ["--verbose", "--of", "res.txt"], str(tmp_path))
     assert "Total time:" in out and "GCUPS" in out
     res = open(tmp_path / "res.txt").read().splitlines()
     assert res[0].startswith("Query 0, header") and ", num overflows 0" in res[0]
     assert res[1] == "Result 0. Score: 25. Length: 256. Header H. referenceId 0"
     assert res[3] == "Result 2. Score: 25. Length: 256. Header H. referenceId 2"
+    with open(os.path.join(golden_dir, "align", "pseudodb.txt")) as f:
+        assert open(tmp_path / "res.txt").read() == f.read()
     if os.path.exists(REF_ALIGN):
-        _run_align(REF_ALIGN, ["--query", "q.fa", "--pseudodb", "5000", "256", "--top", "3", "--dpx", "--uploadFull", "--of", "ref.txt"], str(tmp_path))
+        _run_align(REF_ALIGN, common + ["--dpx", "--uploadFull", "--of", "ref.txt"], str(tmp_path))
         assert open(tmp_path / "ref.txt").read() == open(tmp_path / "res.txt").read()
 
 

@@ -130,20 +130,30 @@ def test_oracle_properties(oracle):
     assert oracle.score(62, q, np.zeros(0, np.uint8), -11, -1) == 0
 
 
-def test_oracle_scan_matches_reference_cpu_routine_live(oracle):
-    """When oracle/_ref/libref_harness.so is present (built from /root/reference by oracle/Makefile; it travels to the GPU
-    box), the oracle's scan must equal the reference's own scalar CPU Gotoh on a fresh random database, subject by
-    subject (the committed fixtures in tests/golden/ref_cpu_gotoh.json pin the same routine on fixed inputs)."""
-    import os
-    import bench
-    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libref_harness.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/libref_harness.so not built here")
-    ref = bench._ReferenceCpuScan(path)
+def live_scan_cases():
+    """The random database and (query, gop, gex) cases of test_oracle_scan_matches_reference_cpu_routine_live."""
     rng = np.random.default_rng(123)
     seqs = [synth.random_residues(rng, int(n)) for n in rng.integers(1, 900, 1500)]
     seqs += [np.full(40, 20, np.uint8), synth.random_residues(rng, 2500)]
     db = dbformat.from_sequences(seqs)
-    for ql, (gop, gex) in zip((1, 37, 400), ((-11, -1), (-5, -3), (-11, -1))):
-        q = synth.random_residues(rng, ql)
-        assert (ref.scan(62, q, db, gop, gex) == oracle.scan(62, q, db, gop, gex)).all()
+    cases = [(synth.random_residues(rng, ql), gop, gex) for ql, (gop, gex) in zip((1, 37, 400), ((-11, -1), (-5, -3), (-11, -1)))]
+    return db, cases
+
+
+def test_oracle_scan_matches_reference_cpu_routine_live(oracle, golden_dir):
+    """The oracle's scan equals the reference's own scalar CPU Gotoh on a random database, subject by subject: against
+    the stored scores of tests/golden/ref_cpu_scan_live.json, and live when oracle/_ref/libref_harness.so has been built
+    from the reference sources (oracle/Makefile). tests/golden/ref_cpu_gotoh.json pins the same routine on other inputs."""
+    import bench
+    with open(os.path.join(golden_dir, "ref_cpu_scan_live.json")) as f:
+        stored = json.load(f)["cases"]
+    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libref_harness.so")
+    ref = bench._ReferenceCpuScan(path) if os.path.exists(path) else None
+    db, cases = live_scan_cases()
+    assert len(stored) == len(cases)
+    for (q, gop, gex), s in zip(cases, stored):
+        got = oracle.scan(62, q, db, gop, gex)
+        assert [len(q), gop, gex] == [s["query_length"], s["gop"], s["gex"]]
+        assert got.tolist() == s["scores"]
+        if ref is not None:
+            assert (ref.scan(62, q, db, gop, gex) == got).all()
