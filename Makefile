@@ -13,7 +13,7 @@ all: lib cli
 
 # one object per kernel family so that they build in parallel (make -j) and independently of the host engine
 # (the two-row kernel additionally once per gap-score set whose values are compiled in as immediates, -DSW4_GAPS=n)
-UNITS    := engine launch_s16 launch_s16_g1 launch_s16_g2 launch_s16_g3 launch_s16_multi launch_s16_multi_g1 launch_s16_multi_g2 launch_s16_multi_g3 launch_s16_wide launch_long
+UNITS    := engine launch_s16 launch_s16_g1 launch_s16_g2 launch_s16_g3 launch_s16_multi launch_s16_multi_g1 launch_s16_multi_g2 launch_s16_multi_g3 launch_s16_wide launch_long launch_coords
 OBJS     := $(patsubst %,build/%.o,$(UNITS))
 
 lib: $(LIB)

@@ -250,6 +250,25 @@ class CudaSW4:
             out.append(ScanResult(scores[i, :c].tolist(), ids[i, :c].tolist(), _stats(per[i])))
         return out, _stats(total)
 
+    def alignmentCoordinates(self, query, ids, stats: BenchmarkStats | None = None) -> np.ndarray:
+        """Where each hit aligns: for every database id in `ids`, one row (score, query_begin, query_end,
+        reference_begin, reference_end) of an int32 array of shape (len(ids), 5). Positions are 0-based and inclusive,
+        -1 when the score is 0; the end is the first cell holding the maximum, the begin that of the shortest optimal
+        alignment ending there (include/sw4b200.h). `stats`, when given, receives the call's device-timed figures."""
+        q = query.encode() if isinstance(query, str) else bytes(query)
+        idv = np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1))
+        if len(idv) and (idv.min() < -2**31 or idv.max() >= 2**31):
+            raise SW4Error(-1, "database id out of range")
+        idv = idv.astype(np.int32)
+        out = np.empty((max(len(idv), 1), 5), dtype=np.int32)
+        st = _lib.Stats()
+        self._check(self._lib.sw4_alignment_coordinates(self._h, q, len(q), idv.ctypes.data, len(idv), out.ctypes.data,
+                                                        ctypes.byref(st)))
+        if stats is not None:
+            for k, v in vars(_stats(st)).items():
+                setattr(stats, k, v)
+        return out[:len(idv)].copy()
+
     def lastScanAllScores(self):
         """(scores, global ids) of every subject this handle scanned in the last scan() (parity helper)."""
         info = self.dbInfo()

@@ -13,7 +13,7 @@ EXPORTS = [
     "sw4_set_database_shard_memory", "sw4_set_pseudo_database", "sw4_set_pseudo_database_lengths", "sw4_upload_database", "sw4_scan", "sw4_scan_many",
     "sw4_last_scan_all_scores", "sw4_reference_header",
     "sw4_reference_length", "sw4_reference_sequence", "sw4_total_timer_start", "sw4_total_timer_stop",
-    "sw4_get_db_info", "sw4_version",
+    "sw4_get_db_info", "sw4_version", "sw4_alignment_coordinates",
 ]
 
 
@@ -25,6 +25,11 @@ class MemConfig(ctypes.Structure):
 class Stats(ctypes.Structure):
     _fields_ = [("num_overflows", ctypes.c_int32), ("seconds", ctypes.c_double), ("gcups", ctypes.c_double),
                 ("kernel_seconds", ctypes.c_double), ("cells", ctypes.c_double), ("kernel_launches", ctypes.c_int32)]
+
+
+class Alignment(ctypes.Structure):
+    _fields_ = [("score", ctypes.c_int32), ("query_begin", ctypes.c_int32), ("query_end", ctypes.c_int32),
+                ("reference_begin", ctypes.c_int32), ("reference_end", ctypes.c_int32)]
 
 
 class DbInfo(ctypes.Structure):
@@ -66,6 +71,8 @@ def load() -> ctypes.CDLL:
                              ctypes.POINTER(Stats)]
     lib.sw4_scan_many.argtypes = [vp, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(ctypes.c_int32), ctypes.c_int32, vp, vp, vp,
                                   ctypes.POINTER(Stats), ctypes.POINTER(Stats)]
+    lib.sw4_alignment_coordinates.argtypes = [vp, ctypes.c_char_p, ctypes.c_int32, vp, ctypes.c_int32, vp,
+                                              ctypes.POINTER(Stats)]
     lib.sw4_last_scan_all_scores.argtypes = [vp, vp, vp, cs, ctypes.POINTER(cs)]
     lib.sw4_reference_header.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(vp), ctypes.POINTER(cs)]
     lib.sw4_reference_length.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32)]

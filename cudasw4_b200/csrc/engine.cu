@@ -363,6 +363,46 @@ static inline int s16WidePeriod(int qlen, int G) { return std::max(32, (qlen + G
 
 struct QueryRef { const char* letters; int length; };
 
+// Everything sw4_alignment_coordinates owns on the handle's first GPU: it shares nothing with the scan (slots, contexts,
+// results), so a scan after the call returns what it would have returned without it.
+struct CoordState {
+    int device = 0;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t evStart = nullptr, evStop = nullptr;
+    DevBuf<char> dQueryLetters;
+    DevBuf<uint8_t> dQueryCodes, dSubjects;
+    DevBuf<int8_t> dMatrix;
+    DevBuf<CoordGroup> dGroups;
+    DevBuf<CoordItem> dItems;
+    DevBuf<int2> dBorder;
+    DevBuf<int4> dEnds;
+    DevBuf<int32_t> dOut;  // [item][5] + error count
+    PinnedBuf<char> hQuery;
+    PinnedBuf<uint8_t> hSubjects;
+    PinnedBuf<CoordGroup> hGroups;
+    PinnedBuf<CoordItem> hItems;
+    PinnedBuf<int32_t> hOut;
+
+    void create(int dev) {
+        device = dev;
+        SW4_CUDA(cudaSetDevice(device));
+        SW4_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+        SW4_CUDA(cudaEventCreate(&evStart));
+        SW4_CUDA(cudaEventCreate(&evStop));
+        dMatrix.alloc(441);
+    }
+    ~CoordState() {
+        cudaSetDevice(device);
+        if (evStart) cudaEventDestroy(evStart);
+        if (evStop) cudaEventDestroy(evStop);
+        if (stream) cudaStreamDestroy(stream);
+    }
+};
+
+// A pair runs on a CTA of up to 16 warps (one per 512-column tile) when it has this many cells and more than one tile;
+// below that one warp per pair, 16 pairs per CTA. One warp needs about 0.3 s for 35 k x 35 k (DESIGN.md 3.2).
+constexpr long long kCoordCtaMinCells = 1ll << 24;
+
 struct Engine {
     std::vector<int> deviceIds;
     int numTop = 10;
@@ -385,6 +425,7 @@ struct Engine {
     int shardRank = 0, shardWorld = 1;
     std::unique_ptr<HostDB> db;
     std::vector<std::unique_ptr<Shard>> shards;
+    std::unique_ptr<CoordState> coord;  // created by the first sw4_alignment_coordinates call
     int8_t matrix[441];
     int maxMatrixEntry = 11;
     std::string lastError;
@@ -1269,6 +1310,146 @@ struct Engine {
         QueryRef q{query, qlen};
         scanMany(&q, 1, outScores, outIds, outCount, stats, nullptr);
     }
+
+    // ---- alignment coordinates: score, end and begin of one optimal local alignment per (query, id) pair ----
+    // Subjects come from the host copy (any database mode, before or after the upload) and go through pinned staging to
+    // the handle's first GPU. Pass 1 leaves the ends on the device for pass 2; the host waits once per chunk of pairs
+    // whose scratch (gathered subjects + border columns) fits max_temp_bytes.
+    void alignmentCoordinates(const char* query, int qlen, const int32_t* ids, int n, sw4_alignment* out, sw4_stats* stats) {
+        if (!db) fail(SW4_ERR_INVALID, "no database set");
+        if (n < 0) fail(SW4_ERR_INVALID, "num_ids must be >= 0 (got %d)", n);
+        if (n > 0 && (!ids || !out)) fail(SW4_ERR_INVALID, "null id or output array");
+        if (qlen < 0 || (qlen > 0 && !query)) fail(SW4_ERR_INVALID, "invalid query");
+        if (qlen > (1 << 24)) fail(SW4_ERR_INVALID, "query too long (%d residues, at most 2^24)", qlen);
+        checkGaps();
+        std::vector<size_t> local((size_t)n);
+        for (int i = 0; i < n; i++) {
+            const int32_t id = ids[i];
+            if (id < 0 || (size_t)id >= db->nGlobal)
+                fail(SW4_ERR_INVALID, "database id %d out of range (the database has %zu sequences)", id, db->nGlobal);
+            local[i] = db->localIndex(id);
+            if (local[i] >= db->n) fail(SW4_ERR_INVALID, "database id %d is not held by this handle (pre-sharded database)", id);
+            const long long bound = (long long)maxMatrixEntry * std::min(qlen, db->lengths[local[i]]);
+            if (topk_shift_for(bound) < 0)
+                fail(SW4_ERR_INVALID, "the score of the query against id %d may reach %lld; scores are exact below 2^24", id, bound);
+        }
+        if (stats) memset(stats, 0, sizeof(*stats));
+        if (n == 0) return;
+        if (!coord) {
+            auto c = std::make_unique<CoordState>();
+            c->create(deviceIds[0]);
+            coord = std::move(c);
+        }
+        CoordState& cs = *coord;
+        SW4_CUDA(cudaSetDevice(cs.device));
+        cudaStream_t st = cs.stream;
+        auto lengthOf = [&](int i) { return (int)db->lengths[local[i]]; };
+        auto tilesOf = [](int len) { return (len + kCoordTileCols - 1) / kCoordTileCols; };
+        auto warpsOf = [&](int len) {
+            const int tiles = tilesOf(len);
+            return (tiles > 1 && (long long)qlen * len >= kCoordCtaMinCells) ? std::min(tiles, kCoordWarps) : 1;
+        };
+        const size_t borderStride = alignUp((size_t)std::max(qlen, 1), 32);
+        auto scratchOf = [&](int len) {
+            size_t b = alignUp((size_t)len, 16);
+            if (tilesOf(len) > 1) b += (size_t)warpsOf(len) * borderStride * sizeof(int2);
+            return b;
+        };
+        // CTA-form pairs first, then the one-warp pairs; longest first within each form
+        std::vector<int> order((size_t)n);
+        for (int i = 0; i < n; i++) order[i] = i;
+        std::stable_sort(order.begin(), order.end(), [&](int a, int b) {
+            const int la = lengthOf(a), lb = lengthOf(b);
+            const bool ca = warpsOf(la) > 1, cb = warpsOf(lb) > 1;
+            if (ca != cb) return ca;
+            return la > lb;
+        });
+
+        int launches = 0;
+        double cells = 0;
+        SW4_CUDA(cudaEventRecord(cs.evStart, st));
+        const int qpad = (qlen + 3) / 4 * 4;
+        cs.hQuery.ensure((size_t)std::max(qlen, 1));
+        if (qlen) memcpy(cs.hQuery.p, query, (size_t)qlen);
+        if ((size_t)qpad + 16 > cs.dQueryCodes.n) { cs.dQueryLetters.alloc((size_t)qpad + 16); cs.dQueryCodes.alloc((size_t)qpad + 16); }
+        if (qlen) SW4_CUDA(cudaMemcpyAsync(cs.dQueryLetters.p, cs.hQuery.p, (size_t)qlen, cudaMemcpyHostToDevice, st));
+        SW4_CUDA(cudaMemcpyAsync(cs.dMatrix.p, matrix, 441, cudaMemcpyHostToDevice, st));
+        if (qpad > 0) {
+            convert_query_kernel<<<(qpad + 255) / 256, 256, 0, st>>>(cs.dQueryLetters.p, cs.dQueryCodes.p, qlen, qpad);
+            SW4_CUDA(cudaGetLastError());
+            launches++;
+        }
+        const size_t budget = mem.max_temp_bytes;
+        for (int pos = 0; pos < n;) {
+            int end = pos;
+            size_t bytes = 0;
+            while (end < n && bytes + scratchOf(lengthOf(order[end])) <= budget) bytes += scratchOf(lengthOf(order[end++]));
+            if (end == pos)
+                fail(SW4_ERR_NOMEM, "max_temp_bytes (%zu bytes) cannot hold the scratch of one pair (%d x %d residues: %zu bytes)", budget,
+                     qlen, lengthOf(order[pos]), scratchOf(lengthOf(order[pos])));
+            const int m = end - pos;
+            cs.hItems.ensure((size_t)m);
+            cs.hGroups.ensure((size_t)m);
+            size_t subjectBytes = 0, borderEntries = 0;
+            int numGroups = 0;
+            for (int k = 0; k < m; k++) {
+                const int len = lengthOf(order[pos + k]), W = warpsOf(len);
+                CoordItem& it = cs.hItems.p[k];
+                it.subjectOffset = subjectBytes;
+                it.subjectLength = len;
+                it.borderOffset = borderEntries;
+                subjectBytes += alignUp((size_t)len, 16);
+                if (tilesOf(len) > 1) borderEntries += (size_t)W * borderStride;
+                CoordGroup* last = numGroups ? &cs.hGroups.p[numGroups - 1] : nullptr;
+                if (W == 1 && last && last->warps == 1 && last->count < kCoordWarps) last->count++;
+                else cs.hGroups.p[numGroups++] = CoordGroup{k, 1, W};
+                cells += (double)qlen * (double)len;
+            }
+            cs.hSubjects.ensure(std::max<size_t>(subjectBytes, 1));
+            for (int k = 0; k < m; k++) {
+                const size_t li = local[order[pos + k]];
+                memcpy(cs.hSubjects.p + cs.hItems.p[k].subjectOffset, db->chars + db->offsets[li], (size_t)db->lengths[li]);
+            }
+            // one scratch arena: subjects, then border columns (16-byte aligned: every subject is padded to 16)
+            const size_t scratchBytes = subjectBytes + borderEntries * sizeof(int2);
+            if (std::max<size_t>(scratchBytes, 16) > cs.dSubjects.n) cs.dSubjects.alloc(std::max<size_t>(scratchBytes, 16));
+            if ((size_t)m > cs.dItems.n) { cs.dItems.alloc((size_t)m); cs.dGroups.alloc((size_t)m); cs.dEnds.alloc((size_t)m); }
+            if ((size_t)m * 5 + 1 > cs.dOut.n) cs.dOut.alloc((size_t)m * 5 + 1);
+            cs.hOut.ensure((size_t)m * 5 + 1);
+            if (subjectBytes) SW4_CUDA(cudaMemcpyAsync(cs.dSubjects.p, cs.hSubjects.p, subjectBytes, cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemcpyAsync(cs.dItems.p, cs.hItems.p, (size_t)m * sizeof(CoordItem), cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemcpyAsync(cs.dGroups.p, cs.hGroups.p, (size_t)numGroups * sizeof(CoordGroup), cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemsetAsync(cs.dOut.p + (size_t)m * 5, 0, sizeof(int32_t), st));
+            CoordParams p{};
+            p.groups = cs.dGroups.p; p.items = cs.dItems.p; p.subjects = cs.dSubjects.p;
+            p.query = cs.dQueryCodes.p; p.qlen = qlen; p.matrix = cs.dMatrix.p; p.gop = gop; p.gex = gex;
+            p.border = reinterpret_cast<int2*>(cs.dSubjects.p + subjectBytes); p.borderStride = (int)borderStride;
+            p.ends = cs.dEnds.p; p.out = cs.dOut.p; p.errors = cs.dOut.p + (size_t)m * 5;
+            SW4_CUDA(launch_coords(false, p, numGroups, st));
+            SW4_CUDA(launch_coords(true, p, numGroups, st));
+            launches += 2;
+            SW4_CUDA(cudaMemcpyAsync(cs.hOut.p, cs.dOut.p, ((size_t)m * 5 + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+            SW4_CUDA(cudaStreamSynchronize(st));
+            if (cs.hOut.p[(size_t)m * 5] != 0)
+                fail(SW4_ERR_CUDA, "internal error: the begin pass of %d pairs did not reach the anchored score", cs.hOut.p[(size_t)m * 5]);
+            for (int k = 0; k < m; k++) {
+                const int32_t* r = cs.hOut.p + (size_t)k * 5;
+                out[order[pos + k]] = sw4_alignment{r[0], r[1], r[2], r[3], r[4]};
+                if (r[0] > 0) cells += (double)(r[2] + 1) * (double)(r[4] + 1);
+            }
+            pos = end;
+        }
+        SW4_CUDA(cudaEventRecord(cs.evStop, st));
+        SW4_CUDA(cudaEventSynchronize(cs.evStop));
+        float ms = 0;
+        SW4_CUDA(cudaEventElapsedTime(&ms, cs.evStart, cs.evStop));
+        if (stats) {
+            stats->seconds = (double)ms * 1e-3;
+            stats->cells = cells;
+            stats->gcups = ms > 0 ? cells / 1e9 / stats->seconds : 0;
+            stats->kernel_launches = launches;
+        }
+    }
 };
 
 }  // namespace sw4
@@ -1616,6 +1797,12 @@ int sw4_scan_many(sw4_handle* h, const char* const* queries, const int32_t* quer
         if (total_stats) memset(total_stats, 0, sizeof(*total_stats));
         h->eng.scanMany(q.data(), num_queries, out_scores, out_ids, out_counts, per_query_stats, total_stats);
     });
+}
+
+int sw4_alignment_coordinates(sw4_handle* h, const char* query, int32_t query_length, const int32_t* ids, int32_t num_ids,
+                              sw4_alignment* out, sw4_stats* stats) {
+    if (!h) return SW4_ERR_INVALID;
+    return guarded(h, [&] { h->eng.alignmentCoordinates(query, query_length, ids, num_ids, out, stats); });
 }
 
 int sw4_last_scan_all_scores(sw4_handle* h, int32_t* out_scores, int32_t* out_ids, size_t capacity, size_t* out_count) {

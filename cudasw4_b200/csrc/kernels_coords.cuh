@@ -1,0 +1,199 @@
+// Alignment coordinates: exact 32-bit Gotoh passes that locate one optimal local alignment of a (query, subject) pair.
+//
+// Pass 1 (forward, REV = false) runs the local recurrence over q x s and keeps the maximum S together with its first
+// cell in (i, j) order: the end (qe, re). Pass 2 (REV = true) runs over the reversed prefixes q[qe..0] x s[re..0]
+// with the corner H(-1, -1) = kCoordAnchor, every other border H = 0 and E/F borders at minus infinity. A path from the
+// corner carries kCoordAnchor + (score of an alignment that ends with the pair (qe, re)); a path restarted at the floor
+// reaches at most S < kCoordAnchor. The optimal anchored alignments never dip below the anchor (a prefix of a score-S
+// alignment scores >= 0, because its suffix is itself an alignment scoring <= S), so the maximum of pass 2 is exactly
+// kCoordAnchor + S and its first cell in reversed (i, j) order is the lexicographically largest begin (qb, rb).
+// The first cell holding a maximum is always a substitution cell: a gap cell with that value has a predecessor with the
+// same value that comes earlier in (i, j) order.
+//
+// Organisation: the wavefront of kernels_s32.cuh (lane l owns 16 consecutive columns of a 512-column tile and runs l
+// query rows behind lane l-1; the last column's (H, E) crosses to the next tile through a border array in global memory).
+// A CTA of 16 warps holds either up to 16 short pairs, one warp each (W = 1), or one long pair whose tiles are dealt
+// round robin to W <= 16 warps: warp w runs tile t = w, w + W, ... and reads the border that warp w - 1 writes for tile
+// t - 1, 32 rows at a time, after that warp has published them in shared memory. A warp overwrites its border array for
+// tile t + W only after the W - 1 warps in between have advanced past those rows, so each border array is read before it
+// is reused.
+#pragma once
+#include <climits>
+#include <cstdint>
+#include <cuda_runtime.h>
+
+#include "kernels_s32.cuh"
+
+namespace sw4 {
+
+constexpr int kCoordThreads = 512;
+constexpr int kCoordWarps = kCoordThreads / 32;
+constexpr int kCoordR = kS32R;                    // columns per lane -> 512 columns per tile
+constexpr int kCoordTileCols = 32 * kCoordR;
+constexpr int kCoordAnchor = 1 << 24;             // scores stay below 2^24 (checked by the host)
+
+struct CoordGroup { int firstItem, count, warps; };    // one per CTA: items [firstItem, firstItem + count), W warps each
+struct CoordItem {
+    size_t subjectOffset;   // into CoordParams::subjects
+    size_t borderOffset;    // into CoordParams::border (warps * borderStride entries; unused for single-tile subjects)
+    int subjectLength;
+};
+
+struct CoordParams {
+    const CoordGroup* groups;
+    const CoordItem* items;
+    const uint8_t* subjects;    // residue codes, gathered per call
+    const uint8_t* query;       // query residue codes
+    int qlen;
+    const int8_t* matrix;       // 21x21
+    int gop, gex;
+    int2* border;
+    int borderStride;           // >= qlen
+    int4* ends;                 // [item] pass 1 writes (S, qe, re, 0); pass 2 reads it
+    int32_t* out;               // [item][5] pass 2 writes (S, qb, qe, rb, re), -1 positions when S == 0
+    int* errors;                // pass 2 counts pairs whose maximum is not kCoordAnchor + S (must stay 0)
+};
+
+// order of the tracker: value descending, then i ascending, then j ascending
+__device__ __forceinline__ bool coord_better(int v, int i, int j, int bv, int bi, int bj) {
+    return v > bv || (v == bv && (i < bi || (i == bi && j < bj)));
+}
+
+template <bool REV>
+__global__ void __launch_bounds__(kCoordThreads, 1) sw_coords_kernel(const CoordParams prm) {
+    constexpr int R = kCoordR;
+    __shared__ int Msm[21 * 21];
+    __shared__ long long progress[kCoordWarps];  // (tile << 32) | rows of that tile's right border already stored
+    __shared__ int redV[kCoordWarps], redI[kCoordWarps], redJ[kCoordWarps];
+    for (int i = threadIdx.x; i < 441; i += blockDim.x) Msm[i] = prm.matrix[i];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) progress[warp] = -1;
+    __syncthreads();
+    const CoordGroup g = prm.groups[blockIdx.x];
+    const int W = g.warps;
+    const int slot = warp / W, wi = warp % W;
+    const int item = g.firstItem + slot;
+    const bool active = slot < g.count;
+    int best = 0, bi = INT_MAX, bj = INT_MAX;
+    int S = 0, qe = 0, re = 0;
+    if (active) {
+        const CoordItem it = prm.items[item];
+        int q = prm.qlen, len = it.subjectLength;
+        if (REV) {
+            const int4 e = prm.ends[item];
+            S = e.x; qe = e.y; re = e.z;
+            q = S > 0 ? qe + 1 : 0;
+            len = S > 0 ? re + 1 : 0;
+        }
+        const uint8_t* s = prm.subjects + it.subjectOffset;
+        int2* outBorder = prm.border + it.borderOffset + (size_t)wi * prm.borderStride;
+        const int2* inBorder = prm.border + it.borderOffset + (size_t)((wi + W - 1) % W) * prm.borderStride;
+        volatile long long* leftProgress = progress + (warp - wi) + (wi + W - 1) % W;
+        volatile long long* myProgress = progress + warp;
+        const int gop = prm.gop, gex = prm.gex;
+        const int tiles = q > 0 ? (len + kCoordTileCols - 1) / kCoordTileCols : 0;
+        for (int tile = wi; tile < tiles; tile += W) {
+            const int col0 = tile * kCoordTileCols + lane * R;
+            int srow[R];
+#pragma unroll
+            for (int j = 0; j < R; j++) {
+                const int c = col0 + j;
+                const int code = c < len ? (int)s[REV ? re - c : c] : 20;
+                srow[j] = min(code, 20);
+            }
+            int Hp[R], F[R];
+#pragma unroll
+            for (int j = 0; j < R; j++) { Hp[j] = 0; F[j] = kNegS32; }
+            int Hlast = 0, Elast = kNegS32;
+            int HinPrev = (REV && tile == 0 && lane == 0) ? kCoordAnchor : 0;  // H(-1, -1)
+            int2 inBuf = make_int2(0, kNegS32), outBuf = make_int2(0, 0);
+            const bool firstTile = tile == 0, lastTile = tile == tiles - 1;
+            const int steps = q + 31;
+            for (int t = 0; t < steps; t++) {
+                if (!firstTile && (t & 31) == 0) {  // next 32 rows of the left border, once the left warp stored them
+                    if (W > 1) {
+                        const long long need = ((long long)(tile - 1) << 32) | (long long)min(q, t + 32);
+                        if (lane == 0)
+                            while (*leftProgress < need) __nanosleep(32);
+                        __syncwarp();
+                        __threadfence_block();
+                    }
+                    const int r = t + lane;
+                    inBuf = (r < q) ? __ldcg(inBorder + r) : make_int2(0, kNegS32);
+                }
+                int Hin = __shfl_up_sync(0xffffffffu, Hlast, 1);
+                int Ein = __shfl_up_sync(0xffffffffu, Elast, 1);
+                const int bH = __shfl_sync(0xffffffffu, inBuf.x, t & 31);
+                const int bE = __shfl_sync(0xffffffffu, inBuf.y, t & 31);
+                if (lane == 0) { Hin = firstTile ? 0 : bH; Ein = firstTile ? kNegS32 : bE; }
+                const int row = t - lane;
+                if (row >= 0 && row < q) {
+                    const int* Mrow = Msm + 21 * prm.query[REV ? qe - row : row];
+                    int E = Ein, diag = HinPrev;
+                    int rowBest = 0, rowJ = 0;  // first maximum of this row segment
+#pragma unroll
+                    for (int j = 0; j < R; j++) {
+                        const int d = diag + Mrow[srow[j]];
+                        diag = Hp[j];
+                        const int h = __vimax3_s32_relu(d, E, F[j]);
+                        Hp[j] = h;
+                        const int tt = h + gop;
+                        E = __viaddmax_s32(E, gex, tt);
+                        F[j] = __viaddmax_s32(F[j], gex, tt);
+                        if (h > rowBest) { rowBest = h; rowJ = j; }
+                    }
+                    // a lane sees its rows in order and its tiles left to right: on a tie only a smaller row wins
+                    if (rowBest > best || (rowBest == best && row < bi)) { best = rowBest; bi = row; bj = col0 + rowJ; }
+                    Hlast = Hp[R - 1];
+                    Elast = E;
+                    HinPrev = Hin;
+                }
+                if (!lastTile) {  // lane 31 finished row t-31: collect 32 rows, then store them coalesced
+                    const int r31 = t - 31;
+                    const int vH = __shfl_sync(0xffffffffu, Hlast, 31);
+                    const int vE = __shfl_sync(0xffffffffu, Elast, 31);
+                    if (r31 >= 0) {
+                        if (lane == (r31 & 31)) outBuf = make_int2(vH, vE);
+                        if ((r31 & 31) == 31 || r31 == q - 1) {
+                            const int r = (r31 & ~31) + lane;
+                            if (lane <= (r31 & 31)) outBorder[r] = outBuf;
+                            if (W > 1) {
+                                __syncwarp();
+                                if (lane == 0) {
+                                    __threadfence_block();
+                                    *myProgress = ((long long)tile << 32) | (long long)(r31 + 1);
+                                }
+                            }
+                        }
+                    }
+                }
+            }
+            __syncwarp();
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const int v = __shfl_xor_sync(0xffffffffu, best, o);
+        const int i = __shfl_xor_sync(0xffffffffu, bi, o);
+        const int j = __shfl_xor_sync(0xffffffffu, bj, o);
+        if (coord_better(v, i, j, best, bi, bj)) { best = v; bi = i; bj = j; }
+    }
+    if (lane == 0) { redV[warp] = best; redI[warp] = bi; redJ[warp] = bj; }
+    __syncthreads();
+    if (!active || wi != 0 || lane != 0) return;
+    for (int w = warp + 1; w < warp + W; w++)
+        if (coord_better(redV[w], redI[w], redJ[w], best, bi, bj)) { best = redV[w]; bi = redI[w]; bj = redJ[w]; }
+    if (!REV) {
+        prm.ends[item] = best > 0 ? make_int4(best, bi, bj, 0) : make_int4(0, -1, -1, 0);
+        return;
+    }
+    int32_t* o = prm.out + (size_t)item * 5;
+    if (S <= 0) {
+        o[0] = 0; o[1] = -1; o[2] = -1; o[3] = -1; o[4] = -1;
+        return;
+    }
+    if (best != kCoordAnchor + S) atomicAdd(prm.errors, 1);
+    o[0] = S; o[1] = qe - bi; o[2] = qe; o[3] = re - bj; o[4] = re;
+}
+
+}  // namespace sw4

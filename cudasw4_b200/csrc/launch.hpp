@@ -10,6 +10,7 @@
 #include "kernels_s16_long2.cuh"
 #include "kernels_s32.cuh"
 #include "kernels_s32_long.cuh"
+#include "kernels_coords.cuh"
 
 namespace sw4 {
 
@@ -26,6 +27,8 @@ cudaError_t launch_s32_long(const S32LongParams& prm, int grid, cudaStream_t str
 cudaError_t launch_s16_long2(const S16Long2Params& prm, int grid, cudaStream_t stream);
 // exact 32-bit wavefront, one subject per warp
 cudaError_t launch_s32(const S32Params& prm, int blocks, cudaStream_t stream);
+// alignment coordinates: pass 1 (ends) or pass 2 (begins), one CTA per CoordGroup
+cudaError_t launch_coords(bool reverse, const CoordParams& prm, int groups, cudaStream_t stream);
 
 // CTAs are launched as clusters of 2 whenever the grid is even: the two SMs of a TPC share an instruction cache, and
 // with many different (large, heavily unrolled) kernels resident at once it pays to give both SMs the same code.

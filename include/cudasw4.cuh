@@ -53,6 +53,8 @@ inline int blosumNumber(BlosumType t) {
 
 struct BenchmarkStats { int numOverflows{}; double seconds{}; double gcups{}; };                       // :76-80
 struct ScanResult { std::vector<int> scores{}; std::vector<ReferenceIdT> referenceIds{}; BenchmarkStats stats{}; };
+// Extension (no reference counterpart): where a hit aligns, 0-based inclusive, -1 when score == 0 (sw4b200.h)
+struct AlignmentCoordinates { int score, queryBegin, queryEnd, referenceBegin, referenceEnd; };
 struct KernelTypeConfig {                                                                             // :88-93
     KernelType singlePassType = KernelType::Half2;
     KernelType manyPassType_small = KernelType::Half2;
@@ -174,7 +176,18 @@ public:
         return out;
     }
 
-    void printDBInfo() const {                                                                        // :799-807
+    // Extension: score, begin and end of one optimal local alignment of the query against each database id.
+    std::vector<AlignmentCoordinates> computeAlignmentCoordinates(const char* query, SequenceLengthT length,
+                                                                  const std::vector<ReferenceIdT>& ids) {
+        std::vector<sw4_alignment> raw(std::max<size_t>(1, ids.size()));
+        check(sw4_alignment_coordinates(handle, query, length, ids.data(), (int32_t)ids.size(), raw.data(), nullptr));
+        std::vector<AlignmentCoordinates> out(ids.size());
+        for (size_t i = 0; i < ids.size(); i++)
+            out[i] = AlignmentCoordinates{raw[i].score, raw[i].query_begin, raw[i].query_end, raw[i].reference_begin, raw[i].reference_end};
+        return out;
+    }
+
+    void printDBInfo() const {                                                                      // :799-807
         sw4_db_info info{}; check(sw4_get_db_info(handle, &info));
         std::cout << info.num_sequences << " sequences, " << info.num_residues << " characters\n";
     }

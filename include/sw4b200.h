@@ -151,6 +151,30 @@ int sw4_scan_many(sw4_handle* h, const char* const* queries, const int32_t* quer
                   int32_t* out_scores, int32_t* out_ids, int32_t* out_counts, sw4_stats* per_query_stats,
                   sw4_stats* total_stats);
 
+/* Where each hit aligns (no reference counterpart): for every id, the exact score and the begin and end of one optimal
+ * local alignment in the query and in the reference, computed on the handle's first GPU on a stream of its own, with
+ * the current matrix and gap scores. Positions are 0-based and inclusive. With H the local Gotoh matrix (i: query,
+ * j: reference) and S = max H:
+ *   end   (query_end, reference_end)     = the smallest (i, j) in (i, j) order with H(i, j) == S;
+ *   begin (query_begin, reference_begin) = the largest (i, j) such that an alignment starting with the pair (i, j) and
+ *                                          ending with the pair at the end scores S (the shortest optimal alignment);
+ *   S == 0 (no positive substitution, empty query or subject): all four positions are -1.
+ * query = residue LETTERS (converted as sw4_scan converts them). ids are global database ids, duplicates allowed;
+ * num_ids == 0 does nothing. Subjects come from the host copy, so the call works before sw4_upload_database and in
+ * every database mode, and leaves the results of later scans unchanged. Pairs whose scratch (subjects + border
+ * columns) does not fit max_temp_bytes at once are processed in chunks; a single pair that cannot fit is
+ * SW4_ERR_NOMEM. SW4_ERR_INVALID: no database, num_ids < 0, an id < 0 or >= num_sequences or not held by a pre-sharded
+ * handle, query_length > 2^24, or a pair whose score could reach 2^24 (max matrix entry x min(query, subject) length).
+ * stats may be NULL: seconds is device-timed (CUDA events), cells counts both passes, kernel_launches the kernels. */
+typedef struct sw4_alignment {
+    int32_t score;                           /* exact Gotoh score (== what sw4_scan reports for this id) */
+    int32_t query_begin, query_end;          /* 0-based, inclusive; -1 when score == 0 */
+    int32_t reference_begin, reference_end;  /* 0-based, inclusive; -1 when score == 0 */
+} sw4_alignment;
+
+int sw4_alignment_coordinates(sw4_handle* h, const char* query, int32_t query_length, const int32_t* ids, int32_t num_ids,
+                              sw4_alignment* out, sw4_stats* stats);
+
 /* Debug / parity helper (the reference's CUDASW_DEBUG_CHECK_CORRECTNESS mode sets numTop to the whole database,
  * src/cudasw4.cuh:505-507): all scores of the last scan for this handle's shard, plus their global ids, in shard
  * order. capacity is in entries; returns the number written in *out_count. */
