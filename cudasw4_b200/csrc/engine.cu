@@ -283,6 +283,7 @@ struct Ctx {
         dClassNs.alloc(96);
         dMatrix.alloc(441);
         dCand.alloc(kTopkMaxCandidates);
+        SW4_CUDA(topk_configure());  // every context sets it on its shard's device (runShard selects it before creating them)
     }
     ~Ctx() {
         for (cudaEvent_t e : {evStart, evK0, evK1, evStop, evFork, evBatchDone[0], evBatchDone[1]})
@@ -795,7 +796,7 @@ struct Engine {
             ctx.dProfile.ensure((size_t)kProfileRows * capStride);
             ctx.dTopScores.ensure(ctx.topCapacity);
             ctx.dTopIds.ensure(ctx.topCapacity);
-            if (k > kTopkMaxCandidates / 2) {
+            if (topk_uses_large_path(k)) {
                 ctx.dTopkWork.ensure(topk_large_work_ints());
                 ctx.dTopkKeys.ensure((size_t)topk_large_num_keys(k));
             }
@@ -1105,27 +1106,10 @@ struct Engine {
         const int k = ctx.k;
         if (k > 0 && n > 0) {
             const long long bound = (long long)maxMatrixEntry * std::min(ctx.qlen, sh.maxLen);
-            const int shift = topk_shift_for(bound);
-            if (shift < 0) fail(SW4_ERR_INVALID, "scores of this scan may reach %lld; the device top-k is exact below 2^24", bound);
-            if (k <= kTopkMaxCandidates / 2) {
-                int blocks = (int)std::min<long long>(std::min<long long>(sh.smCount, kTopkMaxCandidates / k), (n + 4095) / 4096);
-                blocks = std::max(blocks, 1);
-                topk_pass1_kernel<<<blocks, kTopkThreads, 0, st>>>(ctx.dScores.p, nullptr, n, k, shift, ctx.dCand.p);
-                const int numCand = blocks * k;
-                int n2 = 1;
-                while (n2 < numCand) n2 <<= 1;
-                static bool pass2Configured[64] = {};
-                if (!pass2Configured[sh.device & 63]) {
-                    SW4_CUDA(cudaFuncSetAttribute(topk_pass2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTopkMaxCandidates * 8));
-                    pass2Configured[sh.device & 63] = true;
-                }
-                topk_pass2_kernel<<<1, kTopkThreads, (size_t)n2 * 8, st>>>(ctx.dCand.p, numCand, k, sh.dGlobalIds.p, ctx.dTopScores.p,
-                                                                           ctx.dTopIds.p, ctx.dCounters.p + 4);
-                ctx.launches += 2;
-            } else {
-                ctx.launches += topk_large_enqueue(ctx.dScores.p, n, k, shift, sh.dGlobalIds.p, ctx.dTopkWork.p, ctx.dTopkKeys.p,
-                                                   ctx.dTopScores.p, ctx.dTopIds.p, ctx.dCounters.p + 4, st);
-            }
+            const int launches = topk_enqueue(ctx.dScores.p, n, k, bound, sh.smCount, sh.dGlobalIds.p, ctx.dCand.p, ctx.dTopkWork.p,
+                                              ctx.dTopkKeys.p, ctx.dTopScores.p, ctx.dTopIds.p, ctx.dCounters.p + 4, st);
+            if (launches < 0) fail(SW4_ERR_INVALID, "scores of this scan may reach %lld; the device top-k is exact below 2^24", bound);
+            ctx.launches += launches;
             SW4_CUDA(cudaGetLastError());
             SW4_CUDA(cudaMemcpyAsync(ctx.hTop.p, ctx.dTopScores.p, (size_t)k * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
             SW4_CUDA(cudaMemcpyAsync(ctx.hTop.p + k, ctx.dTopIds.p, (size_t)k * sizeof(int32_t), cudaMemcpyDeviceToHost, st));

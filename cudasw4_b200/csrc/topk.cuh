@@ -38,6 +38,8 @@ static inline int topk_shift_for(long long maxScore) {
 // Block-wide: given hist[0..nbins) in shared memory, find the highest bin b such that (count of entries in bins > b) < k
 // <= (count in bins >= b), or b = 0 when even all bins together hold fewer than k. Returns (b, count above b) in
 // sBin/sAbove. Every thread owns nbins/blockDim consecutive bins; the suffix sums come from a reverse block scan.
+// baseAbove (entries above all of hist) is below k. Both barriers are unconditional: every thread derives the total
+// from warpTotals itself, so no thread decides anything from sBin/sAbove while another one may be writing them.
 __device__ __forceinline__ void topk_find_bin(const int* hist, int nbins, int k, int baseAbove, int* warpTotals, int* sBin,
                                               int* sAbove) {
     const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, nthreads = blockDim.x;
@@ -54,10 +56,12 @@ __device__ __forceinline__ void topk_find_bin(const int* hist, int nbins, int k,
         if (lane >= o) incl += v;
     }
     if (lane == 31) warpTotals[w] = incl;
-    if (tid == 0) { *sBin = 0; *sAbove = -1; }
     __syncthreads();
-    int before = baseAbove;
-    for (int x = 0; x < w; x++) before += warpTotals[x];
+    int before = baseAbove, total = baseAbove;
+    for (int x = 0; x < (nthreads + 31) / 32; x++) {
+        if (x < w) before += warpTotals[x];
+        total += warpTotals[x];
+    }
     const int exclusive = before + incl - mine;  // entries in bins above this thread's range
     if (exclusive < k && exclusive + mine >= k) {   // the crossing is inside this thread's bins (exactly one thread)
         int above = exclusive;
@@ -67,16 +71,11 @@ __device__ __forceinline__ void topk_find_bin(const int* hist, int nbins, int k,
             above += c;
         }
     }
-    __syncthreads();
-    if (*sAbove < 0) {  // fewer than k entries in total: bin 0 decides, everything above it is kept
-        if (tid == 0) {
-            int total = baseAbove;
-            for (int x = 0; x < (nthreads + 31) / 32; x++) total += warpTotals[x];
-            *sAbove = total - hist[0];
-            *sBin = 0;
-        }
-        __syncthreads();
+    if (total < k && tid == 0) {  // no crossing (fewer than k entries in total): bin 0 decides, everything above it is kept
+        *sBin = 0;
+        *sAbove = total - hist[0];
     }
+    __syncthreads();
 }
 
 // scores[begin+i]; indexOf = begin+i (or indices[begin+i] when indices != nullptr, which must be ascending)
@@ -85,7 +84,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_pass1_kernel(const int32_t*
                                                                   int k, int shift, TopkCand* __restrict__ out) {
     __shared__ int hist[kTopkHiBins];
     __shared__ int warpTotals[kTopkThreads / 32];
-    __shared__ int sBin, sAbove, sRunning, sEmitted;
+    __shared__ int sBin, sAbove, sRunning, sEmitted, sDone;
     const int tid = threadIdx.x;
     const long long per = (n + gridDim.x - 1) / gridDim.x;
     const long long begin = per * blockIdx.x;
@@ -142,9 +141,11 @@ __global__ void __launch_bounds__(kTopkThreads) topk_pass1_kernel(const int32_t*
             int tot = 0;
             for (int x = 0; x < kTopkThreads / 32; x++) tot += warpTotals[x];
             sRunning += tot;
+            // decided once, between barriers: the next chunk's atomicAdd on sEmitted must not reach a slower warp's test
+            sDone = sRunning >= need && sEmitted >= sAbove;
         }
         __syncthreads();
-        if (sRunning >= need && sEmitted >= sAbove) break;  // uniform: shared values after barrier
+        if (sDone) break;  // uniform: written before the barrier, next written after two more barriers
     }
 }
 
@@ -399,6 +400,44 @@ static inline int topk_large_enqueue(const int32_t* scores, long long n, int k, 
     }
     topkL_write_kernel<<<(k + 255) / 256, 256, 0, stream>>>(keys, k, globalIds, outScores, outIds, outCount);
     return launches + 1;
+}
+
+// -----------------------------------------------------------------------------------------------------------------
+// Dispatch: the one place that picks the path, the shift and the pass-1 split.
+// -----------------------------------------------------------------------------------------------------------------
+static inline bool topk_uses_large_path(int k) { return k > kTopkMaxCandidates / 2; }
+
+// Pass-1 blocks: at most one per SM, at most kTopkMaxCandidates / k (pass 2 sorts all their candidates in shared
+// memory), and no more than one per 4096 entries. Block b owns [b * per, min(n, (b + 1) * per)), per = ceil(n / blocks).
+static inline int topk_pass1_blocks(long long n, int k, int smCount) {
+    const long long blocks = std::min<long long>(std::min<long long>(smCount, kTopkMaxCandidates / k), (n + 4095) / 4096);
+    return (int)std::max<long long>(blocks, 1);
+}
+
+// On the current device, before its first topk_enqueue (repeating it is harmless): pass 2 sorts up to
+// kTopkMaxCandidates keys in dynamic shared memory.
+static inline cudaError_t topk_configure() {
+    return cudaFuncSetAttribute(topk_pass2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTopkMaxCandidates * 8);
+}
+
+// Top-k of scores[0..n) (all >= 0 and <= maxScore, 1 <= k <= n) under (score desc, index asc), written to
+// outScores/outIds[0..k) (index -> globalIds[index] when globalIds != nullptr) and *outCount, enqueued on `stream`.
+// Scratch: cand[kTopkMaxCandidates]; for the large path (topk_uses_large_path) also work[topk_large_work_ints()] and
+// keys[topk_large_num_keys(k)]. Returns the number of kernels launched, or -1 (nothing launched) when maxScore >= 2^24.
+static inline int topk_enqueue(const int32_t* scores, long long n, int k, long long maxScore, int smCount,
+                               const int32_t* globalIds, TopkCand* cand, int* work, unsigned long long* keys,
+                               int32_t* outScores, int32_t* outIds, int* outCount, cudaStream_t stream) {
+    const int shift = topk_shift_for(maxScore);
+    if (shift < 0) return -1;
+    if (topk_uses_large_path(k))
+        return topk_large_enqueue(scores, n, k, shift, globalIds, work, keys, outScores, outIds, outCount, stream);
+    const int blocks = topk_pass1_blocks(n, k, smCount);
+    topk_pass1_kernel<<<blocks, kTopkThreads, 0, stream>>>(scores, nullptr, n, k, shift, cand);
+    const int numCand = blocks * k;
+    int n2 = 1;
+    while (n2 < numCand) n2 <<= 1;
+    topk_pass2_kernel<<<1, kTopkThreads, (size_t)n2 * 8, stream>>>(cand, numCand, k, globalIds, outScores, outIds, outCount);
+    return 2;
 }
 
 }  // namespace sw4
