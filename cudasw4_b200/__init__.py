@@ -14,7 +14,7 @@ import numpy as np
 
 from . import _lib, dbformat
 
-__all__ = ["CudaSW4", "ScanResult", "BenchmarkStats", "KernelType", "KernelTypeConfig", "MemoryConfig", "BlosumType",
+__all__ = ["CudaSW4", "ScanResult", "Alignments", "BenchmarkStats", "KernelType", "KernelTypeConfig", "MemoryConfig", "BlosumType",
            "SW4Error", "dbformat"]
 
 
@@ -73,6 +73,16 @@ class ScanResult:  # reference src/cudasw4.cuh:82-86
     scores: list = field(default_factory=list)
     referenceIds: list = field(default_factory=list)
     stats: BenchmarkStats = field(default_factory=BenchmarkStats)
+
+
+@dataclass
+class Alignments:
+    """What CudaSW4.alignments returns, one row per id: `coordinates` (n, 5) int32 as alignmentCoordinates, `counts`
+    (n, 4) int32 (alignment length, identities, positives, gaps) and `cigars` (SAM-style run-length ops =, X, I, D in
+    query order, with the query as the read; "" when the score is 0)."""
+    coordinates: np.ndarray
+    counts: np.ndarray
+    cigars: list
 
 
 def _stats(s: _lib.Stats) -> BenchmarkStats:
@@ -268,6 +278,31 @@ class CudaSW4:
             for k, v in vars(_stats(st)).items():
                 setattr(stats, k, v)
         return out[:len(idv)].copy()
+
+    def alignments(self, query, ids, stats: BenchmarkStats | None = None) -> Alignments:
+        """How each hit aligns: the coordinates of alignmentCoordinates, and the CIGAR and counts of the one alignment
+        they locate, traced back on the GPU (the rule is in include/sw4b200.h). `stats`, when given, receives the
+        call's device-timed figures (cells and kernel launches of all three passes)."""
+        q = query.encode() if isinstance(query, str) else bytes(query)
+        idv = np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1))
+        if len(idv) and (idv.min() < -2**31 or idv.max() >= 2**31):
+            raise SW4Error(-1, "database id out of range")
+        idv = idv.astype(np.int32)
+        n = len(idv)
+        out = (_lib.AlignmentSummary * max(n, 1))()
+        st = _lib.Stats()
+        self._check(self._lib.sw4_alignment_traceback(self._h, q, len(q), idv.ctypes.data, n, out, ctypes.byref(st)))
+        p = ctypes.c_void_p()
+        size = ctypes.c_size_t(0)
+        self._check(self._lib.sw4_last_cigars(self._h, ctypes.byref(p), ctypes.byref(size)))
+        text = ctypes.string_at(p.value, size.value).decode() if size.value else ""
+        raw = np.frombuffer(out, dtype=np.dtype([("coordinates", "<i4", 5), ("counts", "<i4", 4),
+                                                 ("offset", "<u8"), ("length", "<u8")], align=True))[:n]
+        if stats is not None:
+            for k, v in vars(_stats(st)).items():
+                setattr(stats, k, v)
+        cigars = [text[int(o):int(o) + int(L)] for o, L in zip(raw["offset"], raw["length"])]
+        return Alignments(raw["coordinates"].copy(), raw["counts"].copy(), cigars)
 
     def lastScanAllScores(self):
         """(scores, global ids) of every subject this handle scanned in the last scan() (parity helper)."""

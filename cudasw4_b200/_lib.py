@@ -14,6 +14,7 @@ EXPORTS = [
     "sw4_last_scan_all_scores", "sw4_reference_header",
     "sw4_reference_length", "sw4_reference_sequence", "sw4_total_timer_start", "sw4_total_timer_stop",
     "sw4_get_db_info", "sw4_version", "sw4_alignment_coordinates",
+    "sw4_alignment_traceback", "sw4_last_cigars",
 ]
 
 
@@ -30,6 +31,12 @@ class Stats(ctypes.Structure):
 class Alignment(ctypes.Structure):
     _fields_ = [("score", ctypes.c_int32), ("query_begin", ctypes.c_int32), ("query_end", ctypes.c_int32),
                 ("reference_begin", ctypes.c_int32), ("reference_end", ctypes.c_int32)]
+
+
+class AlignmentSummary(ctypes.Structure):
+    _fields_ = [("coordinates", Alignment), ("length", ctypes.c_int32), ("identities", ctypes.c_int32),
+                ("positives", ctypes.c_int32), ("gaps", ctypes.c_int32), ("cigar_offset", ctypes.c_size_t),
+                ("cigar_length", ctypes.c_size_t)]
 
 
 class DbInfo(ctypes.Structure):
@@ -73,6 +80,9 @@ def load() -> ctypes.CDLL:
                                   ctypes.POINTER(Stats), ctypes.POINTER(Stats)]
     lib.sw4_alignment_coordinates.argtypes = [vp, ctypes.c_char_p, ctypes.c_int32, vp, ctypes.c_int32, vp,
                                               ctypes.POINTER(Stats)]
+    lib.sw4_alignment_traceback.argtypes = [vp, ctypes.c_char_p, ctypes.c_int32, vp, ctypes.c_int32, vp,
+                                            ctypes.POINTER(Stats)]
+    lib.sw4_last_cigars.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(cs)]
     lib.sw4_last_scan_all_scores.argtypes = [vp, vp, vp, cs, ctypes.POINTER(cs)]
     lib.sw4_reference_header.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(vp), ctypes.POINTER(cs)]
     lib.sw4_reference_length.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32)]

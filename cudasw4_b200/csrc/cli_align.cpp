@@ -19,7 +19,7 @@ namespace {
 struct Options {
     enum class Output { Plain, TSV };
     bool help = false, uploadFull = false, pseudo = false, printPartitions = false, interactive = false, verbose = false,
-         prefetchFile = false, coordinates = false;
+         prefetchFile = false, coordinates = false, cigar = false;
     int top = 10, gop = -11, gex = -1, pseudoLen = 0;
     int batchQueries = 1;  // extension: queries handed to one scanMany call (1 = one scan per query, as the reference)
     size_t pseudoNum = 0;
@@ -91,6 +91,7 @@ bool parseArgs(int argc, char** argv, Options& o) {
         else if (a == "--dpx") dpx = true;
         else if (a == "--tsv") o.output = Options::Output::TSV;
         else if (a == "--coordinates") o.coordinates = true;
+        else if (a == "--cigar") o.cigar = true;
         else if (a == "--of") o.outfile = need(i);
         else std::cout << "Unexpected arg " << a << "\n";
     }
@@ -124,6 +125,7 @@ void printHelp(const char* prog) {
               << "   --of file : Result output file. Default /dev/stdout\n"
               << "   --tsv : tab-separated output\n"
               << "   --coordinates : (extension) also print where each hit aligns: 1-based query and reference begin and end\n"
+              << "   --cigar : (extension) also print how each hit aligns: length, identities, positives, gaps and CIGAR\n"
               << "   --verbose, --printLengthPartitions, --interactive, --help\n"
               << "   --batchQueries n : (extension) scan n queries of a file with several scans in flight per GPU; same results\n"
               << "   --prefetchDBFile, --uploadFull, --pseudodb num length\n"
@@ -152,9 +154,10 @@ void printOptions(const Options& o) {
 }
 
 // result printers: formats of reference src/main.cu:34-87 and 243-245. With --coordinates (`coords` non-empty, one
-// entry per hit) every line also carries where the hit aligns, 1-based inclusive as in BLAST (0 = no alignment).
+// entry per hit) every line also carries where the hit aligns, 1-based inclusive as in BLAST (0 = no alignment); with
+// --cigar (`alignments` non-empty) how it aligns: length, identities, positives, gaps and the CIGAR.
 void printPlain(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::CudaSW4& sw,
-                const std::vector<cudasw4::AlignmentCoordinates>& coords) {
+                const std::vector<cudasw4::AlignmentCoordinates>& coords, const std::vector<cudasw4::Alignment>& alignments) {
     for (size_t i = 0; i < r.scores.size(); i++) {
         const auto id = r.referenceIds[i];
         os << "Result " << i << "." << " Score: " << r.scores[i] << "." << " Length: " << sw.getReferenceLength(id) << "."
@@ -164,17 +167,24 @@ void printPlain(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::C
             os << " Query " << c.queryBegin + 1 << "-" << c.queryEnd + 1 << ". Reference " << c.referenceBegin + 1 << "-"
                << c.referenceEnd + 1 << ".";
         }
+        if (!alignments.empty()) {
+            const auto& a = alignments[i];
+            os << " Identities " << a.identities << "/" << a.length << ". Positives " << a.positives << "/" << a.length
+               << ". Gaps " << a.gaps << "/" << a.length << ". CIGAR " << a.cigar << ".";
+        }
         os << "\n";
     }
 }
-void printTSVHeader(std::ostream& os, bool coordinates) {
+void printTSVHeader(std::ostream& os, bool coordinates, bool cigar) {
     os << "Query number\tQuery length\tQuery header\tResult number\tResult score\tReference length\tReference header\t"
           "Reference ID in DB";
     if (coordinates) os << "\tQuery begin\tQuery end\tReference begin\tReference end";
+    if (cigar) os << "\tAlignment length\tIdentities\tPositives\tGaps\tCIGAR";
     os << "\n";
 }
 void printTSV(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::CudaSW4& sw, int64_t qnum, size_t qlen,
-              const std::string& qheader, const std::vector<cudasw4::AlignmentCoordinates>& coords) {
+              const std::string& qheader, const std::vector<cudasw4::AlignmentCoordinates>& coords,
+              const std::vector<cudasw4::Alignment>& alignments) {
     for (size_t i = 0; i < r.scores.size(); i++) {
         const auto id = r.referenceIds[i];
         os << qnum << '\t' << qlen << '\t' << qheader << '\t' << i << '\t' << r.scores[i] << '\t' << sw.getReferenceLength(id)
@@ -182,6 +192,10 @@ void printTSV(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::Cud
         if (!coords.empty()) {
             const auto& c = coords[i];
             os << '\t' << c.queryBegin + 1 << '\t' << c.queryEnd + 1 << '\t' << c.referenceBegin + 1 << '\t' << c.referenceEnd + 1;
+        }
+        if (!alignments.empty()) {
+            const auto& a = alignments[i];
+            os << '\t' << a.length << '\t' << a.identities << '\t' << a.positives << '\t' << a.gaps << '\t' << a.cigar;
         }
         os << "\n";
     }
@@ -215,14 +229,20 @@ void reportQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int6
     else std::cout << "Done.\n";
     if (o.top > 0) {
         std::vector<cudasw4::AlignmentCoordinates> coords;
-        if (o.coordinates && !r.referenceIds.empty())
+        std::vector<cudasw4::Alignment> alignments;
+        if (o.cigar && !r.referenceIds.empty()) {  // the traceback reports the coordinates too
+            alignments = sw.computeAlignments(sequence.data(), (int)sequence.size(), r.referenceIds);
+            if (o.coordinates)
+                for (const auto& a : alignments) coords.push_back(a.coordinates);
+        } else if (o.coordinates && !r.referenceIds.empty()) {
             coords = sw.computeAlignmentCoordinates(sequence.data(), (int)sequence.size(), r.referenceIds);
+        }
         if (o.output == Options::Output::Plain) {
             out << "Query " << qnum << ", header" << header << ", length " << sequence.size() << ", num overflows "
                 << r.stats.numOverflows << "\n";
-            printPlain(out, r, sw, coords);
+            printPlain(out, r, sw, coords, alignments);
         } else {
-            printTSV(out, r, sw, qnum, sequence.size(), header, coords);
+            printTSV(out, r, sw, qnum, sequence.size(), header, coords, alignments);
         }
         out.flush();
     }
@@ -237,7 +257,7 @@ int main(int argc, char** argv) {
         printOptions(o);
         std::ofstream out(o.outfile);
         if (!out) throw std::runtime_error("Cannot open file " + o.outfile);
-        if (o.output == Options::Output::TSV) printTSVHeader(out, o.coordinates);
+        if (o.output == Options::Output::TSV) printTSVHeader(out, o.coordinates, o.cigar);
 
         cudasw4::CudaSW4 sw({}, o.top, o.blosum, o.kernels, o.mem, o.verbose);  // {} = all visible GPUs
         sw.setGapOpenScore(o.gop);

@@ -364,7 +364,7 @@ static inline int s16WidePeriod(int qlen, int G) { return std::max(32, (qlen + G
 
 struct QueryRef { const char* letters; int length; };
 
-// Everything sw4_alignment_coordinates owns on the handle's first GPU: it shares nothing with the scan (slots, contexts,
+// Everything sw4_alignment_coordinates and sw4_alignment_traceback own on the handle's first GPU: it shares nothing with the scan (slots, contexts,
 // results), so a scan after the call returns what it would have returned without it.
 struct CoordState {
     int device = 0;
@@ -383,6 +383,10 @@ struct CoordState {
     PinnedBuf<CoordGroup> hGroups;
     PinnedBuf<CoordItem> hItems;
     PinnedBuf<int32_t> hOut;
+    // traceback: per-pair rectangles, and the ops, counts and error counters copied back
+    DevBuf<TraceItem> dTraceItems;
+    PinnedBuf<TraceItem> hTraceItems;
+    PinnedBuf<char> hTraceOut;
 
     void create(int dev) {
         device = dev;
@@ -426,10 +430,11 @@ struct Engine {
     int shardRank = 0, shardWorld = 1;
     std::unique_ptr<HostDB> db;
     std::vector<std::unique_ptr<Shard>> shards;
-    std::unique_ptr<CoordState> coord;  // created by the first sw4_alignment_coordinates call
+    std::unique_ptr<CoordState> coord;  // created by the first sw4_alignment_coordinates / _traceback call
     int8_t matrix[441];
     int maxMatrixEntry = 11;
     std::string lastError;
+    std::string lastCigars;  // CIGAR text of the last sw4_alignment_traceback (sw4_last_cigars)
     // total timer
     std::chrono::steady_clock::time_point totalStart;
     double totalCells = 0;
@@ -1299,7 +1304,9 @@ struct Engine {
     // Subjects come from the host copy (any database mode, before or after the upload) and go through pinned staging to
     // the handle's first GPU. Pass 1 leaves the ends on the device for pass 2; the host waits once per chunk of pairs
     // whose scratch (gathered subjects + border columns) fits max_temp_bytes.
-    void alignmentCoordinates(const char* query, int qlen, const int32_t* ids, int n, sw4_alignment* out, sw4_stats* stats) {
+    // Checks the arguments shared by sw4_alignment_coordinates and sw4_alignment_traceback; returns the position of
+    // every id in the handle's host arrays.
+    std::vector<size_t> alignmentPairs(const char* query, int qlen, const int32_t* ids, int n, const void* out) {
         if (!db) fail(SW4_ERR_INVALID, "no database set");
         if (n < 0) fail(SW4_ERR_INVALID, "num_ids must be >= 0 (got %d)", n);
         if (n > 0 && (!ids || !out)) fail(SW4_ERR_INVALID, "null id or output array");
@@ -1317,8 +1324,11 @@ struct Engine {
             if (topk_shift_for(bound) < 0)
                 fail(SW4_ERR_INVALID, "the score of the query against id %d may reach %lld; scores are exact below 2^24", id, bound);
         }
-        if (stats) memset(stats, 0, sizeof(*stats));
-        if (n == 0) return;
+        return local;
+    }
+
+    // the CoordState on the handle's first GPU (made current) with the query codes and the matrix uploaded on its stream
+    CoordState& coordQuery(const char* query, int qlen, int& launches) {
         if (!coord) {
             auto c = std::make_unique<CoordState>();
             c->create(deviceIds[0]);
@@ -1326,6 +1336,39 @@ struct Engine {
         }
         CoordState& cs = *coord;
         SW4_CUDA(cudaSetDevice(cs.device));
+        cudaStream_t st = cs.stream;
+        SW4_CUDA(cudaEventRecord(cs.evStart, st));
+        const int qpad = (qlen + 3) / 4 * 4;
+        cs.hQuery.ensure((size_t)std::max(qlen, 1));
+        if (qlen) memcpy(cs.hQuery.p, query, (size_t)qlen);
+        if ((size_t)qpad + 16 > cs.dQueryCodes.n) { cs.dQueryLetters.alloc((size_t)qpad + 16); cs.dQueryCodes.alloc((size_t)qpad + 16); }
+        if (qlen) SW4_CUDA(cudaMemcpyAsync(cs.dQueryLetters.p, cs.hQuery.p, (size_t)qlen, cudaMemcpyHostToDevice, st));
+        SW4_CUDA(cudaMemcpyAsync(cs.dMatrix.p, matrix, 441, cudaMemcpyHostToDevice, st));
+        if (qpad > 0) {
+            convert_query_kernel<<<(qpad + 255) / 256, 256, 0, st>>>(cs.dQueryLetters.p, cs.dQueryCodes.p, qlen, qpad);
+            SW4_CUDA(cudaGetLastError());
+            launches++;
+        }
+        return cs;
+    }
+
+    // stats of a coordinate / traceback call: device time from coordQuery's start event to now
+    void coordStats(CoordState& cs, double cells, int launches, sw4_stats* stats) {
+        SW4_CUDA(cudaEventRecord(cs.evStop, cs.stream));
+        SW4_CUDA(cudaEventSynchronize(cs.evStop));
+        float ms = 0;
+        SW4_CUDA(cudaEventElapsedTime(&ms, cs.evStart, cs.evStop));
+        if (stats) {
+            stats->seconds = (double)ms * 1e-3;
+            stats->cells = cells;
+            stats->gcups = ms > 0 ? cells / 1e9 / stats->seconds : 0;
+            stats->kernel_launches = launches;
+        }
+    }
+
+    // passes 1 and 2 for the pairs (query, local[i]), in chunks under max_temp_bytes; out[i] receives the coordinates
+    void coordPasses(CoordState& cs, int qlen, const std::vector<size_t>& local, sw4_alignment* out, double& cells, int& launches) {
+        const int n = (int)local.size();
         cudaStream_t st = cs.stream;
         auto lengthOf = [&](int i) { return (int)db->lengths[local[i]]; };
         auto tilesOf = [](int len) { return (len + kCoordTileCols - 1) / kCoordTileCols; };
@@ -1349,20 +1392,6 @@ struct Engine {
             return la > lb;
         });
 
-        int launches = 0;
-        double cells = 0;
-        SW4_CUDA(cudaEventRecord(cs.evStart, st));
-        const int qpad = (qlen + 3) / 4 * 4;
-        cs.hQuery.ensure((size_t)std::max(qlen, 1));
-        if (qlen) memcpy(cs.hQuery.p, query, (size_t)qlen);
-        if ((size_t)qpad + 16 > cs.dQueryCodes.n) { cs.dQueryLetters.alloc((size_t)qpad + 16); cs.dQueryCodes.alloc((size_t)qpad + 16); }
-        if (qlen) SW4_CUDA(cudaMemcpyAsync(cs.dQueryLetters.p, cs.hQuery.p, (size_t)qlen, cudaMemcpyHostToDevice, st));
-        SW4_CUDA(cudaMemcpyAsync(cs.dMatrix.p, matrix, 441, cudaMemcpyHostToDevice, st));
-        if (qpad > 0) {
-            convert_query_kernel<<<(qpad + 255) / 256, 256, 0, st>>>(cs.dQueryLetters.p, cs.dQueryCodes.p, qlen, qpad);
-            SW4_CUDA(cudaGetLastError());
-            launches++;
-        }
         const size_t budget = mem.max_temp_bytes;
         for (int pos = 0; pos < n;) {
             int end = pos;
@@ -1423,16 +1452,162 @@ struct Engine {
             }
             pos = end;
         }
-        SW4_CUDA(cudaEventRecord(cs.evStop, st));
-        SW4_CUDA(cudaEventSynchronize(cs.evStop));
-        float ms = 0;
-        SW4_CUDA(cudaEventElapsedTime(&ms, cs.evStart, cs.evStop));
-        if (stats) {
-            stats->seconds = (double)ms * 1e-3;
-            stats->cells = cells;
-            stats->gcups = ms > 0 ? cells / 1e9 / stats->seconds : 0;
-            stats->kernel_launches = launches;
+    }
+
+    void alignmentCoordinates(const char* query, int qlen, const int32_t* ids, int n, sw4_alignment* out, sw4_stats* stats) {
+        const std::vector<size_t> local = alignmentPairs(query, qlen, ids, n, out);
+        if (stats) memset(stats, 0, sizeof(*stats));
+        if (n == 0) return;
+        int launches = 0;
+        double cells = 0;
+        CoordState& cs = coordQuery(query, qlen, launches);
+        coordPasses(cs, qlen, local, out, cells, launches);
+        coordStats(cs, cells, launches, stats);
+    }
+
+    // ---- alignment traceback: the columns of the alignment that sw4_alignment_coordinates locates ----
+    // After the coordinate passes, the pairs with a positive score are chunked again by their trace scratch (subject
+    // slice, border columns, 4-bit direction words, rows + cols op bytes, counts) under max_temp_bytes. Each chunk runs
+    // pass 3 and the walk and copies the ops and counts back: one host synchronisation per chunk.
+    void alignmentTraceback(const char* query, int qlen, const int32_t* ids, int n, sw4_alignment_summary* out, sw4_stats* stats) {
+        lastCigars.clear();
+        const std::vector<size_t> local = alignmentPairs(query, qlen, ids, n, out);
+        if (stats) memset(stats, 0, sizeof(*stats));
+        if (n == 0) return;
+        int launches = 0;
+        double cells = 0;
+        CoordState& cs = coordQuery(query, qlen, launches);
+        std::vector<sw4_alignment> coords((size_t)n);
+        coordPasses(cs, qlen, local, coords.data(), cells, launches);
+        cudaStream_t st = cs.stream;
+
+        std::vector<int> traced;
+        for (int i = 0; i < n; i++) {
+            out[i] = sw4_alignment_summary{};
+            out[i].coordinates = coords[i];
+            if (coords[i].score > 0) traced.push_back(i);
         }
+        auto rowsOf = [&](int i) { return coords[i].query_end - coords[i].query_begin + 1; };
+        auto colsOf = [&](int i) { return coords[i].reference_end - coords[i].reference_begin + 1; };
+        auto tilesOf = [](int cols) { return (cols + kCoordTileCols - 1) / kCoordTileCols; };
+        auto warpsOf = [&](int i) {  // the form of pass 3, from the rectangle
+            const int tiles = tilesOf(colsOf(i));
+            return (tiles > 1 && (long long)rowsOf(i) * colsOf(i) >= kCoordCtaMinCells) ? std::min(tiles, kCoordWarps) : 1;
+        };
+        auto borderOf = [&](int i) {  // int2 entries
+            return tilesOf(colsOf(i)) > 1 ? (size_t)warpsOf(i) * alignUp((size_t)rowsOf(i), 32) : 0;
+        };
+        auto wordsOf = [&](int i) { return (size_t)tilesOf(colsOf(i)) * ((size_t)rowsOf(i) + 31) * 32; };
+        auto opsOf = [&](int i) { return alignUp((size_t)rowsOf(i) + (size_t)colsOf(i), 16); };
+        auto scratchOf = [&](int i) {
+            return alignUp((size_t)colsOf(i), 16) + borderOf(i) * sizeof(int2) + wordsOf(i) * sizeof(unsigned long long) + opsOf(i) +
+                   sizeof(int4);
+        };
+        // CTA-form pairs first, then the one-warp pairs; largest rectangle first within each form
+        std::stable_sort(traced.begin(), traced.end(), [&](int a, int b) {
+            const bool ca = warpsOf(a) > 1, cb = warpsOf(b) > 1;
+            if (ca != cb) return ca;
+            return (long long)rowsOf(a) * colsOf(a) > (long long)rowsOf(b) * colsOf(b);
+        });
+
+        const size_t budget = mem.max_temp_bytes;
+        const int nt = (int)traced.size();
+        for (int pos = 0; pos < nt;) {
+            int end = pos;
+            size_t bytes = 2 * sizeof(int4);  // error counters (padded)
+            while (end < nt && bytes + scratchOf(traced[end]) <= budget) bytes += scratchOf(traced[end++]);
+            if (end == pos)
+                fail(SW4_ERR_NOMEM, "max_temp_bytes (%zu bytes) cannot hold the traceback scratch of one pair (%d x %d rectangle: %zu bytes)",
+                     budget, rowsOf(traced[pos]), colsOf(traced[pos]), scratchOf(traced[pos]) + 2 * sizeof(int4));
+            const int m = end - pos;
+            cs.hItems.ensure((size_t)m);
+            cs.hGroups.ensure((size_t)m);
+            cs.hTraceItems.ensure((size_t)m);
+            size_t subjectBytes = 0, borderEntries = 0, words = 0, opsBytes = 0;
+            int numGroups = 0;
+            for (int k = 0; k < m; k++) {
+                const int i = traced[pos + k], W = warpsOf(i);
+                CoordItem& it = cs.hItems.p[k];
+                it.subjectOffset = subjectBytes;
+                it.subjectLength = colsOf(i);
+                it.borderOffset = borderEntries;
+                TraceItem& ti = cs.hTraceItems.p[k];
+                ti.words = words;
+                ti.ops = opsBytes;
+                ti.queryBegin = coords[i].query_begin;
+                ti.rows = rowsOf(i);
+                ti.score = coords[i].score;
+                subjectBytes += alignUp((size_t)colsOf(i), 16);
+                borderEntries += borderOf(i);
+                words += wordsOf(i);
+                opsBytes += opsOf(i);
+                CoordGroup* last = numGroups ? &cs.hGroups.p[numGroups - 1] : nullptr;
+                if (W == 1 && last && last->warps == 1 && last->count < kCoordWarps) last->count++;
+                else cs.hGroups.p[numGroups++] = CoordGroup{k, 1, W};
+                cells += (double)rowsOf(i) * (double)colsOf(i);
+            }
+            cs.hSubjects.ensure(std::max<size_t>(subjectBytes, 1));
+            for (int k = 0; k < m; k++) {
+                const int i = traced[pos + k];
+                const size_t li = local[i];
+                memcpy(cs.hSubjects.p + cs.hItems.p[k].subjectOffset, db->chars + db->offsets[li] + coords[i].reference_begin,
+                       (size_t)colsOf(i));
+            }
+            // one scratch arena: subject slices | border columns | direction words | ops | counts | 2 error counters
+            // (every part is a multiple of 16 bytes)
+            const size_t borderAt = subjectBytes, wordsAt = borderAt + borderEntries * sizeof(int2);
+            const size_t opsAt = wordsAt + words * sizeof(unsigned long long), countsAt = opsAt + opsBytes;
+            const size_t errorsAt = countsAt + (size_t)m * sizeof(int4), scratchBytes = errorsAt + 2 * sizeof(int4);
+            if (scratchBytes > cs.dSubjects.n) cs.dSubjects.alloc(scratchBytes);
+            if ((size_t)m > cs.dItems.n) { cs.dItems.alloc((size_t)m); cs.dGroups.alloc((size_t)m); cs.dEnds.alloc((size_t)m); }
+            if ((size_t)m > cs.dTraceItems.n) cs.dTraceItems.alloc((size_t)m);
+            cs.hTraceOut.ensure(scratchBytes - opsAt);
+            uint8_t* arena = cs.dSubjects.p;
+            SW4_CUDA(cudaMemcpyAsync(arena, cs.hSubjects.p, subjectBytes, cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemcpyAsync(cs.dItems.p, cs.hItems.p, (size_t)m * sizeof(CoordItem), cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemcpyAsync(cs.dTraceItems.p, cs.hTraceItems.p, (size_t)m * sizeof(TraceItem), cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemcpyAsync(cs.dGroups.p, cs.hGroups.p, (size_t)numGroups * sizeof(CoordGroup), cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemsetAsync(arena + errorsAt, 0, 2 * sizeof(int), st));
+            CoordParams p{};
+            p.groups = cs.dGroups.p; p.items = cs.dItems.p; p.subjects = arena;
+            p.query = cs.dQueryCodes.p; p.qlen = qlen; p.matrix = cs.dMatrix.p; p.gop = gop; p.gex = gex;
+            p.border = reinterpret_cast<int2*>(arena + borderAt);
+            p.errors = reinterpret_cast<int*>(arena + errorsAt);
+            p.traceItems = cs.dTraceItems.p;
+            p.trace = reinterpret_cast<unsigned long long*>(arena + wordsAt);
+            p.ops = reinterpret_cast<char*>(arena + opsAt);
+            p.counts = reinterpret_cast<int4*>(arena + countsAt);
+            p.numItems = m;
+            SW4_CUDA(launch_coords_trace(p, numGroups, st));
+            SW4_CUDA(launch_coords_walk(p, st));
+            launches += 2;
+            SW4_CUDA(cudaMemcpyAsync(cs.hTraceOut.p, arena + opsAt, scratchBytes - opsAt, cudaMemcpyDeviceToHost, st));
+            SW4_CUDA(cudaStreamSynchronize(st));
+            const char* ops = cs.hTraceOut.p;
+            const int4* counts = reinterpret_cast<const int4*>(ops + (countsAt - opsAt));
+            const int* errors = reinterpret_cast<const int*>(ops + (errorsAt - opsAt));
+            if (errors[0] != 0)
+                fail(SW4_ERR_CUDA, "internal error: the traceback pass of %d pairs did not reach the anchored score", errors[0]);
+            if (errors[1] != 0) fail(SW4_ERR_CUDA, "internal error: the walk of %d pairs did not end at the begin", errors[1]);
+            for (int k = 0; k < m; k++) {
+                sw4_alignment_summary& o = out[traced[pos + k]];
+                const int4 c = counts[k];
+                o.length = c.x; o.identities = c.y; o.positives = c.z; o.gaps = c.w;
+                // the walk wrote the ops from the end: run-length encode them backwards, in query order
+                const char* r = ops + cs.hTraceItems.p[k].ops;
+                o.cigar_offset = lastCigars.size();
+                for (int e = c.x - 1; e >= 0;) {
+                    const char op = r[e];
+                    int run = 0;
+                    while (e >= 0 && r[e] == op) { run++; e--; }
+                    lastCigars += std::to_string(run);
+                    lastCigars += op;
+                }
+                o.cigar_length = lastCigars.size() - o.cigar_offset;
+            }
+            pos = end;
+        }
+        coordStats(cs, cells, launches, stats);
     }
 };
 
@@ -1787,6 +1962,21 @@ int sw4_alignment_coordinates(sw4_handle* h, const char* query, int32_t query_le
                               sw4_alignment* out, sw4_stats* stats) {
     if (!h) return SW4_ERR_INVALID;
     return guarded(h, [&] { h->eng.alignmentCoordinates(query, query_length, ids, num_ids, out, stats); });
+}
+
+int sw4_alignment_traceback(sw4_handle* h, const char* query, int32_t query_length, const int32_t* ids, int32_t num_ids,
+                            sw4_alignment_summary* out, sw4_stats* stats) {
+    if (!h) return SW4_ERR_INVALID;
+    const int rc = guarded(h, [&] { h->eng.alignmentTraceback(query, query_length, ids, num_ids, out, stats); });
+    if (rc != SW4_OK) h->eng.lastCigars.clear();
+    return rc;
+}
+
+int sw4_last_cigars(const sw4_handle* h, const char** text, size_t* length) {
+    if (!h || !text || !length) return SW4_ERR_INVALID;
+    *text = h->eng.lastCigars.c_str();
+    *length = h->eng.lastCigars.size();
+    return SW4_OK;
 }
 
 int sw4_last_scan_all_scores(sw4_handle* h, int32_t* out_scores, int32_t* out_ids, size_t capacity, size_t* out_count) {

@@ -29,6 +29,9 @@ cudaError_t launch_s16_long2(const S16Long2Params& prm, int grid, cudaStream_t s
 cudaError_t launch_s32(const S32Params& prm, int blocks, cudaStream_t stream);
 // alignment coordinates: pass 1 (ends) or pass 2 (begins), one CTA per CoordGroup
 cudaError_t launch_coords(bool reverse, const CoordParams& prm, int groups, cudaStream_t stream);
+// alignment traceback: pass 3 (directions over each rectangle, one CTA per CoordGroup), then the walk (prm.numItems pairs)
+cudaError_t launch_coords_trace(const CoordParams& prm, int groups, cudaStream_t stream);
+cudaError_t launch_coords_walk(const CoordParams& prm, cudaStream_t stream);
 
 // CTAs are launched as clusters of 2 whenever the grid is even: the two SMs of a TPC share an instruction cache, and
 // with many different (large, heavily unrolled) kernels resident at once it pays to give both SMs the same code.

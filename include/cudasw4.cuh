@@ -55,6 +55,8 @@ struct BenchmarkStats { int numOverflows{}; double seconds{}; double gcups{}; };
 struct ScanResult { std::vector<int> scores{}; std::vector<ReferenceIdT> referenceIds{}; BenchmarkStats stats{}; };
 // Extension (no reference counterpart): where a hit aligns, 0-based inclusive, -1 when score == 0 (sw4b200.h)
 struct AlignmentCoordinates { int score, queryBegin, queryEnd, referenceBegin, referenceEnd; };
+// Extension: how a hit aligns (sw4b200.h): its coordinates, counts and SAM-style CIGAR (=, X, I, D; "" when score == 0)
+struct Alignment { AlignmentCoordinates coordinates; int length, identities, positives, gaps; std::string cigar; };
 struct KernelTypeConfig {                                                                             // :88-93
     KernelType singlePassType = KernelType::Half2;
     KernelType manyPassType_small = KernelType::Half2;
@@ -184,6 +186,22 @@ public:
         std::vector<AlignmentCoordinates> out(ids.size());
         for (size_t i = 0; i < ids.size(); i++)
             out[i] = AlignmentCoordinates{raw[i].score, raw[i].query_begin, raw[i].query_end, raw[i].reference_begin, raw[i].reference_end};
+        return out;
+    }
+
+    // Extension: coordinates, CIGAR and counts of one optimal local alignment of the query against each database id.
+    std::vector<Alignment> computeAlignments(const char* query, SequenceLengthT length, const std::vector<ReferenceIdT>& ids) {
+        std::vector<sw4_alignment_summary> raw(std::max<size_t>(1, ids.size()));
+        check(sw4_alignment_traceback(handle, query, length, ids.data(), (int32_t)ids.size(), raw.data(), nullptr));
+        const char* text = nullptr; size_t textLength = 0;
+        check(sw4_last_cigars(handle, &text, &textLength));
+        std::vector<Alignment> out(ids.size());
+        for (size_t i = 0; i < ids.size(); i++) {
+            const sw4_alignment& c = raw[i].coordinates;
+            out[i] = Alignment{AlignmentCoordinates{c.score, c.query_begin, c.query_end, c.reference_begin, c.reference_end},
+                               raw[i].length, raw[i].identities, raw[i].positives, raw[i].gaps,
+                               std::string(text + raw[i].cigar_offset, raw[i].cigar_length)};
+        }
         return out;
     }
 

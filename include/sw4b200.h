@@ -175,6 +175,51 @@ typedef struct sw4_alignment {
 int sw4_alignment_coordinates(sw4_handle* h, const char* query, int32_t query_length, const int32_t* ids, int32_t num_ids,
                               sw4_alignment* out, sw4_stats* stats);
 
+/* How each hit aligns (no reference counterpart): the coordinates of sw4_alignment_coordinates, and the columns of the
+ * one alignment they locate, traced back on the same GPU.
+ *
+ * The reported alignment is the one that sw4_alignment_coordinates locates: it starts with the pair (qb, rb), ends
+ * with the pair (qe, re) and scores S. When several alignments qualify, this rule picks exactly one.
+ * Over the rectangle, use the anchored recurrences started at (qb, rb):
+ *   P is the pair state.
+ *   E is a gap column that consumes a reference residue only. Its CIGAR op is D.
+ *   F is a gap column that consumes a query residue only. Its CIGAR op is I.
+ *   X = max(P, E, F).
+ *   E(i,j) = max(X(i,j-1) + gop, E(i,j-1) + gex), and F likewise along i.
+ * Walk back from (qe, re) in state P:
+ *   In P at (i, j): emit the pair (= if the two residue codes are equal, else X). Unless this is (qb, rb), step to
+ *     (i-1, j-1) and take the first state of P, E, F whose value equals X(i-1, j-1).
+ *   In E at (i, j): emit D. Step to (i, j-1). If E(i,j-1) + gex == E(i,j), extend: stay in E. Extend wins a tie.
+ *     Otherwise open: take the first of P, E, F equal to X(i, j-1).
+ *   In F: do the same along i, emitting I.
+ * The walk ends at (qb, rb) in state P. Score 0 gives coordinates of -1, an empty CIGAR and zero counts.
+ *
+ * Per hit, report the coordinates (identical to sw4_alignment_coordinates), the CIGAR and four counts:
+ *   CIGAR: run-length ops =, X, I, D, in query order. I consumes the query only and D the reference only, as in SAM
+ *     with the query as the read.
+ *   length: the number of columns.
+ *   identities: the number of = columns. These compare residue codes, so every non-standard letter counts as code 20.
+ *   positives: pairs with a substitution score > 0.
+ *   gaps: I + D columns.
+ * A CIGAR rescores as follows. A pair scores M[q][r]. A maximal run of k gap columns of one kind scores
+ * gop + (k-1) * max(gop, gex). Adjacent I and D runs each pay their own open. This is what the Gotoh recurrence
+ * computes: H includes E, so when gop > gex (for example 0 / -4096) a gap is "re-opened" rather than extended.
+ * Rescoring every CIGAR gives exactly S.
+ *
+ * Arguments, errors and chunking are those of sw4_alignment_coordinates; the traceback chunks the pairs again by their
+ * trace scratch (about half a byte per cell of the rectangle plus rows + columns bytes; DESIGN.md 3.7), and a single
+ * rectangle that does not fit max_temp_bytes is SW4_ERR_NOMEM. stats may be NULL: seconds is device-timed, cells
+ * counts all three passes, kernel_launches every kernel. */
+typedef struct sw4_alignment_summary {
+    sw4_alignment coordinates;          /* == sw4_alignment_coordinates for this id */
+    int32_t length, identities, positives, gaps;
+    size_t cigar_offset, cigar_length;  /* into the text of sw4_last_cigars */
+} sw4_alignment_summary;
+int sw4_alignment_traceback(sw4_handle* h, const char* query, int32_t query_length, const int32_t* ids,
+                            int32_t num_ids, sw4_alignment_summary* out, sw4_stats* stats);
+/* CIGAR text of the last sw4_alignment_traceback on this handle; valid until the next call or sw4_destroy */
+int sw4_last_cigars(const sw4_handle* h, const char** text, size_t* length);
+
 /* Debug / parity helper (the reference's CUDASW_DEBUG_CHECK_CORRECTNESS mode sets numTop to the whole database,
  * src/cudasw4.cuh:505-507): all scores of the last scan for this handle's shard, plus their global ids, in shard
  * order. capacity is in entries; returns the number written in *out_count. */
