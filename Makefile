@@ -39,7 +39,7 @@ variant:
 	@cat build/variants/$(NAME)/*.ptxas.log | grep -E "spill" | grep -v " 0 bytes spill stores, 0 bytes spill loads" | sort | uniq -c | sort -rn | head -8 || true
 
 cli: build/align build/makedb
-build/align: $(CSRC)/cli_align.cpp include/cudasw4.cuh include/sw4b200.h $(CSRC)/fasta_reader.hpp $(LIB)
+build/align: $(CSRC)/cli_align.cpp include/cudasw4.cuh include/sw4b200.h $(CSRC)/fasta_reader.hpp $(CSRC)/blosum_tables.hpp $(LIB)
 	@mkdir -p build
 	$(CXXHOST) -std=c++17 -O2 -Wall -Iinclude -o $@ $(CSRC)/cli_align.cpp -Lcudasw4_b200 -lsw4b200 -Wl,-rpath,'$$ORIGIN/../cudasw4_b200' -lz
 build/makedb: $(CSRC)/cli_makedb.cpp $(CSRC)/fasta_reader.hpp

@@ -85,6 +85,23 @@ class Alignments:
     cigars: list
 
 
+def _pssm_array(pssm, length: int) -> np.ndarray:
+    """A (length, 21) position-specific scoring matrix as a contiguous int8 array (row p: the scores of query position p
+    against residue codes 0..19 = ARNDCQEGHILKMFPSTWYV and 20 = any other letter). Refuses a wrong shape, a non-integer
+    array, values outside the int8 range and a positive column 20 (code 20 also pads the subjects on the device, see
+    include/sw4b200.h) with ValueError; values are never wrapped."""
+    a = np.asarray(pssm)
+    if a.ndim != 2 or a.shape != (length, 21):
+        raise ValueError(f"pssm must have shape ({length}, 21) for a query of {length} residues, got {a.shape}")
+    if a.size and not (np.issubdtype(a.dtype, np.integer) or np.issubdtype(a.dtype, np.bool_)):
+        raise ValueError(f"pssm must hold integers, got {a.dtype}")
+    if a.size and (int(a.min()) < -128 or int(a.max()) > 127):
+        raise ValueError(f"pssm values must lie in [-128, 127], got [{int(a.min())}, {int(a.max())}]")
+    if a.size and int(a[:, 20].max()) > 0:
+        raise ValueError(f"pssm column 20 (any other letter) must be <= 0, got {int(a[:, 20].max())}")
+    return np.ascontiguousarray(a, dtype=np.int8)
+
+
 def _stats(s: _lib.Stats) -> BenchmarkStats:
     return BenchmarkStats(int(s.num_overflows), float(s.seconds), float(s.gcups), float(s.kernel_seconds),
                           float(s.cells), int(s.kernel_launches))
@@ -225,8 +242,10 @@ class CudaSW4:
         self._check(self._lib.sw4_upload_database(self._h))
 
     # -- the hot path (reference src/cudasw4.cuh:698-765) ---------------------------------------------------------
-    def scan(self, query, length: int | None = None) -> ScanResult:
-        """query: residue letters (str/bytes). Returns the top-`numTop` (score, reference id) pairs."""
+    def scan(self, query, length: int | None = None, pssm=None) -> ScanResult:
+        """query: residue letters (str/bytes). Returns the top-`numTop` (score, reference id) pairs.
+        pssm: a (length, 21) integer array scoring each query position against each residue code instead of the
+        handle's matrix (include/sw4b200.h); the letters then only serve the identities of alignments()."""
         q = query.encode() if isinstance(query, str) else bytes(query)
         n = len(q) if length is None else int(length)
         k = max(self.numTop, 1)
@@ -234,16 +253,26 @@ class CudaSW4:
         ids = np.empty(k, dtype=np.int32)
         count = ctypes.c_int32(0)
         st = _lib.Stats()
-        self._check(self._lib.sw4_scan(self._h, q, n, scores.ctypes.data, ids.ctypes.data, ctypes.byref(count),
-                                       ctypes.byref(st)))
+        if pssm is None:
+            self._check(self._lib.sw4_scan(self._h, q, n, scores.ctypes.data, ids.ctypes.data, ctypes.byref(count),
+                                           ctypes.byref(st)))
+        else:
+            p = _pssm_array(pssm, n)
+            self._check(self._lib.sw4_scan_pssm(self._h, q, p.ctypes.data, n, scores.ctypes.data, ids.ctypes.data,
+                                                ctypes.byref(count), ctypes.byref(st)))
         c = int(count.value)
         return ScanResult(scores[:c].tolist(), ids[:c].tolist(), _stats(st))
 
-    def scanMany(self, queries):
+    def scanMany(self, queries, pssm=None):
         """Query batching (sw4_scan_many): all `queries` (letters) with several scans in flight per GPU. Returns
-        (list of ScanResult in query order, BenchmarkStats of the whole call: device-timed span, total GCUPS)."""
+        (list of ScanResult in query order, BenchmarkStats of the whole call: device-timed span, total GCUPS).
+        pssm: a list of (len(query), 21) arrays, one per query (as scan's pssm)."""
         qs = [q.encode() if isinstance(q, str) else bytes(q) for q in queries]
         nq = len(qs)
+        if pssm is not None:
+            if len(pssm) != nq:
+                raise ValueError(f"one pssm per query: {len(pssm)} for {nq} queries")
+            ps = [_pssm_array(p, len(q)) for p, q in zip(pssm, qs)]
         k = max(self.numTop, 1)
         arr = (ctypes.c_char_p * max(nq, 1))(*qs)
         lens = (ctypes.c_int32 * max(nq, 1))(*[len(q) for q in qs])
@@ -252,19 +281,25 @@ class CudaSW4:
         counts = np.zeros(max(nq, 1), dtype=np.int32)
         per = (_lib.Stats * max(nq, 1))()
         total = _lib.Stats()
-        self._check(self._lib.sw4_scan_many(self._h, arr, lens, nq, scores.ctypes.data, ids.ctypes.data, counts.ctypes.data,
-                                            per, ctypes.byref(total)))
+        if pssm is None:
+            self._check(self._lib.sw4_scan_many(self._h, arr, lens, nq, scores.ctypes.data, ids.ctypes.data,
+                                                counts.ctypes.data, per, ctypes.byref(total)))
+        else:
+            parr = (ctypes.c_void_p * max(nq, 1))(*[p.ctypes.data for p in ps])
+            self._check(self._lib.sw4_scan_many_pssm(self._h, arr, parr, lens, nq, scores.ctypes.data, ids.ctypes.data,
+                                                     counts.ctypes.data, per, ctypes.byref(total)))
         out = []
         for i in range(nq):
             c = int(counts[i]) if self.numTop > 0 else 0
             out.append(ScanResult(scores[i, :c].tolist(), ids[i, :c].tolist(), _stats(per[i])))
         return out, _stats(total)
 
-    def alignmentCoordinates(self, query, ids, stats: BenchmarkStats | None = None) -> np.ndarray:
+    def alignmentCoordinates(self, query, ids, stats: BenchmarkStats | None = None, pssm=None) -> np.ndarray:
         """Where each hit aligns: for every database id in `ids`, one row (score, query_begin, query_end,
         reference_begin, reference_end) of an int32 array of shape (len(ids), 5). Positions are 0-based and inclusive,
         -1 when the score is 0; the end is the first cell holding the maximum, the begin that of the shortest optimal
-        alignment ending there (include/sw4b200.h). `stats`, when given, receives the call's device-timed figures."""
+        alignment ending there (include/sw4b200.h). `stats`, when given, receives the call's device-timed figures.
+        pssm: a (len(query), 21) array, as scan's."""
         q = query.encode() if isinstance(query, str) else bytes(query)
         idv = np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1))
         if len(idv) and (idv.min() < -2**31 or idv.max() >= 2**31):
@@ -272,17 +307,23 @@ class CudaSW4:
         idv = idv.astype(np.int32)
         out = np.empty((max(len(idv), 1), 5), dtype=np.int32)
         st = _lib.Stats()
-        self._check(self._lib.sw4_alignment_coordinates(self._h, q, len(q), idv.ctypes.data, len(idv), out.ctypes.data,
-                                                        ctypes.byref(st)))
+        if pssm is None:
+            self._check(self._lib.sw4_alignment_coordinates(self._h, q, len(q), idv.ctypes.data, len(idv), out.ctypes.data,
+                                                            ctypes.byref(st)))
+        else:
+            p = _pssm_array(pssm, len(q))
+            self._check(self._lib.sw4_alignment_coordinates_pssm(self._h, q, p.ctypes.data, len(q), idv.ctypes.data, len(idv),
+                                                                 out.ctypes.data, ctypes.byref(st)))
         if stats is not None:
             for k, v in vars(_stats(st)).items():
                 setattr(stats, k, v)
         return out[:len(idv)].copy()
 
-    def alignments(self, query, ids, stats: BenchmarkStats | None = None) -> Alignments:
+    def alignments(self, query, ids, stats: BenchmarkStats | None = None, pssm=None) -> Alignments:
         """How each hit aligns: the coordinates of alignmentCoordinates, and the CIGAR and counts of the one alignment
         they locate, traced back on the GPU (the rule is in include/sw4b200.h). `stats`, when given, receives the
-        call's device-timed figures (cells and kernel launches of all three passes)."""
+        call's device-timed figures (cells and kernel launches of all three passes). pssm: a (len(query), 21) array, as
+        scan's; positives are then the pairs it scores above 0."""
         q = query.encode() if isinstance(query, str) else bytes(query)
         idv = np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1))
         if len(idv) and (idv.min() < -2**31 or idv.max() >= 2**31):
@@ -291,7 +332,12 @@ class CudaSW4:
         n = len(idv)
         out = (_lib.AlignmentSummary * max(n, 1))()
         st = _lib.Stats()
-        self._check(self._lib.sw4_alignment_traceback(self._h, q, len(q), idv.ctypes.data, n, out, ctypes.byref(st)))
+        if pssm is None:
+            self._check(self._lib.sw4_alignment_traceback(self._h, q, len(q), idv.ctypes.data, n, out, ctypes.byref(st)))
+        else:
+            p = _pssm_array(pssm, len(q))
+            self._check(self._lib.sw4_alignment_traceback_pssm(self._h, q, p.ctypes.data, len(q), idv.ctypes.data, n, out,
+                                                               ctypes.byref(st)))
         p = ctypes.c_void_p()
         size = ctypes.c_size_t(0)
         self._check(self._lib.sw4_last_cigars(self._h, ctypes.byref(p), ctypes.byref(size)))

@@ -14,7 +14,8 @@ EXPORTS = [
     "sw4_last_scan_all_scores", "sw4_reference_header",
     "sw4_reference_length", "sw4_reference_sequence", "sw4_total_timer_start", "sw4_total_timer_stop",
     "sw4_get_db_info", "sw4_version", "sw4_alignment_coordinates",
-    "sw4_alignment_traceback", "sw4_last_cigars",
+    "sw4_alignment_traceback", "sw4_last_cigars", "sw4_scan_pssm", "sw4_scan_many_pssm", "sw4_alignment_coordinates_pssm",
+    "sw4_alignment_traceback_pssm",
 ]
 
 
@@ -82,6 +83,14 @@ def load() -> ctypes.CDLL:
                                               ctypes.POINTER(Stats)]
     lib.sw4_alignment_traceback.argtypes = [vp, ctypes.c_char_p, ctypes.c_int32, vp, ctypes.c_int32, vp,
                                             ctypes.POINTER(Stats)]
+    lib.sw4_scan_pssm.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_int32, vp, vp, ctypes.POINTER(ctypes.c_int32),
+                                  ctypes.POINTER(Stats)]
+    lib.sw4_scan_many_pssm.argtypes = [vp, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(vp), ctypes.POINTER(ctypes.c_int32),
+                                       ctypes.c_int32, vp, vp, vp, ctypes.POINTER(Stats), ctypes.POINTER(Stats)]
+    lib.sw4_alignment_coordinates_pssm.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_int32, vp, ctypes.c_int32, vp,
+                                                   ctypes.POINTER(Stats)]
+    lib.sw4_alignment_traceback_pssm.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_int32, vp, ctypes.c_int32, vp,
+                                                 ctypes.POINTER(Stats)]
     lib.sw4_last_cigars.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(cs)]
     lib.sw4_last_scan_all_scores.argtypes = [vp, vp, vp, cs, ctypes.POINTER(cs)]
     lib.sw4_reference_header.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(vp), ctypes.POINTER(cs)]

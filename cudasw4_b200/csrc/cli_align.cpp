@@ -3,6 +3,9 @@
 // (include/cudasw4.cuh -> C ABI -> libsw4b200.so). The GPUs used are all visible ones (CUDA_VISIBLE_DEVICES).
 // Unlike the shipped reference binary, --gop/--gex (and the per-matrix defaults) really reach the kernels
 // (SURVEY.md 0-1), and the database is always uploaded in full (--uploadFull is accepted and implied).
+#include <algorithm>
+#include <cctype>
+#include <cerrno>
 #include <cstdlib>
 #include <fstream>
 #include <iostream>
@@ -11,6 +14,7 @@
 #include <string>
 #include <vector>
 
+#include "blosum_tables.hpp"
 #include "cudasw4.cuh"
 #include "fasta_reader.hpp"
 
@@ -29,7 +33,69 @@ struct Options {
     Output output = Output::Plain;
     std::string outfile = "/dev/stdout", db;
     std::vector<std::string> queries;
+    std::vector<std::string> pssmFiles;  // extension: --pssm, PSI-BLAST ASCII PSSM files (one query each)
 };
+
+// One PSSM query: the residue letters of its rows and the [length][21] scores (column 20: the --mat table's `low`).
+struct PssmQuery {
+    std::string path, letters;
+    std::vector<std::int8_t> scores;
+};
+
+// PSI-BLAST's ASCII PSSM (-out_ascii_pssm). The header line starts with the 20 letters A R N D C Q E G H I L K M F P S T
+// W Y V in this order. Each row that follows is "pos letter s1 ... s20 ...", positions 1, 2, ... without gaps; tokens
+// after the 20 scores are ignored. The first line that is not a row ends the matrix.
+PssmQuery readAsciiPssm(const std::string& path, int low) {
+    std::ifstream in(path);
+    if (!in) throw std::runtime_error("cannot open PSSM file " + path);
+    static const char* kOrder = "ARNDCQEGHILKMFPSTWYV";
+    auto bad = [&](const std::string& why) { return std::runtime_error("PSSM file " + path + ": " + why); };
+    auto integer = [](const std::string& t, long& v) {
+        if (t.empty()) return false;
+        char* end = nullptr;
+        errno = 0;
+        v = std::strtol(t.c_str(), &end, 10);
+        return *end == '\0' && errno == 0;
+    };
+    PssmQuery q;
+    q.path = path;
+    std::string line;
+    bool header = false;
+    while (std::getline(in, line)) {  // the header: the first line that starts with 20 one-letter tokens
+        std::istringstream ls(line);
+        std::vector<std::string> t;
+        for (std::string w; ls >> w;) t.push_back(w);
+        if (t.size() < 20 || !std::all_of(t.begin(), t.begin() + 20, [](const std::string& w) {
+                return w.size() == 1 && std::isalpha((unsigned char)w[0]);
+            }))
+            continue;
+        for (int k = 0; k < 20; k++)
+            if (t[k] != std::string(1, kOrder[k])) throw bad("the header's residue order is not A R N D C Q E G H I L K M F P S T W Y V");
+        header = true;
+        break;
+    }
+    if (!header) throw bad("no header line with the residue letters");
+    while (std::getline(in, line)) {
+        std::istringstream ls(line);
+        std::vector<std::string> t;
+        for (std::string w; ls >> w;) t.push_back(w);
+        long pos = 0;
+        if (t.empty() || !integer(t[0], pos)) break;  // not a row: the end of the matrix
+        const long want = (long)q.letters.size() + 1;
+        if (pos != want) throw bad("row " + t[0] + " where row " + std::to_string(want) + " was expected");
+        if (t.size() < 22 || t[1].size() != 1) throw bad("row " + t[0] + " is not 'position letter' and 20 scores");
+        q.letters.push_back(t[1][0]);
+        for (int k = 0; k < 20; k++) {
+            long v = 0;
+            if (!integer(t[2 + k], v)) throw bad("row " + t[0] + ": score '" + t[2 + k] + "' is not an integer");
+            if (v < -128 || v > 127) throw bad("row " + t[0] + ": score " + t[2 + k] + " is outside [-128, 127]");
+            q.scores.push_back((std::int8_t)v);
+        }
+        q.scores.push_back((std::int8_t)low);
+    }
+    if (q.letters.empty()) throw bad("no rows");
+    return q;
+}
 
 size_t parseMemory(const std::string& s) {
     if (s.empty()) return 0;
@@ -75,6 +141,7 @@ bool parseArgs(int argc, char** argv, Options& o) {
         else if (a == "--maxTempBytes") o.mem.maxTempBytes = parseMemory(need(i));
         else if (a == "--maxGpuMem") o.mem.maxGpuMem = parseMemory(need(i));
         else if (a == "--query") { o.queries.push_back(need(i)); gotQuery = true; }
+        else if (a == "--pssm") o.pssmFiles.push_back(need(i));
         else if (a == "--db") { o.db = need(i); gotDB = true; }
         else if (a == "--mat") {
             const std::string v = need(i);
@@ -107,7 +174,8 @@ bool parseArgs(int argc, char** argv, Options& o) {
         o.kernels.manyPassType_large = cudasw4::KernelType::DPXs32;
         o.kernels.overflowType = cudasw4::KernelType::DPXs32;
     }
-    if (!gotQuery && !o.interactive) { std::cout << "Query is missing\n"; return false; }
+    if (gotQuery && !o.pssmFiles.empty()) throw std::runtime_error("--query and --pssm cannot be combined");
+    if (!gotQuery && o.pssmFiles.empty() && !o.interactive) { std::cout << "Query is missing\n"; return false; }
     if (!gotDB) { std::cout << "DB prefix is missing\n"; return false; }
     return true;
 }
@@ -116,6 +184,8 @@ void printHelp(const char* prog) {
     std::cout << "Usage: " << prog << " [options]\n"
               << "The GPUs to use are set via CUDA_VISIBLE_DEVICES environment variable.\n"
               << "   --query queryfile : Mandatory. Fasta or Fastq, may be gzip'ed. Repeatable.\n"
+              << "   --pssm file : (extension) instead of --query: a PSI-BLAST ASCII PSSM (-out_ascii_pssm) scores the query.\n"
+              << "                 Repeatable; the files are numbered as the queries of one query file.\n"
               << "   --db dbPrefix : Mandatory. The same dbPrefix as used for makedb\n"
               << "   --top val : Output the val best scores. Default 10\n"
               << "   --gop val, --gex val : Gap open / extend score. Overwrite the blosum-dependent defaults.\n"
@@ -140,6 +210,7 @@ void printOptions(const Options& o) {
               << "maxBatchBytes: " << o.mem.maxBatchBytes << "\n" << "maxBatchSequences: " << o.mem.maxBatchSequences << "\n"
               << "maxTempBytes: " << o.mem.maxTempBytes << "\n";
     for (size_t i = 0; i < o.queries.size(); i++) std::cout << "queryFile " << i << " : " << o.queries[i] << "\n";
+    for (size_t i = 0; i < o.pssmFiles.size(); i++) std::cout << "pssmFile " << i << " : " << o.pssmFiles[i] << "\n";
     std::cout << "blosum: " << cudasw4::to_string_nodim(o.blosum) << "\n"
               << "singlePassType: " << cudasw4::to_string(o.kernels.singlePassType) << "\n"
               << "manyPassType_small: " << cudasw4::to_string(o.kernels.manyPassType_small) << "\n"
@@ -201,41 +272,46 @@ void printTSV(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::Cud
     }
 }
 
+// (pssm: the query's [length][21] scores, or nullptr for a sequence query)
 void reportQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
-                 const std::string& sequence, const cudasw4::ScanResult& r);
+                 const std::string& sequence, const std::int8_t* pssm, const cudasw4::ScanResult& r);
 
 void processQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
-                  const std::string& sequence) {
+                  const std::string& sequence, const std::int8_t* pssm = nullptr) {
     std::cout << "Processing query " << qnum << " ... ";
     std::cout.flush();
-    cudasw4::ScanResult r = sw.scan(sequence.data(), (int)sequence.size());
-    reportQuery(o, sw, out, qnum, header, sequence, r);
+    cudasw4::ScanResult r = pssm ? sw.scan(sequence.data(), pssm, (int)sequence.size()) : sw.scan(sequence.data(), (int)sequence.size());
+    reportQuery(o, sw, out, qnum, header, sequence, pssm, r);
 }
 
 // --batchQueries: the queries go through one scanMany call; output is written in query order exactly as above
+// (pssms: empty for sequence queries, else one per query)
 void processQueryBatch(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t firstQnum,
-                       const std::vector<std::string>& headers, const std::vector<std::string>& sequences) {
+                       const std::vector<std::string>& headers, const std::vector<std::string>& sequences,
+                       const std::vector<const std::int8_t*>& pssms = {}) {
     std::vector<std::string_view> views(sequences.begin(), sequences.end());
-    const std::vector<cudasw4::ScanResult> results = sw.scanMany(views);
+    const std::vector<cudasw4::ScanResult> results = pssms.empty() ? sw.scanMany(views) : sw.scanMany(views, pssms);
     for (size_t i = 0; i < results.size(); i++) {
         std::cout << "Processing query " << firstQnum + (int64_t)i << " ... ";
-        reportQuery(o, sw, out, firstQnum + (int64_t)i, headers[i], sequences[i], results[i]);
+        reportQuery(o, sw, out, firstQnum + (int64_t)i, headers[i], sequences[i], pssms.empty() ? nullptr : pssms[i], results[i]);
     }
 }
 
 void reportQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
-                 const std::string& sequence, const cudasw4::ScanResult& r) {
+                 const std::string& sequence, const std::int8_t* pssm, const cudasw4::ScanResult& r) {
     if (o.verbose) std::cout << "Done. Scan time: " << r.stats.seconds << " s, " << r.stats.gcups << " GCUPS\n";
     else std::cout << "Done.\n";
     if (o.top > 0) {
         std::vector<cudasw4::AlignmentCoordinates> coords;
         std::vector<cudasw4::Alignment> alignments;
         if (o.cigar && !r.referenceIds.empty()) {  // the traceback reports the coordinates too
-            alignments = sw.computeAlignments(sequence.data(), (int)sequence.size(), r.referenceIds);
+            alignments = pssm ? sw.computeAlignments(sequence.data(), pssm, (int)sequence.size(), r.referenceIds)
+                              : sw.computeAlignments(sequence.data(), (int)sequence.size(), r.referenceIds);
             if (o.coordinates)
                 for (const auto& a : alignments) coords.push_back(a.coordinates);
         } else if (o.coordinates && !r.referenceIds.empty()) {
-            coords = sw.computeAlignmentCoordinates(sequence.data(), (int)sequence.size(), r.referenceIds);
+            coords = pssm ? sw.computeAlignmentCoordinates(sequence.data(), pssm, (int)sequence.size(), r.referenceIds)
+                          : sw.computeAlignmentCoordinates(sequence.data(), (int)sequence.size(), r.referenceIds);
         }
         if (o.output == Options::Output::Plain) {
             out << "Query " << qnum << ", header" << header << ", length " << sequence.size() << ", num overflows "
@@ -254,6 +330,14 @@ int main(int argc, char** argv) {
     Options o;
     try {
         if (!parseArgs(argc, argv, o) || o.help) { printHelp(argv[0]); return 0; }
+        // every PSSM file is read before any GPU work, so that a malformed one fails at once
+        std::vector<PssmQuery> pssmQueries;
+        for (const auto& f : o.pssmFiles) {
+            int low = 0;
+            for (const auto& t : sw4::kSubstitutionTriangles)
+                if (t.id == cudasw4::blosumNumber(o.blosum)) low = t.low;
+            pssmQueries.push_back(readAsciiPssm(f, low));
+        }
         printOptions(o);
         std::ofstream out(o.outfile);
         if (!out) throw std::runtime_error("Cannot open file " + o.outfile);
@@ -275,7 +359,28 @@ int main(int argc, char** argv) {
         }
         sw.prefetchDBToGpus();
 
-        if (!o.interactive) {
+        if (!o.pssmFiles.empty()) {  // the PSSM files are the queries of one query file, header = the path
+            std::cout << "Processing PSSM queries\n";
+            sw.totalTimerStart();
+            for (size_t q0 = 0; q0 < pssmQueries.size(); q0 += (size_t)o.batchQueries) {
+                const size_t q1 = std::min(pssmQueries.size(), q0 + (size_t)o.batchQueries);
+                if (o.batchQueries <= 1) {
+                    const PssmQuery& q = pssmQueries[q0];
+                    processQuery(o, sw, out, (int64_t)q0, q.path, q.letters, q.scores.data());
+                    continue;
+                }
+                std::vector<std::string> headers, sequences;
+                std::vector<const std::int8_t*> pssms;
+                for (size_t i = q0; i < q1; i++) {
+                    headers.push_back(pssmQueries[i].path);
+                    sequences.push_back(pssmQueries[i].letters);
+                    pssms.push_back(pssmQueries[i].scores.data());
+                }
+                processQueryBatch(o, sw, out, (int64_t)q0, headers, sequences, pssms);
+            }
+            const auto total = sw.totalTimerStop();
+            if (o.verbose) std::cout << "Total time: " << total.seconds << " s, " << total.gcups << " GCUPS\n";
+        } else if (!o.interactive) {
             for (const auto& qf : o.queries) {
                 std::cout << "Processing query file " << qf << "\n";
                 sw4::SequenceFileReader reader(qf);

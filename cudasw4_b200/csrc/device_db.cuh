@@ -30,28 +30,43 @@ __global__ void convert_query_kernel(const char* __restrict__ letters, uint8_t* 
     codes[i] = c;
 }
 
-__global__ void build_profile_kernel(const uint8_t* __restrict__ qcodes, int qlen, const int8_t* __restrict__ matrix,
-                                     uint32_t* __restrict__ profile, int stride) {
+// Entry (f, p) of the profile. `scores` holds the 21 scores of query position p against residue codes 0..20: the
+// matrix row of its residue code (sequence query) or row p of a position-specific scoring matrix (PSSM query).
+template <bool PSSM>
+__device__ __forceinline__ void build_profile_entry(const uint8_t* __restrict__ qcodes, int qlen, const int8_t* __restrict__ scores,
+                                                    uint32_t* __restrict__ profile, int stride) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     const int f = blockIdx.y;  // fused pair: s0 = f % 21 (low half), s1 = f / 21 (high half)
     if (p >= stride) return;
+    // (only for p < qlen) the first of the 21 scores, as an index into `scores`
+    auto base = [&] { return (PSSM ? p : (int)qcodes[p]) * 21; };
     uint32_t v = 0xc180c180u;  // (-16000, -16000)
     if (f >= 483) {
-        // rows 483..503: plain int32 plane for the exact 32-bit array kernel (sw_s32_long_kernel)
-        v = p < qlen ? (uint32_t)(int32_t)matrix[qcodes[p] * 21 + (f - 483)] : (uint32_t)(-(1 << 28));
+        // rows 483..503: plain int32 plane for the exact 32-bit kernels (sw_s32_long_kernel, and sw_s32_kernel's PSSM form)
+        v = p < qlen ? (uint32_t)(int32_t)scores[base() + (f - 483)] : (uint32_t)(-(1 << 28));
     } else if (f >= 441) {
         // rows 441..461: single-residue plane with the score in the low half, rows 462..482: the same in the high half
         // (sw_s16_long_kernel adds one entry of each)
         const int s = (f - 441) % 21;
         const bool high = f >= 462;
-        const uint32_t m = p < qlen ? (uint32_t)(uint16_t)(int16_t)matrix[qcodes[p] * 21 + s] : 0xc180u;
+        const uint32_t m = p < qlen ? (uint32_t)(uint16_t)(int16_t)scores[base() + s] : 0xc180u;
         v = high ? (m << 16) : m;
     } else if (p < qlen) {
-        const int qc = qcodes[p];
-        const int lo = matrix[qc * 21 + f % 21], hi = matrix[qc * 21 + f / 21];
+        const int b = base();
+        const int lo = scores[b + f % 21], hi = scores[b + f / 21];
         v = ((uint32_t)(uint16_t)(int16_t)hi << 16) | (uint16_t)(int16_t)lo;
     }
     profile[(size_t)f * stride + p] = v;
+}
+
+__global__ void build_profile_kernel(const uint8_t* __restrict__ qcodes, int qlen, const int8_t* __restrict__ matrix,
+                                     uint32_t* __restrict__ profile, int stride) {
+    build_profile_entry<false>(qcodes, qlen, matrix, profile, stride);
+}
+
+// the profile of a PSSM query: pssm is [qlen][21], row p scoring query position p against residue codes 0..20
+__global__ void build_profile_pssm_kernel(const int8_t* __restrict__ pssm, int qlen, uint32_t* __restrict__ profile, int stride) {
+    build_profile_entry<true>(nullptr, qlen, pssm, profile, stride);
 }
 
 // Work items of a single-segment length class, generated on the device: consecutive subjects [first, first+count) are

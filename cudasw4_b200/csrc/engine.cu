@@ -258,11 +258,16 @@ struct Ctx {
     DevBuf<unsigned long long> dTopkKeys;
     PinnedBuf<char> hQuery;
     PinnedBuf<int32_t> hTop;        // scores[k], ids[k], counters[8]
+    // a PSSM query's [qlen][21] table (allocated by the first PSSM query, grown with queryCapacity)
+    PinnedBuf<int8_t> hPssm;
+    DevBuf<int8_t> dPssm;
     int queryCapacity = 0;
     size_t topCapacity = 0;
     // the query in flight
     bool busy = false;
     int queryIndex = -1, qlen = 0, k = 0, profStride = 0, launches = 0;
+    bool pssm = false;
+    int maxEntry = 1;  // largest score of one residue pair (at least 1): bounds the scores by maxEntry * min(qlen, len)
     bool largeK = false;
 
     void create() {
@@ -362,7 +367,27 @@ static inline int s16Period(int qlen, int G) { return std::max(16, ((qlen + 1) /
 // the wide variant advances one row per step: q + G - 1 rounded up to 8, at least 32
 static inline int s16WidePeriod(int qlen, int G) { return std::max(32, (qlen + G - 1 + 7) / 8 * 8); }
 
-struct QueryRef { const char* letters; int length; };
+// pssm: nullptr for a sequence query; otherwise the query's [length][21] position-specific scores (the letters then
+// only serve the identities of the traceback)
+struct QueryRef { const char* letters; int length; const int8_t* pssm = nullptr; };
+
+// the largest entry of a [qlen][21] PSSM, at least 1 (the bound of sw4b200.h)
+static inline int pssmMaxEntry(const int8_t* pssm, int qlen) {
+    int m = 1;
+    for (size_t i = 0; i < (size_t)qlen * 21; i++) m = std::max(m, (int)pssm[i]);
+    return m;
+}
+
+// Code 20 also pads every subject in the device layouts (pair-blocks, tiles of the exact kernels), and the kernels take
+// the maximum over padded columns too. A padded column cannot raise a score or move a first maximum only while it scores
+// <= 0 against every query position, which the BLOSUM tables guarantee (their `low`) and a PSSM must state: column 20
+// (any other letter) > 0 is refused. `what` names the query in the message.
+static inline void checkPssmColumn20(const int8_t* pssm, int qlen, const char* what) {
+    for (int p = 0; p < qlen; p++)
+        if (pssm[(size_t)p * 21 + 20] > 0)
+            fail(SW4_ERR_INVALID, "%s: pssm[%d][20] = %d; the score of residue code 20 (any other letter) must be <= 0", what, p,
+                 (int)pssm[(size_t)p * 21 + 20]);
+}
 
 // Everything sw4_alignment_coordinates and sw4_alignment_traceback own on the handle's first GPU: it shares nothing with the scan (slots, contexts,
 // results), so a scan after the call returns what it would have returned without it.
@@ -379,6 +404,8 @@ struct CoordState {
     DevBuf<int4> dEnds;
     DevBuf<int32_t> dOut;  // [item][5] + error count
     PinnedBuf<char> hQuery;
+    PinnedBuf<int8_t> hPssm;  // a PSSM query's table (allocated by the first PSSM query)
+    DevBuf<int8_t> dPssm;
     PinnedBuf<uint8_t> hSubjects;
     PinnedBuf<CoordGroup> hGroups;
     PinnedBuf<CoordItem> hItems;
@@ -784,7 +811,7 @@ struct Engine {
 
     // All device scratch of a context is sized here, BEFORE the timed region, for a query capacity that only grows by
     // doubling: cudaMalloc/cudaFree inside the event-bracketed region stall the stream for up to hundreds of ms.
-    void ensureCtx(Shard& sh, Ctx& ctx, int qlen, int k) {
+    void ensureCtx(Shard& sh, Ctx& ctx, int qlen, int k, bool pssm) {
         if ((size_t)qlen > ctx.hQuery.n) ctx.hQuery.ensure(std::max<size_t>((size_t)qlen * 2, 65536));
         const size_t topWords = (size_t)2 * k + 8;
         if (topWords > ctx.hTop.n) ctx.hTop.ensure(topWords + 64);
@@ -829,26 +856,41 @@ struct Engine {
             ctx.borderB = ctx.dBorder.p + (size_t)ctx.borderSlots * groupsPerCta * ctx.borderStride;
             ctx.dBorderSlots.ensure((size_t)std::max(ctx.borderSlots, 1));
         }
+        if (pssm && ctx.dPssm.n < (size_t)ctx.queryCapacity * 21) {
+            SW4_CUDA(cudaStreamSynchronize(ctx.stream));
+            ctx.hPssm.ensure((size_t)ctx.queryCapacity * 21);
+            ctx.dPssm.alloc((size_t)ctx.queryCapacity * 21);
+        }
     }
 
     // ---- one query on one shard, part 1: query upload, profile, score reset (enqueued on ctx.stream) ----
     void enqueuePrologue(Shard& sh, Ctx& ctx, const QueryRef& q, int queryIndex, int k) {
         const int qlen = q.length;
-        ensureCtx(sh, ctx, qlen, k);
+        ensureCtx(sh, ctx, qlen, k, q.pssm != nullptr);
         ctx.busy = true;
         ctx.queryIndex = queryIndex;
         ctx.qlen = qlen;
         ctx.k = k;
         ctx.launches = 0;
+        ctx.pssm = q.pssm != nullptr;
+        ctx.maxEntry = ctx.pssm ? pssmMaxEntry(q.pssm, qlen) : maxMatrixEntry;
         const int qpad = (qlen + 3) / 4 * 4;
         // rows of the positional profile start on 128-byte lines: the ring refill copies 64 contiguous bytes per row, which
         // then always fall into two sectors of one line (a stride of 4 mod 8 words cost 3-4 % on the peak benchmark)
         ctx.profStride = (qlen + 96 + 31) / 32 * 32;  // (the two-row array kernel reads up to q + 80 gap rows)
-        if (qlen) memcpy(ctx.hQuery.p, q.letters, (size_t)qlen);
         cudaStream_t st = ctx.stream;
         SW4_CUDA(cudaEventRecord(ctx.evStart, st));
-        if (qlen) SW4_CUDA(cudaMemcpyAsync(ctx.dQueryLetters.p, ctx.hQuery.p, (size_t)qlen, cudaMemcpyHostToDevice, st));
-        SW4_CUDA(cudaMemcpyAsync(ctx.dMatrix.p, matrix, 441, cudaMemcpyHostToDevice, st));
+        if (ctx.pssm) {
+            // the scan reads only the profile: the letters of a PSSM query are not needed
+            if (qlen) {
+                memcpy(ctx.hPssm.p, q.pssm, (size_t)qlen * 21);
+                SW4_CUDA(cudaMemcpyAsync(ctx.dPssm.p, ctx.hPssm.p, (size_t)qlen * 21, cudaMemcpyHostToDevice, st));
+            }
+        } else {
+            if (qlen) memcpy(ctx.hQuery.p, q.letters, (size_t)qlen);
+            if (qlen) SW4_CUDA(cudaMemcpyAsync(ctx.dQueryLetters.p, ctx.hQuery.p, (size_t)qlen, cudaMemcpyHostToDevice, st));
+            SW4_CUDA(cudaMemcpyAsync(ctx.dMatrix.p, matrix, 441, cudaMemcpyHostToDevice, st));
+        }
         SW4_CUDA(cudaMemsetAsync(ctx.dCounters.p, 0, kNumCounters * sizeof(int), st));
         if (ctx.borderSlots) SW4_CUDA(cudaMemsetAsync(ctx.dBorderSlots.p, 0, (size_t)ctx.borderSlots * sizeof(int), st));
         // every scan starts from "-1 = not scored" so that a subject the kernels missed can never keep an old score;
@@ -856,12 +898,16 @@ struct Engine {
         SW4_CUDA(cudaMemsetAsync(ctx.dScores.p, qlen == 0 ? 0 : 0xff, std::max<size_t>(sh.n, 1) * sizeof(int32_t), st));
         const size_t numZero = std::upper_bound(sh.lengths.begin(), sh.lengths.end(), 0) - sh.lengths.begin();
         if (qlen > 0 && numZero) SW4_CUDA(cudaMemsetAsync(ctx.dScores.p, 0, numZero * sizeof(int32_t), st));
-        if (qpad > 0) {
-            convert_query_kernel<<<(qpad + 255) / 256, 256, 0, st>>>(ctx.dQueryLetters.p, ctx.dQueryCodes.p, qlen, qpad);
-            ctx.launches++;
+        const dim3 profGrid((ctx.profStride + 127) / 128, kProfileRows);
+        if (ctx.pssm) {
+            build_profile_pssm_kernel<<<profGrid, 128, 0, st>>>(ctx.dPssm.p, qlen, ctx.dProfile.p, ctx.profStride);
+        } else {
+            if (qpad > 0) {
+                convert_query_kernel<<<(qpad + 255) / 256, 256, 0, st>>>(ctx.dQueryLetters.p, ctx.dQueryCodes.p, qlen, qpad);
+                ctx.launches++;
+            }
+            build_profile_kernel<<<profGrid, 128, 0, st>>>(ctx.dQueryCodes.p, qlen, ctx.dMatrix.p, ctx.dProfile.p, ctx.profStride);
         }
-        build_profile_kernel<<<dim3((ctx.profStride + 127) / 128, kProfileRows), 128, 0, st>>>(ctx.dQueryCodes.p, qlen, ctx.dMatrix.p,
-                                                                                          ctx.dProfile.p, ctx.profStride);
         SW4_CUDA(cudaGetLastError());
         ctx.launches++;
         SW4_CUDA(cudaEventRecord(ctx.evK0, st));
@@ -1096,7 +1142,13 @@ struct Engine {
                 p.ticket = ctx.dCounters.p + 3; p.scores = ctx.dScores.p;
                 p.statThreshold = 0x7fffffff;
                 p.statCount = ctx.dCounters.p + 1;
-                SW4_CUDA(launch_s32(p, std::max(1, (int)(ctx.borderRowArrays / kS32WarpsPerBlock)), st));
+                const int blocks = std::max(1, (int)(ctx.borderRowArrays / kS32WarpsPerBlock));
+                if (ctx.pssm) {  // scores from the profile's int32 plane: the PSSM query has no matrix rows
+                    const int32_t* prof = reinterpret_cast<const int32_t*>(ctx.dProfile.p + (size_t)(kFused + 42) * profStride);
+                    SW4_CUDA(launch_s32_pssm(p, prof, profStride, blocks, st));
+                } else {
+                    SW4_CUDA(launch_s32(p, blocks, st));
+                }
             }
             ctx.launches++;
         }
@@ -1110,7 +1162,7 @@ struct Engine {
         const long long n = (long long)sh.n;
         const int k = ctx.k;
         if (k > 0 && n > 0) {
-            const long long bound = (long long)maxMatrixEntry * std::min(ctx.qlen, sh.maxLen);
+            const long long bound = (long long)ctx.maxEntry * std::min(ctx.qlen, sh.maxLen);
             const int launches = topk_enqueue(ctx.dScores.p, n, k, bound, sh.smCount, sh.dGlobalIds.p, ctx.dCand.p, ctx.dTopkWork.p,
                                               ctx.dTopkKeys.p, ctx.dTopScores.p, ctx.dTopIds.p, ctx.dCounters.p + 4, st);
             if (launches < 0) fail(SW4_ERR_INVALID, "scores of this scan may reach %lld; the device top-k is exact below 2^24", bound);
@@ -1230,6 +1282,7 @@ struct Engine {
         for (int i = 0; i < nq; i++) {
             if (queries[i].length < 0 || (queries[i].length > 0 && !queries[i].letters)) fail(SW4_ERR_INVALID, "invalid query %d", i);
             if (queries[i].length > (1 << 24)) fail(SW4_ERR_INVALID, "query %d too long (%d)", i, queries[i].length);
+            if (queries[i].pssm) checkPssmColumn20(queries[i].pssm, queries[i].length, ("query " + std::to_string(i)).c_str());
         }
         checkGaps();
         upload();
@@ -1295,8 +1348,8 @@ struct Engine {
         }
     }
 
-    void scan(const char* query, int qlen, int32_t* outScores, int32_t* outIds, int32_t* outCount, sw4_stats* stats) {
-        QueryRef q{query, qlen};
+    void scan(const char* query, int qlen, const int8_t* pssm, int32_t* outScores, int32_t* outIds, int32_t* outCount, sw4_stats* stats) {
+        QueryRef q{query, qlen, pssm};
         scanMany(&q, 1, outScores, outIds, outCount, stats, nullptr);
     }
 
@@ -1306,13 +1359,16 @@ struct Engine {
     // whose scratch (gathered subjects + border columns) fits max_temp_bytes.
     // Checks the arguments shared by sw4_alignment_coordinates and sw4_alignment_traceback; returns the position of
     // every id in the handle's host arrays.
-    std::vector<size_t> alignmentPairs(const char* query, int qlen, const int32_t* ids, int n, const void* out) {
+    // pssm: nullptr (sequence query) or the query's [qlen][21] table (the caller has checked it is there)
+    std::vector<size_t> alignmentPairs(const char* query, int qlen, const int8_t* pssm, const int32_t* ids, int n, const void* out) {
         if (!db) fail(SW4_ERR_INVALID, "no database set");
         if (n < 0) fail(SW4_ERR_INVALID, "num_ids must be >= 0 (got %d)", n);
         if (n > 0 && (!ids || !out)) fail(SW4_ERR_INVALID, "null id or output array");
         if (qlen < 0 || (qlen > 0 && !query)) fail(SW4_ERR_INVALID, "invalid query");
         if (qlen > (1 << 24)) fail(SW4_ERR_INVALID, "query too long (%d residues, at most 2^24)", qlen);
         checkGaps();
+        if (pssm) checkPssmColumn20(pssm, qlen, "query");
+        const int maxEntry = pssm ? pssmMaxEntry(pssm, qlen) : maxMatrixEntry;
         std::vector<size_t> local((size_t)n);
         for (int i = 0; i < n; i++) {
             const int32_t id = ids[i];
@@ -1320,15 +1376,16 @@ struct Engine {
                 fail(SW4_ERR_INVALID, "database id %d out of range (the database has %zu sequences)", id, db->nGlobal);
             local[i] = db->localIndex(id);
             if (local[i] >= db->n) fail(SW4_ERR_INVALID, "database id %d is not held by this handle (pre-sharded database)", id);
-            const long long bound = (long long)maxMatrixEntry * std::min(qlen, db->lengths[local[i]]);
+            const long long bound = (long long)maxEntry * std::min(qlen, db->lengths[local[i]]);
             if (topk_shift_for(bound) < 0)
                 fail(SW4_ERR_INVALID, "the score of the query against id %d may reach %lld; scores are exact below 2^24", id, bound);
         }
         return local;
     }
 
-    // the CoordState on the handle's first GPU (made current) with the query codes and the matrix uploaded on its stream
-    CoordState& coordQuery(const char* query, int qlen, int& launches) {
+    // the CoordState on the handle's first GPU (made current) with the query codes and the matrix uploaded on its stream,
+    // and a PSSM query's table in cs.dPssm
+    CoordState& coordQuery(const char* query, int qlen, const int8_t* pssm, int& launches) {
         if (!coord) {
             auto c = std::make_unique<CoordState>();
             c->create(deviceIds[0]);
@@ -1344,6 +1401,16 @@ struct Engine {
         if ((size_t)qpad + 16 > cs.dQueryCodes.n) { cs.dQueryLetters.alloc((size_t)qpad + 16); cs.dQueryCodes.alloc((size_t)qpad + 16); }
         if (qlen) SW4_CUDA(cudaMemcpyAsync(cs.dQueryLetters.p, cs.hQuery.p, (size_t)qlen, cudaMemcpyHostToDevice, st));
         SW4_CUDA(cudaMemcpyAsync(cs.dMatrix.p, matrix, 441, cudaMemcpyHostToDevice, st));
+        if (pssm && qlen) {
+            const size_t bytes = (size_t)qlen * 21;
+            if (bytes > cs.dPssm.n) {  // (the previous call has synchronised: nothing in flight reads the old buffers)
+                const size_t cap = std::max(bytes * 2, (size_t)8192 * 21);
+                cs.hPssm.ensure(cap);
+                cs.dPssm.alloc(cap);
+            }
+            memcpy(cs.hPssm.p, pssm, bytes);
+            SW4_CUDA(cudaMemcpyAsync(cs.dPssm.p, cs.hPssm.p, bytes, cudaMemcpyHostToDevice, st));
+        }
         if (qpad > 0) {
             convert_query_kernel<<<(qpad + 255) / 256, 256, 0, st>>>(cs.dQueryLetters.p, cs.dQueryCodes.p, qlen, qpad);
             SW4_CUDA(cudaGetLastError());
@@ -1367,7 +1434,9 @@ struct Engine {
     }
 
     // passes 1 and 2 for the pairs (query, local[i]), in chunks under max_temp_bytes; out[i] receives the coordinates
-    void coordPasses(CoordState& cs, int qlen, const std::vector<size_t>& local, sw4_alignment* out, double& cells, int& launches) {
+    // (pssm: the device table of a PSSM query, or nullptr)
+    void coordPasses(CoordState& cs, int qlen, const int8_t* pssm, const std::vector<size_t>& local, sw4_alignment* out, double& cells,
+                     int& launches) {
         const int n = (int)local.size();
         cudaStream_t st = cs.stream;
         auto lengthOf = [&](int i) { return (int)db->lengths[local[i]]; };
@@ -1438,8 +1507,8 @@ struct Engine {
             p.query = cs.dQueryCodes.p; p.qlen = qlen; p.matrix = cs.dMatrix.p; p.gop = gop; p.gex = gex;
             p.border = reinterpret_cast<int2*>(cs.dSubjects.p + subjectBytes); p.borderStride = (int)borderStride;
             p.ends = cs.dEnds.p; p.out = cs.dOut.p; p.errors = cs.dOut.p + (size_t)m * 5;
-            SW4_CUDA(launch_coords(false, p, numGroups, st));
-            SW4_CUDA(launch_coords(true, p, numGroups, st));
+            SW4_CUDA(launch_coords(false, p, numGroups, st, pssm));
+            SW4_CUDA(launch_coords(true, p, numGroups, st, pssm));
             launches += 2;
             SW4_CUDA(cudaMemcpyAsync(cs.hOut.p, cs.dOut.p, ((size_t)m * 5 + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
             SW4_CUDA(cudaStreamSynchronize(st));
@@ -1454,14 +1523,15 @@ struct Engine {
         }
     }
 
-    void alignmentCoordinates(const char* query, int qlen, const int32_t* ids, int n, sw4_alignment* out, sw4_stats* stats) {
-        const std::vector<size_t> local = alignmentPairs(query, qlen, ids, n, out);
+    void alignmentCoordinates(const char* query, int qlen, const int8_t* pssm, const int32_t* ids, int n, sw4_alignment* out,
+                              sw4_stats* stats) {
+        const std::vector<size_t> local = alignmentPairs(query, qlen, pssm, ids, n, out);
         if (stats) memset(stats, 0, sizeof(*stats));
         if (n == 0) return;
         int launches = 0;
         double cells = 0;
-        CoordState& cs = coordQuery(query, qlen, launches);
-        coordPasses(cs, qlen, local, out, cells, launches);
+        CoordState& cs = coordQuery(query, qlen, pssm, launches);
+        coordPasses(cs, qlen, pssm ? cs.dPssm.p : nullptr, local, out, cells, launches);
         coordStats(cs, cells, launches, stats);
     }
 
@@ -1469,16 +1539,18 @@ struct Engine {
     // After the coordinate passes, the pairs with a positive score are chunked again by their trace scratch (subject
     // slice, border columns, 4-bit direction words, rows + cols op bytes, counts) under max_temp_bytes. Each chunk runs
     // pass 3 and the walk and copies the ops and counts back: one host synchronisation per chunk.
-    void alignmentTraceback(const char* query, int qlen, const int32_t* ids, int n, sw4_alignment_summary* out, sw4_stats* stats) {
+    void alignmentTraceback(const char* query, int qlen, const int8_t* pssm, const int32_t* ids, int n, sw4_alignment_summary* out,
+                            sw4_stats* stats) {
         lastCigars.clear();
-        const std::vector<size_t> local = alignmentPairs(query, qlen, ids, n, out);
+        const std::vector<size_t> local = alignmentPairs(query, qlen, pssm, ids, n, out);
         if (stats) memset(stats, 0, sizeof(*stats));
         if (n == 0) return;
         int launches = 0;
         double cells = 0;
-        CoordState& cs = coordQuery(query, qlen, launches);
+        CoordState& cs = coordQuery(query, qlen, pssm, launches);
+        const int8_t* dPssm = pssm ? cs.dPssm.p : nullptr;
         std::vector<sw4_alignment> coords((size_t)n);
-        coordPasses(cs, qlen, local, coords.data(), cells, launches);
+        coordPasses(cs, qlen, dPssm, local, coords.data(), cells, launches);
         cudaStream_t st = cs.stream;
 
         std::vector<int> traced;
@@ -1578,8 +1650,8 @@ struct Engine {
             p.ops = reinterpret_cast<char*>(arena + opsAt);
             p.counts = reinterpret_cast<int4*>(arena + countsAt);
             p.numItems = m;
-            SW4_CUDA(launch_coords_trace(p, numGroups, st));
-            SW4_CUDA(launch_coords_walk(p, st));
+            SW4_CUDA(launch_coords_trace(p, numGroups, st, dPssm));
+            SW4_CUDA(launch_coords_walk(p, st, dPssm));
             launches += 2;
             SW4_CUDA(cudaMemcpyAsync(cs.hTraceOut.p, arena + opsAt, scratchBytes - opsAt, cudaMemcpyDeviceToHost, st));
             SW4_CUDA(cudaStreamSynchronize(st));
@@ -1941,33 +2013,89 @@ int sw4_scan(sw4_handle* h, const char* query, int32_t query_length, int32_t* ou
     if (!h) return SW4_ERR_INVALID;
     return guarded(h, [&] {
         if (h->eng.numTop > 0 && (!out_scores || !out_ids)) sw4::fail(SW4_ERR_INVALID, "null output arrays");
-        h->eng.scan(query, query_length, out_scores, out_ids, out_count, stats);
+        h->eng.scan(query, query_length, nullptr, out_scores, out_ids, out_count, stats);
     });
 }
 
-int sw4_scan_many(sw4_handle* h, const char* const* queries, const int32_t* query_lengths, int32_t num_queries, int32_t* out_scores,
-                  int32_t* out_ids, int32_t* out_counts, sw4_stats* per_query_stats, sw4_stats* total_stats) {
+// (pssms == nullptr: sequence queries)
+static int scanManyQueries(sw4_handle* h, const char* const* queries, const int8_t* const* pssms, const int32_t* query_lengths,
+                           int32_t num_queries, int32_t* out_scores, int32_t* out_ids, int32_t* out_counts, sw4_stats* per_query_stats,
+                           sw4_stats* total_stats) {
     if (!h) return SW4_ERR_INVALID;
     return guarded(h, [&] {
         if (num_queries < 0 || (num_queries > 0 && (!queries || !query_lengths))) sw4::fail(SW4_ERR_INVALID, "invalid query list");
         if (h->eng.numTop > 0 && num_queries > 0 && (!out_scores || !out_ids)) sw4::fail(SW4_ERR_INVALID, "null output arrays");
         std::vector<sw4::QueryRef> q((size_t)num_queries);
-        for (int i = 0; i < num_queries; i++) q[i] = sw4::QueryRef{queries[i], query_lengths[i]};
+        for (int i = 0; i < num_queries; i++) {
+            q[i] = sw4::QueryRef{queries[i], query_lengths[i], pssms ? pssms[i] : nullptr};
+            if (pssms && query_lengths[i] > 0 && !pssms[i]) sw4::fail(SW4_ERR_INVALID, "null pssm of query %d", i);
+        }
         if (total_stats) memset(total_stats, 0, sizeof(*total_stats));
         h->eng.scanMany(q.data(), num_queries, out_scores, out_ids, out_counts, per_query_stats, total_stats);
     });
 }
 
+int sw4_scan_many(sw4_handle* h, const char* const* queries, const int32_t* query_lengths, int32_t num_queries, int32_t* out_scores,
+                  int32_t* out_ids, int32_t* out_counts, sw4_stats* per_query_stats, sw4_stats* total_stats) {
+    return scanManyQueries(h, queries, nullptr, query_lengths, num_queries, out_scores, out_ids, out_counts, per_query_stats, total_stats);
+}
+
 int sw4_alignment_coordinates(sw4_handle* h, const char* query, int32_t query_length, const int32_t* ids, int32_t num_ids,
                               sw4_alignment* out, sw4_stats* stats) {
     if (!h) return SW4_ERR_INVALID;
-    return guarded(h, [&] { h->eng.alignmentCoordinates(query, query_length, ids, num_ids, out, stats); });
+    return guarded(h, [&] { h->eng.alignmentCoordinates(query, query_length, nullptr, ids, num_ids, out, stats); });
 }
 
 int sw4_alignment_traceback(sw4_handle* h, const char* query, int32_t query_length, const int32_t* ids, int32_t num_ids,
                             sw4_alignment_summary* out, sw4_stats* stats) {
     if (!h) return SW4_ERR_INVALID;
-    const int rc = guarded(h, [&] { h->eng.alignmentTraceback(query, query_length, ids, num_ids, out, stats); });
+    const int rc = guarded(h, [&] { h->eng.alignmentTraceback(query, query_length, nullptr, ids, num_ids, out, stats); });
+    if (rc != SW4_OK) h->eng.lastCigars.clear();
+    return rc;
+}
+
+// ---- PSSM queries: the same calls with a [query_length][21] position-specific scoring matrix ----
+// (an empty query may come with a NULL pssm: it still runs as a PSSM query, with no rows)
+static const int8_t kNoPssmRows[1] = {0};
+static const int8_t* pssmQuery(const char* query, const int8_t* pssm, int32_t query_length) {
+    if (query_length > 0 && (!query || !pssm)) sw4::fail(SW4_ERR_INVALID, "null query letters or pssm");
+    return pssm ? pssm : kNoPssmRows;
+}
+
+int sw4_scan_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length, int32_t* out_scores, int32_t* out_ids,
+                  int32_t* out_count, sw4_stats* stats) {
+    if (!h) return SW4_ERR_INVALID;
+    return guarded(h, [&] {
+        const int8_t* rows = pssmQuery(query, pssm, query_length);
+        if (h->eng.numTop > 0 && (!out_scores || !out_ids)) sw4::fail(SW4_ERR_INVALID, "null output arrays");
+        h->eng.scan(query, query_length, rows, out_scores, out_ids, out_count, stats);
+    });
+}
+
+int sw4_scan_many_pssm(sw4_handle* h, const char* const* queries, const int8_t* const* pssms, const int32_t* query_lengths,
+                       int32_t num_queries, int32_t* out_scores, int32_t* out_ids, int32_t* out_counts, sw4_stats* per_query_stats,
+                       sw4_stats* total_stats) {
+    if (!h) return SW4_ERR_INVALID;
+    if (num_queries > 0 && !pssms) return guarded(h, [] { sw4::fail(SW4_ERR_INVALID, "null pssm list"); });
+    std::vector<const int8_t*> p((size_t)std::max(num_queries, 0));  // (scanManyQueries refuses a NULL pssm of a non-empty query)
+    for (size_t i = 0; i < p.size(); i++) p[i] = pssms[i] || (query_lengths && query_lengths[i] > 0) ? pssms[i] : kNoPssmRows;
+    return scanManyQueries(h, queries, p.data(), query_lengths, num_queries, out_scores, out_ids, out_counts, per_query_stats, total_stats);
+}
+
+int sw4_alignment_coordinates_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length, const int32_t* ids,
+                                   int32_t num_ids, sw4_alignment* out, sw4_stats* stats) {
+    if (!h) return SW4_ERR_INVALID;
+    return guarded(h, [&] {
+        h->eng.alignmentCoordinates(query, query_length, pssmQuery(query, pssm, query_length), ids, num_ids, out, stats);
+    });
+}
+
+int sw4_alignment_traceback_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length, const int32_t* ids,
+                                 int32_t num_ids, sw4_alignment_summary* out, sw4_stats* stats) {
+    if (!h) return SW4_ERR_INVALID;
+    const int rc = guarded(h, [&] {
+        h->eng.alignmentTraceback(query, query_length, pssmQuery(query, pssm, query_length), ids, num_ids, out, stats);
+    });
     if (rc != SW4_OK) h->eng.lastCigars.clear();
     return rc;
 }

@@ -96,14 +96,17 @@ __device__ __forceinline__ bool coord_better(int v, int i, int j, int bv, int bi
     return v > bv || (v == bv && (i < bi || (i == bi && j < bj)));
 }
 
-template <int MODE>
-__device__ __forceinline__ void coords_pass(const CoordParams& prm) {
+// PSSM: query position i scores pssm[21 * i + code] (a [qlen][21] table in global memory) instead of the matrix row
+// of its residue code; prm.matrix is not read.
+template <int MODE, bool PSSM = false>
+__device__ __forceinline__ void coords_pass(const CoordParams& prm, const int8_t* __restrict__ pssm = nullptr) {
     constexpr bool REV = MODE == kCoordBegins, TRACE = MODE == kCoordTrace;
     constexpr int R = kCoordR;
-    __shared__ int Msm[21 * 21];
+    __shared__ int Msm[PSSM ? 1 : 21 * 21];
     __shared__ long long progress[kCoordWarps];  // (tile << 32) | rows of that tile's right border already stored
     __shared__ int redV[kCoordWarps], redI[kCoordWarps], redJ[kCoordWarps];
-    for (int i = threadIdx.x; i < 441; i += blockDim.x) Msm[i] = prm.matrix[i];
+    if (!PSSM)
+        for (int i = threadIdx.x; i < 441; i += blockDim.x) Msm[i] = prm.matrix[i];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (lane == 0) progress[warp] = -1;
     __syncthreads();
@@ -174,13 +177,15 @@ __device__ __forceinline__ void coords_pass(const CoordParams& prm) {
                 if (lane == 0) { Hin = firstTile ? 0 : bH; Ein = firstTile ? kNegS32 : bE; }
                 const int row = t - lane;
                 if (row >= 0 && row < q) {
-                    const int* Mrow = Msm + 21 * prm.query[REV ? qe - row : (TRACE ? q0 + row : row)];
+                    const int qrow = REV ? qe - row : (TRACE ? q0 + row : row);
+                    const int* Mrow = PSSM ? nullptr : Msm + 21 * prm.query[qrow];
+                    const int8_t* Prow = PSSM ? pssm + 21 * (size_t)qrow : nullptr;
                     int E = Ein, diag = HinPrev;
                     int rowBest = 0, rowJ = 0;  // first maximum of this row segment
                     unsigned dirs[2] = {0u, 0u};  // pass 3: nibbles of columns 0-7 and 8-15
 #pragma unroll
                     for (int j = 0; j < R; j++) {
-                        const int d = diag + Mrow[srow[j]];
+                        const int d = diag + (PSSM ? (int)__ldg(Prow + srow[j]) : Mrow[srow[j]]);
                         diag = Hp[j];
                         const int h = __vimax3_s32_relu(d, E, F[j]);
                         Hp[j] = h;
@@ -264,6 +269,11 @@ template <bool REV>
 __global__ void __launch_bounds__(kCoordThreads, 1) sw_coords_kernel(const CoordParams prm) {
     coords_pass<REV ? kCoordBegins : kCoordEnds>(prm);
 }
+// the same for a PSSM query (pssm: [qlen][21])
+template <bool REV>
+__global__ void __launch_bounds__(kCoordThreads, 1) sw_coords_pssm_kernel(const CoordParams prm, const int8_t* pssm) {
+    coords_pass<REV ? kCoordBegins : kCoordEnds, true>(prm, pssm);
+}
 
 // pass 3: the same wavefront over each pair's rectangle, storing the 4-bit directions instead of tracking a maximum
 // (this kernel and the walk are templates only so that the header can be included by several translation units)
@@ -271,14 +281,20 @@ template <int kInstance = 0>
 __global__ void __launch_bounds__(kCoordThreads, 1) sw_coords_trace_kernel(const CoordParams prm) {
     coords_pass<kCoordTrace>(prm);
 }
+template <int kInstance = 0>
+__global__ void __launch_bounds__(kCoordThreads, 1) sw_coords_trace_pssm_kernel(const CoordParams prm, const int8_t* pssm) {
+    coords_pass<kCoordTrace, true>(prm, pssm);
+}
 
 constexpr int kWalkThreads = 128;
 
 // The walk: one thread per traced pair, from (qe, re) in state P back to (qb, rb), by the rule of include/sw4b200.h.
-template <int kInstance = 0>
-__global__ void __launch_bounds__(kWalkThreads) sw_coords_walk_kernel(const CoordParams prm) {
-    __shared__ int Msm[21 * 21];
-    for (int i = threadIdx.x; i < 441; i += blockDim.x) Msm[i] = prm.matrix[i];
+// PSSM: a pair at query position i is a positive when pssm[21 * i + code] > 0.
+template <bool PSSM>
+__device__ __forceinline__ void coords_walk(const CoordParams& prm, const int8_t* __restrict__ pssm) {
+    __shared__ int Msm[PSSM ? 1 : 21 * 21];
+    if (!PSSM)
+        for (int i = threadIdx.x; i < 441; i += blockDim.x) Msm[i] = prm.matrix[i];
     __syncthreads();
     const int item = blockIdx.x * blockDim.x + threadIdx.x;
     if (item >= prm.numItems) return;
@@ -302,7 +318,7 @@ __global__ void __launch_bounds__(kWalkThreads) sw_coords_walk_kernel(const Coor
             const int a = min((int)qy[i], 20), b = min((int)s[c], 20);
             ops[len++] = a == b ? '=' : 'X';
             idents += a == b;
-            pos += Msm[21 * a + b] > 0;
+            pos += (PSSM ? (int)pssm[21 * ((size_t)ti.queryBegin + i) + b] : Msm[21 * a + b]) > 0;
             if (i == 0 && c == 0) { ok = true; break; }
             if (--i < 0 || --c < 0) break;
             state = (int)(nibble(i, c) & 3u);
@@ -322,6 +338,15 @@ __global__ void __launch_bounds__(kWalkThreads) sw_coords_walk_kernel(const Coor
     }
     prm.counts[item] = make_int4(len, idents, pos, gaps);
     if (!ok) atomicAdd(prm.errors + 1, 1);
+}
+
+template <int kInstance = 0>
+__global__ void __launch_bounds__(kWalkThreads) sw_coords_walk_kernel(const CoordParams prm) {
+    coords_walk<false>(prm, nullptr);
+}
+template <int kInstance = 0>
+__global__ void __launch_bounds__(kWalkThreads) sw_coords_walk_pssm_kernel(const CoordParams prm, const int8_t* pssm) {
+    coords_walk<true>(prm, pssm);
 }
 
 }  // namespace sw4

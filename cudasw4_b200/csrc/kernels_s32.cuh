@@ -41,13 +41,17 @@ struct S32Params {
     int* statCount;
 };
 
-// (a template only so that the header can be included by several translation units)
-template <int kInstance = 0>
-__global__ void __launch_bounds__(kS32Threads) sw_s32_kernel(const S32Params prm) {
+// The body of both forms. Sequence form: row `row` scores Msm[21 * query[row] + code] (the matrix in shared memory).
+// PSSM form: it scores prof[code * profStride + row], the int32 plane of the query profile (rows 483..503 of
+// build_profile_kernel), so the query may have any length.
+template <bool PSSM>
+__device__ __forceinline__ void sw_s32_body(const S32Params& prm, const int32_t* __restrict__ prof, int profStride) {
     constexpr int R = kS32R;
-    __shared__ int Msm[21 * 21];
-    for (int i = threadIdx.x; i < 441; i += blockDim.x) Msm[i] = prm.matrix[i];
-    __syncthreads();
+    __shared__ int Msm[PSSM ? 1 : 21 * 21];
+    if (!PSSM) {
+        for (int i = threadIdx.x; i < 441; i += blockDim.x) Msm[i] = prm.matrix[i];
+        __syncthreads();
+    }
     const int lane = threadIdx.x & 31;
     const int warpGlobal = blockIdx.x * kS32WarpsPerBlock + (threadIdx.x >> 5);
     int2* border = prm.border + (size_t)warpGlobal * prm.borderStride;
@@ -66,9 +70,9 @@ __global__ void __launch_bounds__(kS32Threads) sw_s32_kernel(const S32Params prm
         const int tiles = (len + 32 * R - 1) / (32 * R);
         for (int tile = 0; tile < tiles; tile++) {
             const int col0 = tile * 32 * R + lane * R;
-            int srow[R];  // 21 * residue code: row offset is added per query row
+            int srow[R];  // residue code (PSSM form: code * profStride); the query row is added per row
 #pragma unroll
-            for (int j = 0; j < R; j++) srow[j] = (col0 + j < len) ? s[col0 + j] : 20;
+            for (int j = 0; j < R; j++) srow[j] = ((col0 + j < len) ? s[col0 + j] : 20) * (PSSM ? profStride : 1);
             int Hp[R], F[R];
 #pragma unroll
             for (int j = 0; j < R; j++) { Hp[j] = 0; F[j] = kNegS32; }
@@ -88,11 +92,11 @@ __global__ void __launch_bounds__(kS32Threads) sw_s32_kernel(const S32Params prm
                 if (lane == 0) { Hin = firstTile ? 0 : bH; Ein = firstTile ? kNegS32 : bE; }
                 const int row = t - lane;
                 if (row >= 0 && row < q) {
-                    const int* Mrow = Msm + 21 * prm.query[row];
+                    const int* Mrow = PSSM ? prof + row : Msm + 21 * prm.query[row];
                     int E = Ein, diag = HinPrev;
 #pragma unroll
                     for (int j = 0; j < R; j++) {
-                        const int d = diag + Mrow[srow[j]];
+                        const int d = diag + (PSSM ? __ldg(Mrow + srow[j]) : Mrow[srow[j]]);
                         diag = Hp[j];
                         const int h = __vimax3_s32_relu(d, E, F[j]);
                         Hp[j] = h;
@@ -127,6 +131,18 @@ __global__ void __launch_bounds__(kS32Threads) sw_s32_kernel(const S32Params prm
             if (best >= prm.statThreshold && len > 240 && len <= 8000) atomicAdd(prm.statCount, 1);
         }
     }
+}
+
+// (templates only so that the header can be included by several translation units)
+template <int kInstance = 0>
+__global__ void __launch_bounds__(kS32Threads) sw_s32_kernel(const S32Params prm) {
+    sw_s32_body<false>(prm, nullptr, 0);
+}
+
+// PSSM queries: prof = the profile's int32 plane (profile + 483 * profStride); prm.query and prm.matrix are not read
+template <int kInstance = 0>
+__global__ void __launch_bounds__(kS32Threads) sw_s32_pssm_kernel(const S32Params prm, const int32_t* prof, int profStride) {
+    sw_s32_body<true>(prm, prof, profStride);
 }
 
 }  // namespace sw4

@@ -27,11 +27,14 @@ cudaError_t launch_s32_long(const S32LongParams& prm, int grid, cudaStream_t str
 cudaError_t launch_s16_long2(const S16Long2Params& prm, int grid, cudaStream_t stream);
 // exact 32-bit wavefront, one subject per warp
 cudaError_t launch_s32(const S32Params& prm, int blocks, cudaStream_t stream);
-// alignment coordinates: pass 1 (ends) or pass 2 (begins), one CTA per CoordGroup
-cudaError_t launch_coords(bool reverse, const CoordParams& prm, int groups, cudaStream_t stream);
+// its PSSM form: scores from the int32 plane of the query profile (prof = profile + 483 * profStride)
+cudaError_t launch_s32_pssm(const S32Params& prm, const int32_t* prof, int profStride, int blocks, cudaStream_t stream);
+// alignment coordinates: pass 1 (ends) or pass 2 (begins), one CTA per CoordGroup. The coordinate and traceback
+// launchers take a PSSM query's [qlen][21] device table as `pssm` (nullptr: a sequence query scored with prm.matrix).
+cudaError_t launch_coords(bool reverse, const CoordParams& prm, int groups, cudaStream_t stream, const int8_t* pssm = nullptr);
 // alignment traceback: pass 3 (directions over each rectangle, one CTA per CoordGroup), then the walk (prm.numItems pairs)
-cudaError_t launch_coords_trace(const CoordParams& prm, int groups, cudaStream_t stream);
-cudaError_t launch_coords_walk(const CoordParams& prm, cudaStream_t stream);
+cudaError_t launch_coords_trace(const CoordParams& prm, int groups, cudaStream_t stream, const int8_t* pssm = nullptr);
+cudaError_t launch_coords_walk(const CoordParams& prm, cudaStream_t stream, const int8_t* pssm = nullptr);
 
 // CTAs are launched as clusters of 2 whenever the grid is even: the two SMs of a TPC share an instruction cache, and
 // with many different (large, heavily unrolled) kernels resident at once it pays to give both SMs the same code.

@@ -3,22 +3,30 @@
 
 namespace sw4 {
 
-cudaError_t launch_coords(bool reverse, const CoordParams& prm, int groups, cudaStream_t stream) {
+cudaError_t launch_coords(bool reverse, const CoordParams& prm, int groups, cudaStream_t stream, const int8_t* pssm) {
     if (groups <= 0) return cudaSuccess;
-    if (reverse) sw_coords_kernel<true><<<groups, kCoordThreads, 0, stream>>>(prm);
-    else sw_coords_kernel<false><<<groups, kCoordThreads, 0, stream>>>(prm);
+    if (pssm) {
+        if (reverse) sw_coords_pssm_kernel<true><<<groups, kCoordThreads, 0, stream>>>(prm, pssm);
+        else sw_coords_pssm_kernel<false><<<groups, kCoordThreads, 0, stream>>>(prm, pssm);
+    } else {
+        if (reverse) sw_coords_kernel<true><<<groups, kCoordThreads, 0, stream>>>(prm);
+        else sw_coords_kernel<false><<<groups, kCoordThreads, 0, stream>>>(prm);
+    }
     return cudaGetLastError();
 }
 
-cudaError_t launch_coords_trace(const CoordParams& prm, int groups, cudaStream_t stream) {
+cudaError_t launch_coords_trace(const CoordParams& prm, int groups, cudaStream_t stream, const int8_t* pssm) {
     if (groups <= 0) return cudaSuccess;
-    sw_coords_trace_kernel<><<<groups, kCoordThreads, 0, stream>>>(prm);
+    if (pssm) sw_coords_trace_pssm_kernel<><<<groups, kCoordThreads, 0, stream>>>(prm, pssm);
+    else sw_coords_trace_kernel<><<<groups, kCoordThreads, 0, stream>>>(prm);
     return cudaGetLastError();
 }
 
-cudaError_t launch_coords_walk(const CoordParams& prm, cudaStream_t stream) {
+cudaError_t launch_coords_walk(const CoordParams& prm, cudaStream_t stream, const int8_t* pssm) {
     if (prm.numItems <= 0) return cudaSuccess;
-    sw_coords_walk_kernel<><<<(prm.numItems + kWalkThreads - 1) / kWalkThreads, kWalkThreads, 0, stream>>>(prm);
+    const int blocks = (prm.numItems + kWalkThreads - 1) / kWalkThreads;
+    if (pssm) sw_coords_walk_pssm_kernel<><<<blocks, kWalkThreads, 0, stream>>>(prm, pssm);
+    else sw_coords_walk_kernel<><<<blocks, kWalkThreads, 0, stream>>>(prm);
     return cudaGetLastError();
 }
 

@@ -60,4 +60,9 @@ cudaError_t launch_s32(const S32Params& prm, int blocks, cudaStream_t stream) {
     return cudaGetLastError();
 }
 
+cudaError_t launch_s32_pssm(const S32Params& prm, const int32_t* prof, int profStride, int blocks, cudaStream_t stream) {
+    sw_s32_pssm_kernel<0><<<blocks, kS32Threads, 0, stream>>>(prm, prof, profStride);
+    return cudaGetLastError();
+}
+
 }  // namespace sw4

@@ -220,6 +220,40 @@ int sw4_alignment_traceback(sw4_handle* h, const char* query, int32_t query_leng
 /* CIGAR text of the last sw4_alignment_traceback on this handle; valid until the next call or sw4_destroy */
 int sw4_last_cigars(const sw4_handle* h, const char** text, size_t* length);
 
+/* Search with a position-specific scoring matrix (PSSM; no reference counterpart), such as PSI-BLAST's
+ * -out_ascii_pssm writes it.
+ *
+ * A PSSM query is query_length residue letters plus int8_t pssm[query_length][21], row-major. pssm[p][r] is the score
+ * of query position p against residue code r. Codes 0..19 are ARNDCQEGHILKMFPSTWYV (the order in which letters are
+ * converted); code 20 is every other letter. Columns 0..19 take the whole int8 range; column 20 takes [-128, 0], and a
+ * positive pssm[p][20] is SW4_ERR_INVALID. Code 20 also pads every subject in the engine's device layout, so a padded
+ * column scores like a non-standard residue; it cannot raise a score or move a first maximum only while that score is
+ * <= 0 against every query position (the BLOSUM tables give it their negative `low`).
+ *
+ * Every score, coordinate and CIGAR definition above holds with M[q_i][r] replaced by pssm[i][r]. Positives are the
+ * pair columns with pssm[i][r] > 0. Identities and the =/X ops still compare residue codes; that is the only use of
+ * the letters, and scores never depend on them. The handle's gap scores apply; its BLOSUM table is not used. The bound
+ * that keeps scores below 2^24 uses the PSSM's own largest entry (at least 1) x min(query, subject) length, per query.
+ *
+ * Why the 16-bit scan stays exact with any int8 entries: a packed score is checked against the re-scoring threshold
+ * 25000 after every cell, and one cell adds at most 127, so the first crossing is seen at a value <= 25000 + 127 <
+ * 32767, before any 16-bit wrap; the subject is then re-scored in 32 bit. Downwards, the gap rows' sentinel -16000 and
+ * the E / F floors take at most -128 (one entry) or -4096 (one gap score) per step before the local floor at 0 or the
+ * maximum with the sentinel resets them, far from -32768.
+ *
+ * The calls below behave as their sequence forms (arguments, outputs, errors, chunking, streaming, sharding, query
+ * batching, sw4_last_cigars and sw4_last_scan_all_scores). query and pssm may be NULL only when query_length == 0;
+ * otherwise a NULL one is SW4_ERR_INVALID, as is a positive entry in column 20. pssms[i] of sw4_scan_many_pssm belongs to queries[i]. */
+int sw4_scan_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length, int32_t* out_scores,
+                  int32_t* out_ids, int32_t* out_count, sw4_stats* stats);
+int sw4_scan_many_pssm(sw4_handle* h, const char* const* queries, const int8_t* const* pssms,
+                       const int32_t* query_lengths, int32_t num_queries, int32_t* out_scores, int32_t* out_ids,
+                       int32_t* out_counts, sw4_stats* per_query_stats, sw4_stats* total_stats);
+int sw4_alignment_coordinates_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length,
+                                   const int32_t* ids, int32_t num_ids, sw4_alignment* out, sw4_stats* stats);
+int sw4_alignment_traceback_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length,
+                                 const int32_t* ids, int32_t num_ids, sw4_alignment_summary* out, sw4_stats* stats);
+
 /* Debug / parity helper (the reference's CUDASW_DEBUG_CHECK_CORRECTNESS mode sets numTop to the whole database,
  * src/cudasw4.cuh:505-507): all scores of the last scan for this handle's shard, plus their global ids, in shard
  * order. capacity is in entries; returns the number written in *out_count. */
