@@ -8,13 +8,14 @@ from __future__ import annotations
 
 import ctypes
 import enum
+import math
 from dataclasses import dataclass, field
 
 import numpy as np
 
 from . import _lib, dbformat
 
-__all__ = ["CudaSW4", "ScanResult", "Alignments", "BenchmarkStats", "KernelType", "KernelTypeConfig", "MemoryConfig", "BlosumType",
+__all__ = ["CudaSW4", "ScanResult", "Alignments", "BenchmarkStats", "ScoreStatistics", "fit_score_statistics", "KernelType", "KernelTypeConfig", "MemoryConfig", "BlosumType",
            "SW4Error", "dbformat"]
 
 
@@ -69,10 +70,40 @@ class BenchmarkStats:  # reference src/cudasw4.cuh:76-80
 
 
 @dataclass
+class ScoreStatistics:
+    """The fit of a query's score histogram (sw4_score_statistics in include/sw4b200.h). `ok` is False when too few
+    subjects could be fitted; lambda_ and K are then NaN."""
+    ok: bool
+    whole_database: bool
+    lambda_: float
+    K: float
+    query_length: int
+    db_residues: int
+    num_subjects: int
+    fitted: int
+    left_censored: int
+    right_censored: int
+    c_lo: int
+    c_hi: int
+
+    def evalue(self, score: int) -> float:
+        """E = K m D e^(-lambda S): the expected number of subjects with a score >= S under the fitted model."""
+        return self.K * float(self.query_length) * float(self.db_residues) * math.exp(-self.lambda_ * score)
+
+    def bit_score(self, score: int) -> float:
+        return (self.lambda_ * score - math.log(self.K)) / math.log(2.0)
+
+
+@dataclass
 class ScanResult:  # reference src/cudasw4.cuh:82-86
     scores: list = field(default_factory=list)
     referenceIds: list = field(default_factory=list)
     stats: BenchmarkStats = field(default_factory=BenchmarkStats)
+    # with score statistics enabled (CudaSW4.setScoreStatistics): one E-value and bit score per hit (empty when the
+    # fit had too few subjects) and the fit itself; empty / None otherwise
+    evalues: list = field(default_factory=list)
+    bitScores: list = field(default_factory=list)
+    statistics: ScoreStatistics | None = None
 
 
 @dataclass
@@ -102,6 +133,26 @@ def _pssm_array(pssm, length: int) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.int8)
 
 
+def _score_statistics(s: _lib.ScoreStatistics) -> ScoreStatistics:
+    return ScoreStatistics(int(s.status) == 0, bool(s.whole_database), float(s.lambda_), float(s.K), int(s.query_length),
+                           int(s.db_residues), int(s.num_subjects), int(s.fitted), int(s.left_censored),
+                           int(s.right_censored), int(s.c_lo), int(s.c_hi))
+
+
+def fit_score_statistics(counts, lensums, query_length: int) -> ScoreStatistics:
+    """The E-value fit of sw4_fit_score_statistics on a histogram of len(counts) - 1 score bins plus the overflow bin
+    (for example one summed over the ranks of a sharded search). Host code only: needs no device."""
+    c = np.ascontiguousarray(counts, dtype=np.int64)
+    L = np.ascontiguousarray(lensums, dtype=np.int64)
+    if c.ndim != 1 or c.shape != L.shape or len(c) < 2:
+        raise ValueError("counts and lensums must be 1-D arrays of equal length >= 2")
+    out = _lib.ScoreStatistics()
+    rc = _lib.load().sw4_fit_score_statistics(c.ctypes.data, L.ctypes.data, len(c) - 1, int(query_length), ctypes.byref(out))
+    if rc != 0:
+        raise ValueError("invalid histogram (negative entries?)")
+    return _score_statistics(out)
+
+
 def _stats(s: _lib.Stats) -> BenchmarkStats:
     return BenchmarkStats(int(s.num_overflows), float(s.seconds), float(s.gcups), float(s.kernel_seconds),
                           float(s.cells), int(s.kernel_launches))
@@ -128,6 +179,7 @@ class CudaSW4:
         if rc != 0:
             raise SW4Error(rc, (self._lib.sw4_last_error(None) or b"").decode())
         self.numTop = int(numTop)
+        self._scoreStatistics = False
         self._gop = -11 if gop is None else int(gop)
         self._gex = -1 if gex is None else int(gex)
         if kernelTypeConfig is not None:
@@ -181,6 +233,37 @@ class CudaSW4:
     def setMemoryConfig(self, val: MemoryConfig):
         mem = _lib.MemConfig(val.maxBatchBytes, val.maxBatchSequences, val.maxTempBytes, min(val.maxGpuMem, 2**64 - 1))
         self._check(self._lib.sw4_set_mem_config(self._h, ctypes.byref(mem)))
+
+    def setScoreStatistics(self, enabled: bool = True, maxEvalue: float = math.inf):
+        """Report E-values and bit scores: every following scan also builds the query's score histogram on the GPU and
+        fits lambda and K to it (include/sw4b200.h). A finite maxEvalue drops the hits with E > maxEvalue, when this
+        handle holds the whole database. Off by default."""
+        self._check(self._lib.sw4_set_score_statistics(self._h, int(bool(enabled)), float(maxEvalue)))
+        self._scoreStatistics = bool(enabled)
+
+    def lastScoreStatistics(self, queryIndex: int = 0) -> ScoreStatistics:
+        """The fit of query `queryIndex` of the last scan call (0 after scan())."""
+        out = _lib.ScoreStatistics()
+        self._check(self._lib.sw4_last_score_statistics(self._h, int(queryIndex), ctypes.byref(out)))
+        return _score_statistics(out)
+
+    def lastScoreHistogram(self, queryIndex: int = 0):
+        """(counts, lensums): int64 arrays of SCORE_BINS + 1 entries (the last one is the overflow bin) over the
+        subjects this handle scanned for query `queryIndex` of the last scan call."""
+        counts = np.zeros(_lib.SCORE_BINS + 1, dtype=np.int64)
+        lensums = np.zeros(_lib.SCORE_BINS + 1, dtype=np.int64)
+        self._check(self._lib.sw4_last_score_histogram(self._h, int(queryIndex), counts.ctypes.data, lensums.ctypes.data,
+                                                       _lib.SCORE_BINS))
+        return counts, lensums
+
+    def _with_statistics(self, r: ScanResult, queryIndex: int) -> ScanResult:
+        if self._scoreStatistics:
+            st = self.lastScoreStatistics(queryIndex)
+            r.statistics = st
+            if st.ok:
+                r.evalues = [st.evalue(s) for s in r.scores]
+                r.bitScores = [st.bit_score(s) for s in r.scores]
+        return r
 
     def setShard(self, rank: int, world: int):
         """One process per GPU: scan only shard `rank` of `world`; ids stay global (no reference equivalent: the
@@ -261,7 +344,7 @@ class CudaSW4:
             self._check(self._lib.sw4_scan_pssm(self._h, q, p.ctypes.data, n, scores.ctypes.data, ids.ctypes.data,
                                                 ctypes.byref(count), ctypes.byref(st)))
         c = int(count.value)
-        return ScanResult(scores[:c].tolist(), ids[:c].tolist(), _stats(st))
+        return self._with_statistics(ScanResult(scores[:c].tolist(), ids[:c].tolist(), _stats(st)), 0)
 
     def scanMany(self, queries, pssm=None):
         """Query batching (sw4_scan_many): all `queries` (letters) with several scans in flight per GPU. Returns
@@ -291,7 +374,7 @@ class CudaSW4:
         out = []
         for i in range(nq):
             c = int(counts[i]) if self.numTop > 0 else 0
-            out.append(ScanResult(scores[i, :c].tolist(), ids[i, :c].tolist(), _stats(per[i])))
+            out.append(self._with_statistics(ScanResult(scores[i, :c].tolist(), ids[i, :c].tolist(), _stats(per[i])), i))
         return out, _stats(total)
 
     def alignmentCoordinates(self, query, ids, stats: BenchmarkStats | None = None, pssm=None) -> np.ndarray:

@@ -15,8 +15,11 @@ EXPORTS = [
     "sw4_reference_length", "sw4_reference_sequence", "sw4_total_timer_start", "sw4_total_timer_stop",
     "sw4_get_db_info", "sw4_version", "sw4_alignment_coordinates",
     "sw4_alignment_traceback", "sw4_last_cigars", "sw4_scan_pssm", "sw4_scan_many_pssm", "sw4_alignment_coordinates_pssm",
-    "sw4_alignment_traceback_pssm",
+    "sw4_alignment_traceback_pssm", "sw4_fit_score_statistics", "sw4_set_score_statistics", "sw4_last_score_statistics",
+    "sw4_last_score_histogram",
 ]
+
+SCORE_BINS = 4096  # SW4_SCORE_BINS: score bins of the histogram, plus one overflow bin
 
 
 class MemConfig(ctypes.Structure):
@@ -38,6 +41,13 @@ class AlignmentSummary(ctypes.Structure):
     _fields_ = [("coordinates", Alignment), ("length", ctypes.c_int32), ("identities", ctypes.c_int32),
                 ("positives", ctypes.c_int32), ("gaps", ctypes.c_int32), ("cigar_offset", ctypes.c_size_t),
                 ("cigar_length", ctypes.c_size_t)]
+
+
+class ScoreStatistics(ctypes.Structure):
+    _fields_ = [("status", ctypes.c_int32), ("whole_database", ctypes.c_int32), ("lambda_", ctypes.c_double),
+                ("K", ctypes.c_double), ("query_length", ctypes.c_int64), ("db_residues", ctypes.c_int64),
+                ("num_subjects", ctypes.c_int64), ("fitted", ctypes.c_int64), ("left_censored", ctypes.c_int64),
+                ("right_censored", ctypes.c_int64), ("c_lo", ctypes.c_int32), ("c_hi", ctypes.c_int32)]
 
 
 class DbInfo(ctypes.Structure):
@@ -92,6 +102,10 @@ def load() -> ctypes.CDLL:
     lib.sw4_alignment_traceback_pssm.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_int32, vp, ctypes.c_int32, vp,
                                                  ctypes.POINTER(Stats)]
     lib.sw4_last_cigars.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(cs)]
+    lib.sw4_fit_score_statistics.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int64, ctypes.POINTER(ScoreStatistics)]
+    lib.sw4_set_score_statistics.argtypes = [vp, ci, ctypes.c_double]
+    lib.sw4_last_score_statistics.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(ScoreStatistics)]
+    lib.sw4_last_score_histogram.argtypes = [vp, ctypes.c_int32, vp, vp, ctypes.c_int32]
     lib.sw4_last_scan_all_scores.argtypes = [vp, vp, vp, cs, ctypes.POINTER(cs)]
     lib.sw4_reference_header.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(vp), ctypes.POINTER(cs)]
     lib.sw4_reference_length.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32)]

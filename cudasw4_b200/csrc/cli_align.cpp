@@ -6,6 +6,8 @@
 #include <algorithm>
 #include <cctype>
 #include <cerrno>
+#include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <fstream>
 #include <iostream>
@@ -23,7 +25,8 @@ namespace {
 struct Options {
     enum class Output { Plain, TSV };
     bool help = false, uploadFull = false, pseudo = false, printPartitions = false, interactive = false, verbose = false,
-         prefetchFile = false, coordinates = false, cigar = false;
+         prefetchFile = false, coordinates = false, cigar = false, evalue = false;
+    double maxEvalue = INFINITY;  // extension: --maxEvalue (implies --evalue)
     int top = 10, gop = -11, gex = -1, pseudoLen = 0;
     int batchQueries = 1;  // extension: queries handed to one scanMany call (1 = one scan per query, as the reference)
     size_t pseudoNum = 0;
@@ -159,6 +162,14 @@ bool parseArgs(int argc, char** argv, Options& o) {
         else if (a == "--tsv") o.output = Options::Output::TSV;
         else if (a == "--coordinates") o.coordinates = true;
         else if (a == "--cigar") o.cigar = true;
+        else if (a == "--evalue") o.evalue = true;
+        else if (a == "--maxEvalue") {
+            const std::string v = need(i);
+            char* end = nullptr;
+            o.maxEvalue = std::strtod(v.c_str(), &end);
+            if (v.empty() || *end != '\0' || !(o.maxEvalue >= 0)) throw std::runtime_error("--maxEvalue needs a number >= 0, got " + v);
+            o.evalue = true;
+        }
         else if (a == "--of") o.outfile = need(i);
         else std::cout << "Unexpected arg " << a << "\n";
     }
@@ -196,6 +207,9 @@ void printHelp(const char* prog) {
               << "   --tsv : tab-separated output\n"
               << "   --coordinates : (extension) also print where each hit aligns: 1-based query and reference begin and end\n"
               << "   --cigar : (extension) also print how each hit aligns: length, identities, positives, gaps and CIGAR\n"
+              << "   --evalue : (extension) also print each hit's E-value and bit score, fitted to the query's own scores (NA:\n"
+              << "              too few subjects to fit)\n"
+              << "   --maxEvalue val : (extension) implies --evalue; report only the hits with E-value <= val\n"
               << "   --verbose, --printLengthPartitions, --interactive, --help\n"
               << "   --batchQueries n : (extension) scan n queries of a file with several scans in flight per GPU; same results\n"
               << "   --prefetchDBFile, --uploadFull, --pseudodb num length\n"
@@ -226,9 +240,19 @@ void printOptions(const Options& o) {
 
 // result printers: formats of reference src/main.cu:34-87 and 243-245. With --coordinates (`coords` non-empty, one
 // entry per hit) every line also carries where the hit aligns, 1-based inclusive as in BLAST (0 = no alignment); with
-// --cigar (`alignments` non-empty) how it aligns: length, identities, positives, gaps and the CIGAR.
+// --cigar (`alignments` non-empty) how it aligns: length, identities, positives, gaps and the CIGAR; with --evalue
+// (`stats` not null) its E-value and bit score.
+std::string formatNumber(double v) {
+    char buf[32];
+    snprintf(buf, sizeof(buf), "%.6g", v);
+    return buf;
+}
+std::string evalueText(const cudasw4::ScoreStatistics& st, int score) { return st.ok ? formatNumber(st.evalue(score)) : "NA"; }
+std::string bitScoreText(const cudasw4::ScoreStatistics& st, int score) { return st.ok ? formatNumber(st.bitScore(score)) : "NA"; }
+
 void printPlain(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::CudaSW4& sw,
-                const std::vector<cudasw4::AlignmentCoordinates>& coords, const std::vector<cudasw4::Alignment>& alignments) {
+                const std::vector<cudasw4::AlignmentCoordinates>& coords, const std::vector<cudasw4::Alignment>& alignments,
+                const cudasw4::ScoreStatistics* stats) {
     for (size_t i = 0; i < r.scores.size(); i++) {
         const auto id = r.referenceIds[i];
         os << "Result " << i << "." << " Score: " << r.scores[i] << "." << " Length: " << sw.getReferenceLength(id) << "."
@@ -243,19 +267,21 @@ void printPlain(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::C
             os << " Identities " << a.identities << "/" << a.length << ". Positives " << a.positives << "/" << a.length
                << ". Gaps " << a.gaps << "/" << a.length << ". CIGAR " << a.cigar << ".";
         }
+        if (stats) os << " E-value " << evalueText(*stats, r.scores[i]) << ". Bit score " << bitScoreText(*stats, r.scores[i]) << ".";
         os << "\n";
     }
 }
-void printTSVHeader(std::ostream& os, bool coordinates, bool cigar) {
+void printTSVHeader(std::ostream& os, bool coordinates, bool cigar, bool evalue) {
     os << "Query number\tQuery length\tQuery header\tResult number\tResult score\tReference length\tReference header\t"
           "Reference ID in DB";
     if (coordinates) os << "\tQuery begin\tQuery end\tReference begin\tReference end";
     if (cigar) os << "\tAlignment length\tIdentities\tPositives\tGaps\tCIGAR";
+    if (evalue) os << "\tE-value\tBit score";
     os << "\n";
 }
 void printTSV(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::CudaSW4& sw, int64_t qnum, size_t qlen,
               const std::string& qheader, const std::vector<cudasw4::AlignmentCoordinates>& coords,
-              const std::vector<cudasw4::Alignment>& alignments) {
+              const std::vector<cudasw4::Alignment>& alignments, const cudasw4::ScoreStatistics* stats) {
     for (size_t i = 0; i < r.scores.size(); i++) {
         const auto id = r.referenceIds[i];
         os << qnum << '\t' << qlen << '\t' << qheader << '\t' << i << '\t' << r.scores[i] << '\t' << sw.getReferenceLength(id)
@@ -268,20 +294,22 @@ void printTSV(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::Cud
             const auto& a = alignments[i];
             os << '\t' << a.length << '\t' << a.identities << '\t' << a.positives << '\t' << a.gaps << '\t' << a.cigar;
         }
+        if (stats) os << '\t' << evalueText(*stats, r.scores[i]) << '\t' << bitScoreText(*stats, r.scores[i]);
         os << "\n";
     }
 }
 
-// (pssm: the query's [length][21] scores, or nullptr for a sequence query)
+// (pssm: the query's [length][21] scores, or nullptr for a sequence query; scanIndex: the query's index in the scan call
+// that produced r, for its score statistics)
 void reportQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
-                 const std::string& sequence, const std::int8_t* pssm, const cudasw4::ScanResult& r);
+                 const std::string& sequence, const std::int8_t* pssm, const cudasw4::ScanResult& r, int scanIndex);
 
 void processQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
                   const std::string& sequence, const std::int8_t* pssm = nullptr) {
     std::cout << "Processing query " << qnum << " ... ";
     std::cout.flush();
     cudasw4::ScanResult r = pssm ? sw.scan(sequence.data(), pssm, (int)sequence.size()) : sw.scan(sequence.data(), (int)sequence.size());
-    reportQuery(o, sw, out, qnum, header, sequence, pssm, r);
+    reportQuery(o, sw, out, qnum, header, sequence, pssm, r, 0);
 }
 
 // --batchQueries: the queries go through one scanMany call; output is written in query order exactly as above
@@ -293,15 +321,18 @@ void processQueryBatch(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out
     const std::vector<cudasw4::ScanResult> results = pssms.empty() ? sw.scanMany(views) : sw.scanMany(views, pssms);
     for (size_t i = 0; i < results.size(); i++) {
         std::cout << "Processing query " << firstQnum + (int64_t)i << " ... ";
-        reportQuery(o, sw, out, firstQnum + (int64_t)i, headers[i], sequences[i], pssms.empty() ? nullptr : pssms[i], results[i]);
+        reportQuery(o, sw, out, firstQnum + (int64_t)i, headers[i], sequences[i], pssms.empty() ? nullptr : pssms[i], results[i],
+                    (int)i);
     }
 }
 
 void reportQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
-                 const std::string& sequence, const std::int8_t* pssm, const cudasw4::ScanResult& r) {
+                 const std::string& sequence, const std::int8_t* pssm, const cudasw4::ScanResult& r, int scanIndex) {
     if (o.verbose) std::cout << "Done. Scan time: " << r.stats.seconds << " s, " << r.stats.gcups << " GCUPS\n";
     else std::cout << "Done.\n";
     if (o.top > 0) {
+        cudasw4::ScoreStatistics stats{};
+        if (o.evalue) stats = sw.lastScoreStatistics(scanIndex);
         std::vector<cudasw4::AlignmentCoordinates> coords;
         std::vector<cudasw4::Alignment> alignments;
         if (o.cigar && !r.referenceIds.empty()) {  // the traceback reports the coordinates too
@@ -316,9 +347,9 @@ void reportQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int6
         if (o.output == Options::Output::Plain) {
             out << "Query " << qnum << ", header" << header << ", length " << sequence.size() << ", num overflows "
                 << r.stats.numOverflows << "\n";
-            printPlain(out, r, sw, coords, alignments);
+            printPlain(out, r, sw, coords, alignments, o.evalue ? &stats : nullptr);
         } else {
-            printTSV(out, r, sw, qnum, sequence.size(), header, coords, alignments);
+            printTSV(out, r, sw, qnum, sequence.size(), header, coords, alignments, o.evalue ? &stats : nullptr);
         }
         out.flush();
     }
@@ -341,11 +372,12 @@ int main(int argc, char** argv) {
         printOptions(o);
         std::ofstream out(o.outfile);
         if (!out) throw std::runtime_error("Cannot open file " + o.outfile);
-        if (o.output == Options::Output::TSV) printTSVHeader(out, o.coordinates, o.cigar);
+        if (o.output == Options::Output::TSV) printTSVHeader(out, o.coordinates, o.cigar, o.evalue);
 
         cudasw4::CudaSW4 sw({}, o.top, o.blosum, o.kernels, o.mem, o.verbose);  // {} = all visible GPUs
         sw.setGapOpenScore(o.gop);
         sw.setGapExtendScore(o.gex);
+        if (o.evalue) sw.setScoreStatistics(true, o.maxEvalue);
         if (!o.pseudo) {
             if (o.verbose) std::cout << "Reading Database: \n";
             sw.setDatabase(std::make_shared<cudasw4::DB>(cudasw4::loadDB(o.db, false, o.prefetchFile)));

@@ -13,6 +13,7 @@
 //     host; one host thread per GPU.
 #include <algorithm>
 #include <cerrno>
+#include <cmath>
 #include <chrono>
 #include <cstdarg>
 #include <cstdio>
@@ -34,6 +35,7 @@
 #include "blosum_tables.hpp"
 #include "device_db.cuh"
 #include "launch.hpp"
+#include "stats.cuh"
 #include "topk.cuh"
 
 namespace sw4 {
@@ -261,12 +263,16 @@ struct Ctx {
     // a PSSM query's [qlen][21] table (allocated by the first PSSM query, grown with queryCapacity)
     PinnedBuf<int8_t> hPssm;
     DevBuf<int8_t> dPssm;
+    // score histogram of the query (statistics enabled; allocated by the first such scan): counts, then lensums
+    DevBuf<unsigned long long> dHist;
+    PinnedBuf<unsigned long long> hHist;
     int queryCapacity = 0;
     size_t topCapacity = 0;
     // the query in flight
     bool busy = false;
     int queryIndex = -1, qlen = 0, k = 0, profStride = 0, launches = 0;
     bool pssm = false;
+    bool stats = false;  // the scan also builds the score histogram
     int maxEntry = 1;  // largest score of one residue pair (at least 1): bounds the scores by maxEntry * min(qlen, len)
     bool largeK = false;
 
@@ -289,6 +295,7 @@ struct Ctx {
         dMatrix.alloc(441);
         dCand.alloc(kTopkMaxCandidates);
         SW4_CUDA(topk_configure());  // every context sets it on its shard's device (runShard selects it before creating them)
+        SW4_CUDA(score_histogram_configure());
     }
     ~Ctx() {
         for (cudaEvent_t e : {evStart, evK0, evK1, evStop, evFork, evBatchDone[0], evBatchDone[1]})
@@ -306,6 +313,7 @@ struct Ctx {
 // what one shard reports for one query
 struct ShardResult {
     std::vector<int32_t> scores, ids;
+    std::vector<int64_t> hist;  // counts then lensums, 2 * kHistEntries (statistics enabled only)
     int statCount = 0, launches = 0;
     double seconds = 0, kernelSeconds = 0;
 };
@@ -462,6 +470,11 @@ struct Engine {
     int maxMatrixEntry = 11;
     std::string lastError;
     std::string lastCigars;  // CIGAR text of the last sw4_alignment_traceback (sw4_last_cigars)
+    // score statistics (sw4_set_score_statistics) and, per query of the last scan call, the histogram and its fit
+    bool statsEnabled = false;
+    double maxEvalue = INFINITY;
+    std::vector<std::vector<int64_t>> lastHists;
+    std::vector<sw4_score_statistics> lastStats;
     // total timer
     std::chrono::steady_clock::time_point totalStart;
     double totalCells = 0;
@@ -811,7 +824,7 @@ struct Engine {
 
     // All device scratch of a context is sized here, BEFORE the timed region, for a query capacity that only grows by
     // doubling: cudaMalloc/cudaFree inside the event-bracketed region stall the stream for up to hundreds of ms.
-    void ensureCtx(Shard& sh, Ctx& ctx, int qlen, int k, bool pssm) {
+    void ensureCtx(Shard& sh, Ctx& ctx, int qlen, int k, bool pssm, bool stats) {
         if ((size_t)qlen > ctx.hQuery.n) ctx.hQuery.ensure(std::max<size_t>((size_t)qlen * 2, 65536));
         const size_t topWords = (size_t)2 * k + 8;
         if (topWords > ctx.hTop.n) ctx.hTop.ensure(topWords + 64);
@@ -861,18 +874,23 @@ struct Engine {
             ctx.hPssm.ensure((size_t)ctx.queryCapacity * 21);
             ctx.dPssm.alloc((size_t)ctx.queryCapacity * 21);
         }
+        if (stats && !ctx.dHist.p) {
+            ctx.dHist.alloc(2 * kHistEntries);
+            ctx.hHist.ensure(2 * kHistEntries);
+        }
     }
 
     // ---- one query on one shard, part 1: query upload, profile, score reset (enqueued on ctx.stream) ----
     void enqueuePrologue(Shard& sh, Ctx& ctx, const QueryRef& q, int queryIndex, int k) {
         const int qlen = q.length;
-        ensureCtx(sh, ctx, qlen, k, q.pssm != nullptr);
+        ensureCtx(sh, ctx, qlen, k, q.pssm != nullptr, statsEnabled);
         ctx.busy = true;
         ctx.queryIndex = queryIndex;
         ctx.qlen = qlen;
         ctx.k = k;
         ctx.launches = 0;
         ctx.pssm = q.pssm != nullptr;
+        ctx.stats = statsEnabled;
         ctx.maxEntry = ctx.pssm ? pssmMaxEntry(q.pssm, qlen) : maxMatrixEntry;
         const int qpad = (qlen + 3) / 4 * 4;
         // rows of the positional profile start on 128-byte lines: the ring refill copies 64 contiguous bytes per row, which
@@ -1171,6 +1189,12 @@ struct Engine {
             SW4_CUDA(cudaMemcpyAsync(ctx.hTop.p, ctx.dTopScores.p, (size_t)k * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
             SW4_CUDA(cudaMemcpyAsync(ctx.hTop.p + k, ctx.dTopIds.p, (size_t)k * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         }
+        if (ctx.stats) {  // the histogram of the scores and lengths of the shard (stats.cuh), next to the top-k
+            SW4_CUDA(cudaMemsetAsync(ctx.dHist.p, 0, ctx.dHist.bytes(), st));
+            ctx.launches += score_histogram_enqueue(ctx.dScores.p, sh.dLengths.p, n, sh.smCount, ctx.dHist.p, st);
+            SW4_CUDA(cudaGetLastError());
+            SW4_CUDA(cudaMemcpyAsync(ctx.hHist.p, ctx.dHist.p, ctx.dHist.bytes(), cudaMemcpyDeviceToHost, st));
+        }
         SW4_CUDA(cudaMemcpyAsync(ctx.hTop.p + 2 * k, ctx.dCounters.p, 8 * sizeof(int), cudaMemcpyDeviceToHost, st));
         SW4_CUDA(cudaEventRecord(ctx.evStop, st));
     }
@@ -1187,6 +1211,7 @@ struct Engine {
         out.ids.assign(ctx.hTop.p + k, ctx.hTop.p + k + cnt);
         out.statCount = counters[1];
         out.launches = ctx.launches;
+        if (ctx.stats) out.hist.assign(ctx.hHist.p, ctx.hHist.p + 2 * kHistEntries);
         out.seconds = (double)ms * 1e-3;
         out.kernelSeconds = (double)kms * 1e-3;
         ctx.busy = false;
@@ -1285,6 +1310,8 @@ struct Engine {
             if (queries[i].pssm) checkPssmColumn20(queries[i].pssm, queries[i].length, ("query " + std::to_string(i)).c_str());
         }
         checkGaps();
+        lastHists.clear();
+        lastStats.clear();
         upload();
         const size_t nTotal = db->nGlobal;
         const int k = (int)std::min<size_t>((size_t)std::max(numTop, 0), nTotal);
@@ -1311,12 +1338,27 @@ struct Engine {
                 overflows += r.statCount;
                 launches += r.launches;
             }
-            const int got = (int)std::min<size_t>((size_t)k, merged.size());
+            int got = (int)std::min<size_t>((size_t)k, merged.size());
             if (shards.size() > 1)
                 std::partial_sort(merged.begin(), merged.begin() + got, merged.end(), [](const Entry& a, const Entry& b) {
                     if (a.score != b.score) return a.score > b.score;
                     return a.id < b.id;
                 });
+            if (statsEnabled) {  // the shards' histograms summed, their fit, and the E-value cutoff
+                std::vector<int64_t> hist(2 * kHistEntries, 0);
+                for (size_t s = 0; s < shards.size(); s++)
+                    for (size_t b = 0; b < hist.size(); b++) hist[b] += results[s][qi].hist[b];
+                sw4_score_statistics st;
+                sw4_fit_score_statistics(hist.data(), hist.data() + kHistEntries, SW4_SCORE_BINS, queries[qi].length, &st);
+                st.whole_database = holdsWholeDatabase() ? 1 : 0;
+                if (st.whole_database && st.status == SW4_STATS_OK && std::isfinite(maxEvalue)) {
+                    int keep = 0;  // E grows as the score falls: the hits to keep are a prefix
+                    while (keep < got && evalueOf(st, merged[keep].score) <= maxEvalue) keep++;
+                    got = keep;
+                }
+                lastHists.push_back(std::move(hist));
+                lastStats.push_back(st);
+            }
             for (int i = 0; i < got; i++) {
                 outScores[(size_t)qi * numTop + i] = merged[i].score;
                 outIds[(size_t)qi * numTop + i] = merged[i].id;
@@ -1346,6 +1388,16 @@ struct Engine {
             total->cells = sumCells;
             total->kernel_launches = sumLaunches;
         }
+    }
+
+    // Does this handle scan every sequence of the database? Not when sw4_set_shard splits it (world > 1), and not when
+    // the handle holds only some of the sequences (sw4_set_database_shard_memory, or the generated shard of
+    // sw4_set_pseudo_database_lengths, which gives every database global ids, sharded or not).
+    bool holdsWholeDatabase() const { return db->globalIds ? db->n == db->nGlobal : shardWorld == 1; }
+
+    // E = K m D e^(-lambda S) (sw4b200.h)
+    static double evalueOf(const sw4_score_statistics& st, int score) {
+        return st.K * (double)st.query_length * (double)st.db_residues * std::exp(-st.lambda * score);
     }
 
     void scan(const char* query, int qlen, const int8_t* pssm, int32_t* outScores, int32_t* outIds, int32_t* outCount, sw4_stats* stats) {
@@ -2104,6 +2156,40 @@ int sw4_last_cigars(const sw4_handle* h, const char** text, size_t* length) {
     if (!h || !text || !length) return SW4_ERR_INVALID;
     *text = h->eng.lastCigars.c_str();
     *length = h->eng.lastCigars.size();
+    return SW4_OK;
+}
+
+int sw4_set_score_statistics(sw4_handle* h, int enabled, double max_evalue) {
+    if (!h) return SW4_ERR_INVALID;
+    return guarded(h, [&] {
+        if (std::isnan(max_evalue) || max_evalue < 0) sw4::fail(SW4_ERR_INVALID, "max_evalue must be >= 0 or INFINITY (got %g)", max_evalue);
+        h->eng.statsEnabled = enabled != 0;
+        h->eng.maxEvalue = max_evalue;
+    });
+}
+
+// (query_index of the last scan call; fails when it ran without statistics)
+static const char* lastStatsError(const sw4_handle* h, int32_t query_index) {
+    if (h->eng.lastStats.empty()) return "the last scan ran without score statistics (sw4_set_score_statistics)";
+    if (query_index < 0 || (size_t)query_index >= h->eng.lastStats.size()) return "query_index out of range";
+    return nullptr;
+}
+
+int sw4_last_score_statistics(const sw4_handle* h, int32_t query_index, sw4_score_statistics* out) {
+    if (!h || !out) return SW4_ERR_INVALID;
+    if (const char* e = lastStatsError(h, query_index)) { const_cast<sw4_handle*>(h)->eng.lastError = e; return SW4_ERR_INVALID; }
+    *out = h->eng.lastStats[(size_t)query_index];
+    return SW4_OK;
+}
+
+int sw4_last_score_histogram(const sw4_handle* h, int32_t query_index, int64_t* counts, int64_t* lensums, int32_t bins) {
+    if (!h || !counts || !lensums) return SW4_ERR_INVALID;
+    const char* e = lastStatsError(h, query_index);
+    if (!e && bins != SW4_SCORE_BINS) e = "bins must be SW4_SCORE_BINS";
+    if (e) { const_cast<sw4_handle*>(h)->eng.lastError = e; return SW4_ERR_INVALID; }
+    const std::vector<int64_t>& hist = h->eng.lastHists[(size_t)query_index];
+    memcpy(counts, hist.data(), sw4::kHistEntries * sizeof(int64_t));
+    memcpy(lensums, hist.data() + sw4::kHistEntries, sw4::kHistEntries * sizeof(int64_t));
     return SW4_OK;
 }
 

@@ -13,6 +13,7 @@
 #ifndef CUDASW4_B200_FACADE_CUH
 #define CUDASW4_B200_FACADE_CUH
 
+#include <cmath>
 #include <cstdint>
 #include <iostream>
 #include <limits>
@@ -57,6 +58,17 @@ struct ScanResult { std::vector<int> scores{}; std::vector<ReferenceIdT> referen
 struct AlignmentCoordinates { int score, queryBegin, queryEnd, referenceBegin, referenceEnd; };
 // Extension: how a hit aligns (sw4b200.h): its coordinates, counts and SAM-style CIGAR (=, X, I, D; "" when score == 0)
 struct Alignment { AlignmentCoordinates coordinates; int length, identities, positives, gaps; std::string cigar; };
+// Extension: the score statistics of one query's search (sw4_score_statistics in sw4b200.h); ok == false: too few
+// subjects to fit, lambda and K are NaN
+struct ScoreStatistics {
+    bool ok, wholeDatabase;
+    double lambda, K;
+    std::int64_t queryLength, dbResidues, numSubjects, fitted, leftCensored, rightCensored;
+    int cLo, cHi;
+    // E = K m D e^(-lambda S) and the bit score (lambda S - ln K) / ln 2 of a hit with score S
+    double evalue(int score) const { return K * (double)queryLength * (double)dbResidues * std::exp(-lambda * score); }
+    double bitScore(int score) const { return (lambda * score - std::log(K)) / std::log(2.0); }
+};
 struct KernelTypeConfig {                                                                             // :88-93
     KernelType singlePassType = KernelType::Half2;
     KernelType manyPassType_small = KernelType::Half2;
@@ -178,6 +190,23 @@ public:
     std::vector<Alignment> computeAlignments(const char* query, const std::int8_t* pssm, SequenceLengthT length,
                                              const std::vector<ReferenceIdT>& ids) {
         return alignmentsImpl(query, pssm, true, length, ids);
+    }
+
+    // Extension (sw4b200.h): E-values. enabled: every following scan also fits its score statistics; a finite maxEvalue
+    // drops the hits with E > maxEvalue when the handle holds the whole database.
+    void setScoreStatistics(bool enabled, double maxEvalue = INFINITY) { check(sw4_set_score_statistics(handle, enabled ? 1 : 0, maxEvalue)); }
+    // the statistics of query queryIndex of the last scan() / scanMany() call
+    ScoreStatistics lastScoreStatistics(int queryIndex = 0) const {
+        sw4_score_statistics s{};
+        check(sw4_last_score_statistics(handle, queryIndex, &s));
+        return ScoreStatistics{s.status == SW4_STATS_OK, s.whole_database != 0, s.lambda, s.K, s.query_length, s.db_residues,
+                               s.num_subjects, s.fitted, s.left_censored, s.right_censored, s.c_lo, s.c_hi};
+    }
+    // its histogram over this handle's subjects: SW4_SCORE_BINS + 1 entries each (the last is the overflow bin)
+    void lastScoreHistogram(int queryIndex, std::vector<std::int64_t>& counts, std::vector<std::int64_t>& lensums) const {
+        counts.assign(SW4_SCORE_BINS + 1, 0);
+        lensums.assign(SW4_SCORE_BINS + 1, 0);
+        check(sw4_last_score_histogram(handle, queryIndex, counts.data(), lensums.data(), SW4_SCORE_BINS));
     }
 
     void printDBInfo() const {                                                                      // :799-807

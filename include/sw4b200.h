@@ -254,6 +254,65 @@ int sw4_alignment_coordinates_pssm(sw4_handle* h, const char* query, const int8_
 int sw4_alignment_traceback_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length,
                                  const int32_t* ids, int32_t num_ids, sw4_alignment_summary* out, sw4_stats* stats);
 
+/* Significance of the hits (no reference counterpart): E-values and bit scores from score statistics that each query's
+ * own search yields. Every scan with statistics enabled also builds, on the GPU, a histogram of the scores of the
+ * subjects it scanned: count[s] subjects and lensum[s] residues (the sum of their lengths) per score s, for
+ * s = 0 .. SW4_SCORE_BINS - 1, and an overflow bin s = SW4_SCORE_BINS for all higher scores. Subjects of length 0 are
+ * left out. In a database almost every subject is unrelated to the query, so this is the null distribution, and the fit
+ * below turns it into lambda and K. It needs no tabulated constants and serves PSSM queries at any score scale.
+ *
+ * Model: with m the query length and n_j the length of subject j, its score behaves like x_j = s_j + 1/2 with
+ * P(x_j >= x) = 1 - exp(-K m n_j e^(-lambda x)).
+ * Censoring, with N the subjects of length >= 1:
+ *   c_lo = the median score: the smallest s with #(score <= s) >= N / 2. Lower scores are left-censored.
+ *   c_hi = the smallest s > c_lo with #(score >= s) <= floor(N / 1000); SW4_SCORE_BINS when no such s is below it.
+ *          Scores >= c_hi are right-censored (the homologs end up there).
+ * Maximum likelihood: U subjects with c_lo <= s < c_hi contribute ln lambda + ln(K m n_j) - lambda x_j - K m n_j
+ * e^(-lambda x_j); a left-censored one -K m n_j e^(-lambda c_lo); the R right-censored ones ln(K m n_j) - lambda c_hi.
+ * dlnL/dK = 0 gives K = (U + R) / (m A(lambda)) with A(lambda) = sum_fitted lensum[s] e^(-lambda (s + 1/2)) +
+ * e^(-lambda c_lo) sum_{s < c_lo} lensum[s]. The profile likelihood is strictly concave in lambda; its derivative
+ * U / lambda - sum_fitted count[s] (s + 1/2) - R c_hi + (U + R) B(lambda) / A(lambda), with B = A with each term
+ * weighted by its x (s + 1/2, or c_lo), is bisected on [1e-4, 10] until the interval cannot shrink in double.
+ * status SW4_STATS_TOO_FEW (lambda = K = NaN: no E-values, no cutoff) when U < 100, c_lo >= SW4_SCORE_BINS or m < 1.
+ *
+ * A hit with score S has E = K m D e^(-lambda S) (D = sum of lensum: the residues of the subjects; E is the expected
+ * number of subjects with a score >= S under the model) and the bit score (lambda S - ln K) / ln 2. E decreases with S,
+ * so a cutoff on E only shortens a result list. */
+#define SW4_SCORE_BINS 4096
+#define SW4_STATS_OK 0
+#define SW4_STATS_TOO_FEW 1
+typedef struct sw4_score_statistics {
+    int32_t status;          /* SW4_STATS_OK or SW4_STATS_TOO_FEW                                                    */
+    int32_t whole_database;  /* 1 when the histogram covers the whole database; 0 when the handle scans only a shard   *
+                              * (sw4_set_shard with world > 1, or a database of which it holds only some sequences:    *
+                              * sw4_set_database_shard_memory, sw4_set_pseudo_database_lengths under sw4_set_shard)     */
+    double lambda, K;        /* NaN unless status == SW4_STATS_OK                                                     */
+    int64_t query_length;    /* m */
+    int64_t db_residues;     /* D = sum of lensum */
+    int64_t num_subjects;    /* N = sum of count */
+    int64_t fitted, left_censored, right_censored;  /* U, the subjects below c_lo, R */
+    int32_t c_lo, c_hi;
+} sw4_score_statistics;
+
+/* The fit above, on a histogram of bins + 1 entries per array (entry `bins` is the overflow bin), for example one summed
+ * over the shards of a sharded search. Pure host code: it needs no handle and no device. whole_database is set to 1.
+ * SW4_ERR_INVALID: NULL arrays or out, bins < 1, or a negative entry. */
+int sw4_fit_score_statistics(const int64_t* counts, const int64_t* lensums, int32_t bins, int64_t query_length,
+                             sw4_score_statistics* out);
+
+/* enabled != 0: every following scan also builds the score histogram of each query (one more kernel per query and GPU)
+ * and fits it. max_evalue (INFINITY: no cutoff) then drops the hits with E > max_evalue from out_scores / out_ids /
+ * *out_count of every scan call (sw4_scan, sw4_scan_many and their _pssm forms), but only when the handle holds the
+ * whole database and the fit succeeded. enabled == 0 (the default): a scan does exactly what it did without statistics.
+ * SW4_ERR_INVALID: max_evalue NaN or < 0. */
+int sw4_set_score_statistics(sw4_handle* h, int enabled, double max_evalue);
+/* The statistics of query `query_index` of the last scan call (0 after sw4_scan). A handle on several GPUs sums their
+ * histograms before the fit. SW4_ERR_INVALID when the last scan ran without statistics or query_index is out of range. */
+int sw4_last_score_statistics(const sw4_handle* h, int32_t query_index, sw4_score_statistics* out);
+/* The histogram behind sw4_last_score_statistics (this handle's shards summed): counts and lensums hold bins + 1 entries,
+ * and bins must be SW4_SCORE_BINS. A sharded search sums these over its ranks and calls sw4_fit_score_statistics. */
+int sw4_last_score_histogram(const sw4_handle* h, int32_t query_index, int64_t* counts, int64_t* lensums, int32_t bins);
+
 /* Debug / parity helper (the reference's CUDASW_DEBUG_CHECK_CORRECTNESS mode sets numTop to the whole database,
  * src/cudasw4.cuh:505-507): all scores of the last scan for this handle's shard, plus their global ids, in shard
  * order. capacity is in entries; returns the number written in *out_count. */
