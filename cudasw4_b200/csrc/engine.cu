@@ -1139,7 +1139,8 @@ struct Engine {
             // exact 32-bit path for whatever saturated in 16 bit (the list and its length live on the device)
             const int p0 = (qlen + 32 + 15) / 16 * 16;
             if (useLongKernel && kLongLag * kLongMaxWarps + 64 <= p0) {
-                // long queries (the only ones that can saturate 16 bits) re-score on the CTA-wide array, 16 warps per subject
+                // long queries re-score on the CTA-wide array, 16 warps per subject, whatever the subject's length (with a
+                // PSSM, subjects of any class from 197 residues on can saturate 16 bits)
                 S32LongParams lp{};
                 lp.chars = arena; lp.offsets = offsetsBySubject; lp.lengths = sh.dLengths.p;
                 lp.list = ctx.dOvfList.p; lp.listCountPtr = ctx.dCounters.p + 0; lp.ticket = ctx.dCounters.p + 3;

@@ -235,9 +235,13 @@ int sw4_last_cigars(const sw4_handle* h, const char** text, size_t* length);
  * the letters, and scores never depend on them. The handle's gap scores apply; its BLOSUM table is not used. The bound
  * that keeps scores below 2^24 uses the PSSM's own largest entry (at least 1) x min(query, subject) length, per query.
  *
- * Why the 16-bit scan stays exact with any int8 entries: a packed score is checked against the re-scoring threshold
- * 25000 after every cell, and one cell adds at most 127, so the first crossing is seen at a value <= 25000 + 127 <
- * 32767, before any 16-bit wrap; the subject is then re-scored in 32 bit. Downwards, the gap rows' sentinel -16000 and
+ * Why the 16-bit scan stays exact with any int8 entries: every s16 kernel (two-row, multi-segment, one-row wide and
+ * both array kernels) keeps, per subject of a packed pair, a running maximum of the diagonal term H[i-1][j-1] +
+ * pssm[i][s_j] of every cell, and compares it with the re-scoring threshold 25000 once, when the pair is finished (the
+ * array kernels fold the maxima of a pair's column blocks with a max first). Until some H reaches 25000 every value is
+ * exact, and the first H to reach it is a diagonal term (E and F never exceed an earlier H), of at most 24999 + 127 <
+ * 32767: it enters the running maximum before any 16-bit wrap, and a maximum never decreases, so the subject is
+ * re-scored in 32 bit whatever wraps after it. Downwards, the gap rows' sentinel -16000 and
  * the E / F floors take at most -128 (one entry) or -4096 (one gap score) per step before the local floor at 0 or the
  * maximum with the sentinel resets them, far from -32768.
  *
