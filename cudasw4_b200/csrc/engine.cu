@@ -822,6 +822,23 @@ struct Engine {
         return *sh.ctxs[c];
     }
 
+    // The query capacity a context grows to for a qlen-residue query (from `current`, 0 for a new context), by doubling.
+    static int queryCapacityFor(int qlen, int current) {
+        int cap = std::max(current, 8192);
+        while (cap < qlen) cap *= 2;
+        return cap;
+    }
+    static size_t borderStrideFor(int cap) { return (size_t)(cap + 31) / 32 * 32 + 128; }
+    // Every scan needs at least kS16Warps border row arrays of its context's capacity within max_temp_bytes. Contexts are
+    // recreated when the memory configuration changes, so a query that passes at its own capacity,
+    // queryCapacityFor(qlen, 0), passes in any context that a later query of the same call grows.
+    void checkBorderRows(int cap, int qlen) const {
+        const size_t stride = borderStrideFor(cap);
+        if (mem.max_temp_bytes / (stride * sizeof(uint2)) < (size_t)kS16Warps)
+            fail(SW4_ERR_NOMEM, "max_temp_bytes (%zu MiB) cannot hold the border rows of a %d-residue query (%zu MiB needed at least)",
+                 mem.max_temp_bytes >> 20, qlen, (kS16Warps * stride * sizeof(uint2)) >> 20);
+    }
+
     // All device scratch of a context is sized here, BEFORE the timed region, for a query capacity that only grows by
     // doubling: cudaMalloc/cudaFree inside the event-bracketed region stall the stream for up to hundreds of ms.
     void ensureCtx(Shard& sh, Ctx& ctx, int qlen, int k, bool pssm, bool stats) {
@@ -831,8 +848,7 @@ struct Engine {
         if (ctx.dScores.n < std::max<size_t>(sh.n, 1)) { ctx.dScores.alloc(sh.n); ctx.dOvfList.alloc(sh.n); }
         if (qlen > ctx.queryCapacity || (size_t)k > ctx.topCapacity) {
             SW4_CUDA(cudaStreamSynchronize(ctx.stream));
-            int cap = std::max(ctx.queryCapacity, 8192);
-            while (cap < qlen) cap *= 2;
+            const int cap = queryCapacityFor(qlen, ctx.queryCapacity);
             ctx.queryCapacity = cap;
             ctx.topCapacity = std::max(ctx.topCapacity, (size_t)std::max(k, 64));
             const size_t capStride = (size_t)(cap + 96 + 31) / 32 * 32;
@@ -850,14 +866,12 @@ struct Engine {
             // size is bounded by max_temp_bytes: fewer row arrays = fewer CTAs on those kernels.
             // (one row array = cap + 128 (H, E) pairs; the two-row multi-segment kernel keeps one per GROUP, two per warp, as
             // cap / 2 + 64 entries of both rows of a step)
-            ctx.borderStride = (size_t)(cap + 31) / 32 * 32 + 128;
+            checkBorderRows(cap, qlen);
+            ctx.borderStride = borderStrideFor(cap);
             const bool needBorder = sh.maxLen > 512;
             const size_t groupsPerCta = (size_t)kS16Warps * 2;
             size_t rows = needBorder ? (size_t)sh.smCount * (groupsPerCta + kS16Warps) : (size_t)kS16Warps;
             const size_t maxRows = mem.max_temp_bytes / (ctx.borderStride * sizeof(uint2));
-            if (maxRows < (size_t)kS16Warps)
-                fail(SW4_ERR_NOMEM, "max_temp_bytes (%zu MiB) cannot hold the border rows of a %d-residue query (%zu MiB needed at least)",
-                     mem.max_temp_bytes >> 20, qlen, (kS16Warps * ctx.borderStride * sizeof(uint2)) >> 20);
             rows = std::min(rows, maxRows / kS16Warps * kS16Warps);
             // two thirds for the slots of the multi-segment kernels (none when the budget is that small: those classes
             // then fall back to the one-warp-per-pair kernel)
@@ -1181,10 +1195,10 @@ struct Engine {
         const long long n = (long long)sh.n;
         const int k = ctx.k;
         if (k > 0 && n > 0) {
-            const long long bound = (long long)ctx.maxEntry * std::min(ctx.qlen, sh.maxLen);
+            const long long bound = scanScoreBound(ctx.maxEntry, ctx.qlen, sh);
             const int launches = topk_enqueue(ctx.dScores.p, n, k, bound, sh.smCount, sh.dGlobalIds.p, ctx.dCand.p, ctx.dTopkWork.p,
                                               ctx.dTopkKeys.p, ctx.dTopScores.p, ctx.dTopIds.p, ctx.dCounters.p + 4, st);
-            if (launches < 0) fail(SW4_ERR_INVALID, "scores of this scan may reach %lld; the device top-k is exact below 2^24", bound);
+            if (launches < 0) refuseScoreBound(bound);  // (checkScanQueries refuses the call before this can happen)
             ctx.launches += launches;
             SW4_CUDA(cudaGetLastError());
             SW4_CUDA(cudaMemcpyAsync(ctx.hTop.p, ctx.dTopScores.p, (size_t)k * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -1200,7 +1214,11 @@ struct Engine {
         SW4_CUDA(cudaEventRecord(ctx.evStop, st));
     }
 
-    void collect(Shard& sh, Ctx& ctx, ShardResult& out) {
+    // the result of the context's query goes to results[ctx.queryIndex]
+    void collect(Shard& sh, Ctx& ctx, std::vector<ShardResult>& results) {
+        if (ctx.queryIndex < 0 || (size_t)ctx.queryIndex >= results.size())
+            fail(SW4_ERR_CUDA, "internal error: a context holds query %d of a call with %zu queries", ctx.queryIndex, results.size());
+        ShardResult& out = results[(size_t)ctx.queryIndex];
         SW4_CUDA(cudaEventSynchronize(ctx.evStop));
         float ms = 0, kms = 0;
         SW4_CUDA(cudaEventElapsedTime(&ms, ctx.evStart, ctx.evStop));
@@ -1222,7 +1240,29 @@ struct Engine {
     // Resident shard: a rolling pipeline of `pipelineDepth` contexts; the host only blocks on the oldest query in flight.
     // Streaming shard: groups of up to kMaxContexts queries; every batch is uploaded once per group and scanned by all of
     // its queries while the next batch is on its way into the other slot.
+    // An exception (a CUDA error: checkScanQueries has refused every bad query up front) waits for the work of the
+    // shard's busy contexts and marks them idle before it leaves, so that the next call neither collects a query of this
+    // one nor reuses buffers that are still being written.
     void runShard(Shard& sh, const QueryRef* queries, int nq, int kGlobal, std::vector<ShardResult>& results) {
+        try {
+            runShardQueries(sh, queries, nq, kGlobal, results);
+        } catch (...) {
+            cudaSetDevice(sh.device);
+            for (auto& c : sh.ctxs) {
+                if (!c->busy) continue;
+                for (int i = 0; i < kMaxClassStreams; i++) {  // (errors ignored: the first one is on its way out)
+                    cudaStreamSynchronize(c->classStreams[i]);
+                    cudaStreamSynchronize(c->oddStreams[i]);
+                }
+                cudaStreamSynchronize(c->stream);
+                c->busy = false;
+            }
+            cudaStreamSynchronize(sh.copyStream);
+            throw;
+        }
+    }
+
+    void runShardQueries(Shard& sh, const QueryRef* queries, int nq, int kGlobal, std::vector<ShardResult>& results) {
         SW4_CUDA(cudaSetDevice(sh.device));
         results.assign(nq, ShardResult{});
         sh.lastSpanSeconds = 0;
@@ -1243,7 +1283,7 @@ struct Engine {
             for (int qi = 0; qi < nq; qi++) {
                 Ctx& ctx = context(sh, qi % depth);
                 if (qi == 0) spanStart(ctx);
-                if (ctx.busy) collect(sh, ctx, results[ctx.queryIndex]);
+                if (ctx.busy) collect(sh, ctx, results);
                 enqueuePrologue(sh, ctx, queries[qi], qi, k);
                 enqueueBatch(sh, ctx, 0, 0, true);
                 enqueueEpilogue(sh, ctx);
@@ -1251,7 +1291,7 @@ struct Engine {
             }
             for (int c = 0; c < depth; c++) {
                 Ctx& ctx = context(sh, (nq + c) % depth);  // oldest first
-                if (ctx.busy) collect(sh, ctx, results[ctx.queryIndex]);
+                if (ctx.busy) collect(sh, ctx, results);
             }
             spanStop();
             return;
@@ -1275,7 +1315,7 @@ struct Engine {
                 if (bi + 1 < numBatches) stage(bi + 1);
             }
             for (int qi = q0; qi < q1; qi++) enqueueEpilogue(sh, context(sh, qi - q0));
-            for (int qi = q0; qi < q1; qi++) collect(sh, context(sh, qi - q0), results[qi]);
+            for (int qi = q0; qi < q1; qi++) collect(sh, context(sh, qi - q0), results);
             sh.lastCtx = q1 - q0 - 1;
         }
         spanStop();
@@ -1300,6 +1340,29 @@ struct Engine {
             if (e.code != SW4_OK) throw e;
     }
 
+    // The scores of a query whose largest pair score is maxEntry stay below this bound on the shard; the device top-k
+    // is exact only while it is below 2^24.
+    static long long scanScoreBound(int maxEntry, int qlen, const Shard& sh) { return (long long)maxEntry * std::min(qlen, sh.maxLen); }
+    [[noreturn]] static void refuseScoreBound(long long bound) {
+        fail(SW4_ERR_INVALID, "scores of this scan may reach %lld; the device top-k is exact below 2^24", bound);
+    }
+
+    // Every per-query refusal of a scan call (the top-k bound of enqueueEpilogue, the border rows of ensureCtx), decided
+    // before the first query is enqueued: a refused call leaves the contexts, the last scan's scores and its statistics
+    // as they were. kGlobal: the call's k.
+    void checkScanQueries(const QueryRef* queries, int nq, int kGlobal) const {
+        for (int i = 0; i < nq; i++) {
+            const QueryRef& q = queries[i];
+            checkBorderRows(queryCapacityFor(q.length, 0), q.length);
+            const int maxEntry = q.pssm ? pssmMaxEntry(q.pssm, q.length) : maxMatrixEntry;
+            for (const auto& sh : shards) {
+                const int k = (int)std::min<size_t>((size_t)kGlobal, sh->n);
+                if (k > 0 && sh->n > 0 && topk_shift_for(scanScoreBound(maxEntry, q.length, *sh)) < 0)
+                    refuseScoreBound(scanScoreBound(maxEntry, q.length, *sh));
+            }
+        }
+    }
+
     // ---- the public scans ----
     // outScores/outIds: [nq][numTop] (row stride numTop), outCounts[nq]; perQuery[nq] and total may be null.
     void scanMany(const QueryRef* queries, int nq, int32_t* outScores, int32_t* outIds, int32_t* outCounts, sw4_stats* perQuery,
@@ -1311,11 +1374,12 @@ struct Engine {
             if (queries[i].pssm) checkPssmColumn20(queries[i].pssm, queries[i].length, ("query " + std::to_string(i)).c_str());
         }
         checkGaps();
+        const size_t nTotal = db->nGlobal;
+        const int k = (int)std::min<size_t>((size_t)std::max(numTop, 0), nTotal);
+        checkScanQueries(queries, nq, k);
         lastHists.clear();
         lastStats.clear();
         upload();
-        const size_t nTotal = db->nGlobal;
-        const int k = (int)std::min<size_t>((size_t)std::max(numTop, 0), nTotal);
         std::vector<std::vector<ShardResult>> results;
         runAllShards(queries, nq, k, results);
         double span = 0;  // device-timed, max over the GPUs
