@@ -15,7 +15,7 @@ import numpy as np
 
 from . import _lib, dbformat
 
-__all__ = ["CudaSW4", "ScanResult", "Alignments", "BenchmarkStats", "ScoreStatistics", "fit_score_statistics", "KernelType", "KernelTypeConfig", "MemoryConfig", "BlosumType",
+__all__ = ["CudaSW4", "ScanResult", "Alignments", "IterativeResult", "BenchmarkStats", "ScoreStatistics", "fit_score_statistics", "KernelType", "KernelTypeConfig", "MemoryConfig", "BlosumType",
            "SW4Error", "dbformat"]
 
 
@@ -114,6 +114,17 @@ class Alignments:
     coordinates: np.ndarray
     counts: np.ndarray
     cigars: list
+
+
+@dataclass
+class IterativeResult:
+    """What CudaSW4.searchIterative returns: the last round's hits (`result`, with E-values, exactly as that round's
+    scan reports them), the (m, 21) int8 PSSM that round searched with (`pssm`; after one round the matrix rows), the
+    number of rounds and whether they stopped because the included hits repeated (`converged`)."""
+    result: ScanResult
+    pssm: np.ndarray
+    iterations: int
+    converged: bool
 
 
 def _pssm_array(pssm, length: int) -> np.ndarray:
@@ -432,6 +443,47 @@ class CudaSW4:
                 setattr(stats, k, v)
         cigars = [text[int(o):int(o) + int(L)] for o, L in zip(raw["offset"], raw["length"])]
         return Alignments(raw["coordinates"].copy(), raw["counts"].copy(), cigars)
+
+    def buildPssm(self, query, ids, pssm=None, pseudocountWeight: float = 10.0, stats: BenchmarkStats | None = None) -> np.ndarray:
+        """The profile of the query and the hits `ids`, built on the GPU (sw4_build_pssm, include/sw4b200.h): the
+        alignments of alignments() for that query form, a query-anchored MSA, Henikoff position-based weights and
+        pseudocounts of weight `pseudocountWeight`. Returns an (m, 21) int8 array that scan(pssm=...) takes. `ids` may
+        be empty (then the rows are the matrix rows of the query's residues); pssm: the query form to align with."""
+        q = query.encode() if isinstance(query, str) else bytes(query)
+        idv = np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1))
+        if len(idv) and (idv.min() < -2**31 or idv.max() >= 2**31):
+            raise SW4Error(-1, "database id out of range")
+        idv = idv.astype(np.int32)
+        out = np.zeros((max(len(q), 1), 21), dtype=np.int8)
+        p = None if pssm is None else _pssm_array(pssm, len(q))
+        st = _lib.Stats()
+        self._check(self._lib.sw4_build_pssm(self._h, q, None if p is None else p.ctypes.data, len(q), idv.ctypes.data, len(idv),
+                                             float(pseudocountWeight), out.ctypes.data, ctypes.byref(st)))
+        if stats is not None:
+            for k, v in vars(_stats(st)).items():
+                setattr(stats, k, v)
+        return out[:len(q)].copy()
+
+    def searchIterative(self, query, iterations: int = 3, inclusionEvalue: float = 0.002,
+                        pseudocountWeight: float = 10.0) -> IterativeResult:
+        """Iterative profile search (sw4_search_iterative): scan, take the hits with E <= inclusionEvalue (before the
+        handle's maxEvalue cutoff), build their profile with buildPssm and scan again with it, for at most `iterations`
+        rounds or until no hit is included or the included set repeats. Needs setScoreStatistics(True) and a handle
+        that scans the whole database."""
+        q = query.encode() if isinstance(query, str) else bytes(query)
+        k = max(self.numTop, 1)
+        scores = np.empty(k, dtype=np.int32)
+        ids = np.empty(k, dtype=np.int32)
+        pssm = np.zeros((max(len(q), 1), 21), dtype=np.int8)
+        count, rounds, converged = ctypes.c_int32(0), ctypes.c_int32(0), ctypes.c_int32(0)
+        st = _lib.Stats()
+        self._check(self._lib.sw4_search_iterative(self._h, q, len(q), int(iterations), float(inclusionEvalue),
+                                                   float(pseudocountWeight), scores.ctypes.data, ids.ctypes.data,
+                                                   ctypes.byref(count), pssm.ctypes.data, ctypes.byref(rounds),
+                                                   ctypes.byref(converged), ctypes.byref(st)))
+        c = int(count.value)
+        r = self._with_statistics(ScanResult(scores[:c].tolist(), ids[:c].tolist(), _stats(st)), 0)
+        return IterativeResult(r, pssm[:len(q)].copy(), int(rounds.value), bool(converged.value))
 
     def lastScanAllScores(self):
         """(scores, global ids) of every subject this handle scanned in the last scan() (parity helper)."""

@@ -16,7 +16,7 @@ EXPORTS = [
     "sw4_get_db_info", "sw4_version", "sw4_alignment_coordinates",
     "sw4_alignment_traceback", "sw4_last_cigars", "sw4_scan_pssm", "sw4_scan_many_pssm", "sw4_alignment_coordinates_pssm",
     "sw4_alignment_traceback_pssm", "sw4_fit_score_statistics", "sw4_set_score_statistics", "sw4_last_score_statistics",
-    "sw4_last_score_histogram",
+    "sw4_last_score_histogram", "sw4_build_pssm", "sw4_search_iterative",
 ]
 
 SCORE_BINS = 4096  # SW4_SCORE_BINS: score bins of the histogram, plus one overflow bin
@@ -106,6 +106,11 @@ def load() -> ctypes.CDLL:
     lib.sw4_set_score_statistics.argtypes = [vp, ci, ctypes.c_double]
     lib.sw4_last_score_statistics.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(ScoreStatistics)]
     lib.sw4_last_score_histogram.argtypes = [vp, ctypes.c_int32, vp, vp, ctypes.c_int32]
+    lib.sw4_build_pssm.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_int32, vp, ctypes.c_int32, ctypes.c_double, vp,
+                                   ctypes.POINTER(Stats)]
+    i32p = ctypes.POINTER(ctypes.c_int32)
+    lib.sw4_search_iterative.argtypes = [vp, ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_double, ctypes.c_double,
+                                         vp, vp, i32p, vp, i32p, i32p, ctypes.POINTER(Stats)]
     lib.sw4_last_scan_all_scores.argtypes = [vp, vp, vp, cs, ctypes.POINTER(cs)]
     lib.sw4_reference_header.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(vp), ctypes.POINTER(cs)]
     lib.sw4_reference_length.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32)]

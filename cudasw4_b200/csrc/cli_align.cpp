@@ -27,6 +27,11 @@ struct Options {
     bool help = false, uploadFull = false, pseudo = false, printPartitions = false, interactive = false, verbose = false,
          prefetchFile = false, coordinates = false, cigar = false, evalue = false;
     double maxEvalue = INFINITY;  // extension: --maxEvalue (implies --evalue)
+    // extension: iterative profile search (--iterations, --inclusionEvalue) and the final PSSMs (--outPssm PREFIX)
+    int iterations = 1;
+    double inclusionEvalue = 0.002;
+    std::string outPssm;
+    bool iterative() const { return iterations > 1 || !outPssm.empty(); }
     int top = 10, gop = -11, gex = -1, pseudoLen = 0;
     int batchQueries = 1;  // extension: queries handed to one scanMany call (1 = one scan per query, as the reference)
     size_t pseudoNum = 0;
@@ -122,7 +127,7 @@ cudasw4::KernelType parseKernelType(const std::string& s) {
 }
 
 bool parseArgs(int argc, char** argv, Options& o) {
-    bool gotQuery = false, gotDB = false, gotGop = false, gotGex = false, dpx = false;
+    bool gotQuery = false, gotDB = false, gotGop = false, gotGex = false, dpx = false, gotIterationOption = false;
     auto need = [&](int& i) -> std::string {
         if (i + 1 >= argc) throw std::runtime_error(std::string("missing value for ") + argv[i]);
         return argv[++i];
@@ -170,6 +175,22 @@ bool parseArgs(int argc, char** argv, Options& o) {
             if (v.empty() || *end != '\0' || !(o.maxEvalue >= 0)) throw std::runtime_error("--maxEvalue needs a number >= 0, got " + v);
             o.evalue = true;
         }
+        else if (a == "--iterations") {
+            const std::string v = need(i);
+            char* end = nullptr;
+            const long n = std::strtol(v.c_str(), &end, 10);
+            if (v.empty() || *end != '\0' || n < 1 || n > 1000000) throw std::runtime_error("--iterations needs an integer >= 1, got " + v);
+            o.iterations = (int)n;
+            gotIterationOption = true;
+        }
+        else if (a == "--inclusionEvalue") {
+            const std::string v = need(i);
+            char* end = nullptr;
+            o.inclusionEvalue = std::strtod(v.c_str(), &end);
+            if (v.empty() || *end != '\0' || !(o.inclusionEvalue >= 0)) throw std::runtime_error("--inclusionEvalue needs a number >= 0, got " + v);
+            gotIterationOption = true;
+        }
+        else if (a == "--outPssm") { o.outPssm = need(i); gotIterationOption = true; }
         else if (a == "--of") o.outfile = need(i);
         else std::cout << "Unexpected arg " << a << "\n";
     }
@@ -186,6 +207,8 @@ bool parseArgs(int argc, char** argv, Options& o) {
         o.kernels.overflowType = cudasw4::KernelType::DPXs32;
     }
     if (gotQuery && !o.pssmFiles.empty()) throw std::runtime_error("--query and --pssm cannot be combined");
+    if (gotIterationOption && !o.pssmFiles.empty())
+        throw std::runtime_error("--iterations, --inclusionEvalue and --outPssm start from a --query sequence; they cannot be combined with --pssm");
     if (!gotQuery && o.pssmFiles.empty() && !o.interactive) { std::cout << "Query is missing\n"; return false; }
     if (!gotDB) { std::cout << "DB prefix is missing\n"; return false; }
     return true;
@@ -210,6 +233,11 @@ void printHelp(const char* prog) {
               << "   --evalue : (extension) also print each hit's E-value and bit score, fitted to the query's own scores (NA:\n"
               << "              too few subjects to fit)\n"
               << "   --maxEvalue val : (extension) implies --evalue; report only the hits with E-value <= val\n"
+              << "   --iterations n : (extension) iterative profile search: up to n rounds of scan, profile of the hits with\n"
+              << "                    E-value <= --inclusionEvalue, scan with that profile. Reports the last round. Default 1\n"
+              << "   --inclusionEvalue val : (extension) E-value a hit needs to enter the next round's profile. Default 0.002\n"
+              << "   --outPssm prefix : (extension) write each query's last profile to prefix.<query number>.pssm, in the\n"
+              << "                      ASCII format --pssm reads\n"
               << "   --verbose, --printLengthPartitions, --interactive, --help\n"
               << "   --batchQueries n : (extension) scan n queries of a file with several scans in flight per GPU; same results\n"
               << "   --prefetchDBFile, --uploadFull, --pseudodb num length\n"
@@ -304,8 +332,41 @@ void printTSV(std::ostream& os, const cudasw4::ScanResult& r, const cudasw4::Cud
 void reportQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
                  const std::string& sequence, const std::int8_t* pssm, const cudasw4::ScanResult& r, int scanIndex);
 
+// --outPssm: the ASCII PSSM that readAsciiPssm reads back unchanged (column 20 is the table's `low` on both sides)
+void writeAsciiPssm(const std::string& path, const std::string& letters, const std::vector<std::int8_t>& pssm) {
+    std::ofstream f(path);
+    if (!f) throw std::runtime_error("cannot write PSSM file " + path);
+    f << "Last position-specific scoring matrix computed\n        ";
+    for (const char* c = "ARNDCQEGHILKMFPSTWYV"; *c; c++) f << "   " << *c;
+    f << "\n";
+    for (size_t p = 0; p < letters.size(); p++) {
+        char buf[32];
+        snprintf(buf, sizeof(buf), "%5zu %c ", p + 1, std::isgraph((unsigned char)letters[p]) ? letters[p] : 'X');
+        f << buf;
+        for (int a = 0; a < 20; a++) {
+            snprintf(buf, sizeof(buf), "%4d", (int)pssm[p * 21 + a]);
+            f << buf;
+        }
+        f << "\n";
+    }
+    if (!f) throw std::runtime_error("cannot write PSSM file " + path);
+}
+
+// --iterations / --outPssm: one query's rounds (one at a time, also under --batchQueries), reported as its last scan
+void processQueryIterative(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
+                           const std::string& sequence) {
+    std::cout << "Processing query " << qnum << " ... ";
+    std::cout.flush();
+    const cudasw4::IterativeSearchResult it = sw.searchIterative(sequence.data(), (int)sequence.size(), o.iterations, o.inclusionEvalue);
+    if (!o.outPssm.empty()) writeAsciiPssm(o.outPssm + "." + std::to_string(qnum) + ".pssm", sequence, it.pssm);
+    reportQuery(o, sw, out, qnum, header, sequence, it.pssm.data(), it.result, 0);
+    std::cout << "Query " << qnum << ": " << it.iterations << (it.iterations == 1 ? " round, " : " rounds, ")
+              << (it.converged ? "converged" : "not converged") << "\n";
+}
+
 void processQuery(const Options& o, cudasw4::CudaSW4& sw, std::ostream& out, int64_t qnum, const std::string& header,
                   const std::string& sequence, const std::int8_t* pssm = nullptr) {
+    if (o.iterative() && !pssm) return processQueryIterative(o, sw, out, qnum, header, sequence);
     std::cout << "Processing query " << qnum << " ... ";
     std::cout.flush();
     cudasw4::ScanResult r = pssm ? sw.scan(sequence.data(), pssm, (int)sequence.size()) : sw.scan(sequence.data(), (int)sequence.size());
@@ -377,7 +438,7 @@ int main(int argc, char** argv) {
         cudasw4::CudaSW4 sw({}, o.top, o.blosum, o.kernels, o.mem, o.verbose);  // {} = all visible GPUs
         sw.setGapOpenScore(o.gop);
         sw.setGapExtendScore(o.gex);
-        if (o.evalue) sw.setScoreStatistics(true, o.maxEvalue);
+        if (o.evalue || o.iterative()) sw.setScoreStatistics(true, o.maxEvalue);  // the rounds need the E-values
         if (!o.pseudo) {
             if (o.verbose) std::cout << "Reading Database: \n";
             sw.setDatabase(std::make_shared<cudasw4::DB>(cudasw4::loadDB(o.db, false, o.prefetchFile)));
@@ -418,7 +479,7 @@ int main(int argc, char** argv) {
                 sw4::SequenceFileReader reader(qf);
                 int64_t qnum = 0;
                 sw.totalTimerStart();
-                if (o.batchQueries <= 1) {
+                if (o.batchQueries <= 1 || o.iterative()) {
                     while (reader.next()) {
                         processQuery(o, sw, out, qnum, reader.getCurrentHeader(), reader.getCurrentSequence());
                         qnum++;

@@ -35,6 +35,7 @@
 #include "blosum_tables.hpp"
 #include "device_db.cuh"
 #include "launch.hpp"
+#include "profile.cuh"
 #include "stats.cuh"
 #include "topk.cuh"
 
@@ -97,6 +98,10 @@ static const int kRefBoundaries[36] = {48,  64,  80,  96,  112, 128, 144, 160, 1
                                        704, 768, 832, 896, 960, 1024, 1088, 1152, 1216, 1280, 8000, 2147483646};
 
 static inline size_t alignUp(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// UniProt background frequencies in 1/256 steps (cumulative), residue codes 0..19: the residues of generated databases
+// (sw4_set_pseudo_database_lengths) and the background p_a of the profile construction (sw4_build_pssm)
+static const int kPseudoCumulative[20] = {21, 35, 46, 60, 63, 73, 91, 109, 115, 130, 155, 170, 176, 186, 198, 214, 228, 231, 238, 256};
 
 // ---------------------------------------------------------------------------------------------------------------
 // host database (makedb format)
@@ -422,6 +427,17 @@ struct CoordState {
     DevBuf<TraceItem> dTraceItems;
     PinnedBuf<TraceItem> hTraceItems;
     PinnedBuf<char> hTraceOut;
+    // profile construction (sw4_build_pssm): the MSA (apart from the arena), each traced pair's MSA row per chunk, the
+    // column statistics, row weights, background tables and the [m][21] result
+    DevBuf<uint8_t> dMsa;
+    DevBuf<int> dMsaRows, dProfileCounts;
+    PinnedBuf<int> hMsaRows;
+    DevBuf<int2> dProfileDistinct;
+    DevBuf<unsigned long long> dProfileNsum;
+    DevBuf<double> dProfileWeights, dProfileTables;  // tables: q_ab / p_b [400], then p_a [20]
+    PinnedBuf<double> hProfileTables;
+    DevBuf<int8_t> dProfileOut;
+    PinnedBuf<int8_t> hProfileOut;
 
     void create(int dev) {
         device = dev;
@@ -436,6 +452,34 @@ struct CoordState {
         if (evStart) cudaEventDestroy(evStart);
         if (evStop) cudaEventDestroy(evStop);
         if (stream) cudaStreamDestroy(stream);
+    }
+};
+
+// The ungapped background of a substitution table M (sw4_build_pssm): p_a from kPseudoCumulative, lambda_u the root of
+// sum_{a,b<20} p_a p_b e^(lambda M[a][b]) = 1, bisected in double on [1e-3, 2] until the interval stops shrinking, and
+// q_ab = p_a p_b e^(lambda_u M[a][b]) / Z with Z that sum. qOverP[a][b] = q_ab / p_b.
+struct ProfileBackground {
+    int blosum = 0;  // the table it was computed for (0: none yet)
+    double lambda = 0, p[20] = {}, qOverP[400] = {};
+    void compute(int id, const int8_t* matrix) {
+        for (int a = 0; a < 20; a++) p[a] = (kPseudoCumulative[a] - (a ? kPseudoCumulative[a - 1] : 0)) / 256.0;
+        auto sum = [&](double lam) {
+            double z = 0;
+            for (int a = 0; a < 20; a++)
+                for (int b = 0; b < 20; b++) z += p[a] * p[b] * std::exp(lam * matrix[a * 21 + b]);
+            return z;
+        };
+        double lo = 1e-3, hi = 2.0;  // below the root the sum is < 1
+        for (;;) {
+            const double mid = (lo + hi) / 2;
+            if (!(mid > lo && mid < hi)) break;
+            (sum(mid) < 1 ? lo : hi) = mid;
+        }
+        lambda = lo;
+        const double z = sum(lambda);
+        for (int a = 0; a < 20; a++)
+            for (int b = 0; b < 20; b++) qOverP[a * 20 + b] = p[a] * p[b] * std::exp(lambda * matrix[a * 21 + b]) / z / p[b];
+        blosum = id;
     }
 };
 
@@ -475,6 +519,7 @@ struct Engine {
     double maxEvalue = INFINITY;
     std::vector<std::vector<int64_t>> lastHists;
     std::vector<sw4_score_statistics> lastStats;
+    ProfileBackground profileBg;  // of the current table, computed by the first sw4_build_pssm that needs it
     // total timer
     std::chrono::steady_clock::time_point totalStart;
     double totalCells = 0;
@@ -1656,12 +1701,15 @@ struct Engine {
     // After the coordinate passes, the pairs with a positive score are chunked again by their trace scratch (subject
     // slice, border columns, 4-bit direction words, rows + cols op bytes, counts) under max_temp_bytes. Each chunk runs
     // pass 3 and the walk and copies the ops and counts back: one host synchronisation per chunk.
+    // profile: the pseudocount weight of sw4_build_pssm, whose MSA the chunks then fill (each pair's row right after the
+    // walk) and whose PSSM follows the last chunk into cs.hProfileOut; nullptr: the traceback alone, which leaves
+    // sw4_last_cigars to this call. Without a profile the call enqueues nothing else.
     void alignmentTraceback(const char* query, int qlen, const int8_t* pssm, const int32_t* ids, int n, sw4_alignment_summary* out,
-                            sw4_stats* stats) {
-        lastCigars.clear();
+                            sw4_stats* stats, const double* profile = nullptr) {
+        if (!profile) lastCigars.clear();
         const std::vector<size_t> local = alignmentPairs(query, qlen, pssm, ids, n, out);
         if (stats) memset(stats, 0, sizeof(*stats));
-        if (n == 0) return;
+        if (n == 0 && !profile) return;
         int launches = 0;
         double cells = 0;
         CoordState& cs = coordQuery(query, qlen, pssm, launches);
@@ -1692,6 +1740,22 @@ struct Engine {
             return alignUp((size_t)colsOf(i), 16) + borderOf(i) * sizeof(int2) + wordsOf(i) * sizeof(unsigned long long) + opsOf(i) +
                    sizeof(int4);
         };
+        // the profile's MSA: row 0 the query, then one row per traced id in call order, allocated apart from the arena
+        std::vector<int> msaRow;
+        int msaRows = 1;
+        if (profile) {
+            msaRow.assign((size_t)n, 0);
+            for (int i : traced) msaRow[i] = msaRows++;
+            const size_t msaBytes = (size_t)msaRows * (size_t)qlen;
+            if (msaBytes > mem.max_temp_bytes)
+                fail(SW4_ERR_NOMEM, "max_temp_bytes (%zu bytes) cannot hold the MSA of the profile (%d rows x %d columns)",
+                     mem.max_temp_bytes, msaRows, qlen);
+            cs.dMsa.ensure(std::max<size_t>(msaBytes, 1));
+            if (qlen) {
+                SW4_CUDA(cudaMemsetAsync(cs.dMsa.p, kMsaEmpty, msaBytes, st));
+                SW4_CUDA(cudaMemcpyAsync(cs.dMsa.p, cs.dQueryCodes.p, (size_t)qlen, cudaMemcpyDeviceToDevice, st));
+            }
+        }
         // CTA-form pairs first, then the one-warp pairs; largest rectangle first within each form
         std::stable_sort(traced.begin(), traced.end(), [&](int a, int b) {
             const bool ca = warpsOf(a) > 1, cb = warpsOf(b) > 1;
@@ -1770,6 +1834,14 @@ struct Engine {
             SW4_CUDA(launch_coords_trace(p, numGroups, st, dPssm));
             SW4_CUDA(launch_coords_walk(p, st, dPssm));
             launches += 2;
+            if (profile && qlen) {  // the chunk's MSA rows, while its subject slices and ops are in the arena
+                cs.hMsaRows.ensure((size_t)m);
+                for (int k = 0; k < m; k++) cs.hMsaRows.p[k] = msaRow[traced[pos + k]];
+                cs.dMsaRows.ensure((size_t)m);
+                SW4_CUDA(cudaMemcpyAsync(cs.dMsaRows.p, cs.hMsaRows.p, (size_t)m * sizeof(int), cudaMemcpyHostToDevice, st));
+                SW4_CUDA(launch_profile_scatter(p, cs.dMsaRows.p, cs.dMsa.p, qlen, st));
+                launches++;
+            }
             SW4_CUDA(cudaMemcpyAsync(cs.hTraceOut.p, arena + opsAt, scratchBytes - opsAt, cudaMemcpyDeviceToHost, st));
             SW4_CUDA(cudaStreamSynchronize(st));
             const char* ops = cs.hTraceOut.p;
@@ -1782,6 +1854,7 @@ struct Engine {
                 sw4_alignment_summary& o = out[traced[pos + k]];
                 const int4 c = counts[k];
                 o.length = c.x; o.identities = c.y; o.positives = c.z; o.gaps = c.w;
+                if (profile) continue;
                 // the walk wrote the ops from the end: run-length encode them backwards, in query order
                 const char* r = ops + cs.hTraceItems.p[k].ops;
                 o.cigar_offset = lastCigars.size();
@@ -1796,7 +1869,118 @@ struct Engine {
             }
             pos = end;
         }
+        if (profile) profileScores(cs, qlen, msaRows, *profile, launches);
         coordStats(cs, cells, launches, stats);
+    }
+
+    // steps 3-6 of the profile over the finished MSA of msaRows rows (profile.cuh); the result lands in cs.hProfileOut
+    // once the stream is synchronised
+    void profileScores(CoordState& cs, int qlen, int msaRows, double beta, int& launches) {
+        if (qlen == 0) return;
+        cudaStream_t st = cs.stream;
+        if (profileBg.blosum != blosum) profileBg.compute(blosum, matrix);
+        cs.hProfileTables.ensure(420);
+        memcpy(cs.hProfileTables.p, profileBg.qOverP, 400 * sizeof(double));
+        memcpy(cs.hProfileTables.p + 400, profileBg.p, 20 * sizeof(double));
+        cs.dProfileTables.ensure(420);
+        cs.dProfileCounts.ensure((size_t)kMsaSymbols * qlen);
+        cs.dProfileDistinct.ensure((size_t)qlen);
+        cs.dProfileNsum.ensure(2);
+        cs.dProfileWeights.ensure((size_t)msaRows);
+        cs.dProfileOut.ensure((size_t)qlen * 21);
+        cs.hProfileOut.ensure((size_t)qlen * 21);
+        SW4_CUDA(cudaMemcpyAsync(cs.dProfileTables.p, cs.hProfileTables.p, 420 * sizeof(double), cudaMemcpyHostToDevice, st));
+        SW4_CUDA(cudaMemsetAsync(cs.dProfileNsum.p, 0, 2 * sizeof(unsigned long long), st));
+        ProfileParams p{};
+        p.msa = cs.dMsa.p; p.rows = msaRows; p.m = qlen;
+        p.counts = cs.dProfileCounts.p; p.distinct = cs.dProfileDistinct.p; p.nsum = cs.dProfileNsum.p;
+        p.weights = cs.dProfileWeights.p; p.qOverP = cs.dProfileTables.p; p.p = cs.dProfileTables.p + 400;
+        p.lambda = profileBg.lambda; p.beta = beta; p.low = matrix[20 * 21 + 20];
+        p.out = cs.dProfileOut.p;
+        SW4_CUDA(launch_profile_build(p, st, &launches));
+        SW4_CUDA(cudaMemcpyAsync(cs.hProfileOut.p, cs.dProfileOut.p, (size_t)qlen * 21, cudaMemcpyDeviceToHost, st));
+    }
+
+    // ---- profile construction and the iterative search (sw4_build_pssm, sw4_search_iterative) ----
+    static void checkBeta(double beta) {
+        if (!(beta > 0) || !std::isfinite(beta)) fail(SW4_ERR_INVALID, "the pseudocount weight must be a finite number > 0 (got %g)", beta);
+    }
+
+    void buildPssm(const char* query, int qlen, const int8_t* pssm, const int32_t* ids, int n, double beta, int8_t* out, sw4_stats* stats) {
+        checkBeta(beta);
+        if (qlen > 0 && !out) fail(SW4_ERR_INVALID, "null output array");
+        std::vector<sw4_alignment_summary> alignments((size_t)std::max(n, 1));
+        alignmentTraceback(query, qlen, pssm, ids, n, alignments.data(), stats, &beta);
+        if (qlen > 0) memcpy(out, coord->hProfileOut.p, (size_t)qlen * 21);
+    }
+
+    // P_1 = the sequence; round i scans with P_i (statistics on, no E-value cutoff), H_i = the ids of its list with
+    // E <= inclusionE; the rounds stop at maxIt, at an empty H_i or at set(H_i) == set(H_{i-1}) (converged), else
+    // P_{i+1} = the profile of H_i aligned with P_i. The last scan's list is reported with the handle's cutoff applied.
+    void searchIterative(const char* query, int qlen, int maxIt, double inclusionE, double beta, int32_t* outScores, int32_t* outIds,
+                         int32_t* outCount, int8_t* outPssm, int32_t* outIterations, int32_t* outConverged, sw4_stats* stats) {
+        if (!db) fail(SW4_ERR_INVALID, "no database set");
+        if (!statsEnabled) fail(SW4_ERR_INVALID, "the iterative search needs score statistics (sw4_set_score_statistics)");
+        if (!holdsWholeDatabase()) fail(SW4_ERR_INVALID, "the iterative search needs a handle that scans the whole database");
+        if (maxIt < 1) fail(SW4_ERR_INVALID, "max_iterations must be >= 1 (got %d)", maxIt);
+        if (std::isnan(inclusionE) || inclusionE < 0) fail(SW4_ERR_INVALID, "inclusion_evalue must be >= 0 (got %g)", inclusionE);
+        checkBeta(beta);
+        if (qlen < 0 || (qlen > 0 && (!query || !outPssm))) fail(SW4_ERR_INVALID, "invalid query or null PSSM output");
+        if (numTop > 0 && (!outScores || !outIds)) fail(SW4_ERR_INVALID, "null output arrays");
+        if (!outCount || !outIterations || !outConverged) fail(SW4_ERR_INVALID, "null output");
+        sw4_stats total{};
+        auto add = [&](const sw4_stats& s) {
+            total.num_overflows += s.num_overflows;
+            total.seconds += s.seconds;
+            total.kernel_seconds += s.kernel_seconds;
+            total.cells += s.cells;
+            total.kernel_launches += s.kernel_launches;
+        };
+        const size_t k = (size_t)std::max(numTop, 1);
+        std::vector<int32_t> scores(k), ids(k), hits, prev;
+        std::vector<int8_t> P, next((size_t)std::max(qlen, 1) * 21);
+        int32_t count = 0;
+        int iteration = 1;
+        bool converged = false;
+        const double cutoff = maxEvalue;
+        struct RestoreCutoff { double& v; double keep; ~RestoreCutoff() { v = keep; } } restore{maxEvalue, cutoff};
+        maxEvalue = INFINITY;  // the rounds take their hits before the cutoff
+        for (;; iteration++) {
+            sw4_stats s{};
+            scan(query, qlen, P.empty() ? nullptr : P.data(), scores.data(), ids.data(), &count, &s);
+            add(s);
+            const sw4_score_statistics& st = lastStats[0];
+            hits.clear();
+            if (st.status == SW4_STATS_OK)
+                for (int i = 0; i < count && evalueOf(st, scores[i]) <= inclusionE; i++) hits.push_back(ids[i]);
+            std::vector<int32_t> sorted = hits;
+            std::sort(sorted.begin(), sorted.end());
+            converged = iteration > 1 && !hits.empty() && sorted == prev;
+            if (iteration == maxIt || hits.empty() || converged) break;
+            buildPssm(query, qlen, P.empty() ? nullptr : P.data(), hits.data(), (int)hits.size(), beta, next.data(), &s);
+            add(s);
+            P.assign(next.begin(), next.begin() + (size_t)qlen * 21);
+            prev = std::move(sorted);
+        }
+        maxEvalue = cutoff;  // (restore does it on an error)
+        if (P.empty()) {  // one round: the sequence's profile, the matrix rows
+            sw4_stats s{};
+            buildPssm(query, qlen, nullptr, nullptr, 0, beta, next.data(), &s);
+            add(s);
+            P.assign(next.begin(), next.begin() + (size_t)qlen * 21);
+        }
+        const sw4_score_statistics& st = lastStats[0];
+        if (st.status == SW4_STATS_OK && std::isfinite(maxEvalue))
+            while (count > 0 && evalueOf(st, scores[count - 1]) > maxEvalue) count--;
+        for (int i = 0; i < count; i++) { outScores[i] = scores[i]; outIds[i] = ids[i]; }
+        *outCount = count;
+        if (qlen > 0) memcpy(outPssm, P.data(), (size_t)qlen * 21);
+        *outIterations = iteration;
+        *outConverged = converged ? 1 : 0;
+        if (stats) {
+            *stats = total;
+            stats->gcups = total.seconds > 0 ? total.cells / 1e9 / total.seconds : 0;
+        }
     }
 };
 
@@ -2050,7 +2234,6 @@ static inline uint64_t sw4_mix64(uint64_t z) {
     z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
     return z ^ (z >> 31);
 }
-static const int kPseudoCumulative[20] = {21, 35, 46, 60, 63, 73, 91, 109, 115, 130, 155, 170, 176, 186, 198, 214, 228, 231, 238, 256};
 
 int sw4_set_pseudo_database_lengths(sw4_handle* h, const int32_t* lengths, size_t num_sequences, uint64_t seed,
                                     const int32_t* planted_ids, const uint8_t* const* planted_codes, int32_t num_planted) {
@@ -2060,7 +2243,7 @@ int sw4_set_pseudo_database_lengths(sw4_handle* h, const int32_t* lengths, size_
         if (num_planted < 0 || (num_planted > 0 && (!planted_ids || !planted_codes))) sw4::fail(SW4_ERR_INVALID, "invalid planted list");
         if (num_sequences > (size_t)0x7ffffffe) sw4::fail(SW4_ERR_INVALID, "too many sequences");
         uint8_t table[256];
-        for (int b = 0, c = 0; b < 256; b++) { while (b >= kPseudoCumulative[c]) c++; table[b] = (uint8_t)c; }
+        for (int b = 0, c = 0; b < 256; b++) { while (b >= sw4::kPseudoCumulative[c]) c++; table[b] = (uint8_t)c; }
         auto db = std::make_unique<sw4::HostDB>();
         const size_t rank = (size_t)h->eng.shardRank, world = (size_t)h->eng.shardWorld;
         const size_t numBlocks = (num_sequences + sw4::kShardBlock - 1) / sw4::kShardBlock;
@@ -2215,6 +2398,24 @@ int sw4_alignment_traceback_pssm(sw4_handle* h, const char* query, const int8_t*
     });
     if (rc != SW4_OK) h->eng.lastCigars.clear();
     return rc;
+}
+
+int sw4_build_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length, const int32_t* ids, int32_t num_ids,
+                   double beta, int8_t* out, sw4_stats* stats) {
+    if (!h) return SW4_ERR_INVALID;
+    return guarded(h, [&] {
+        h->eng.buildPssm(query, query_length, pssm ? pssmQuery(query, pssm, query_length) : nullptr, ids, num_ids, beta, out, stats);
+    });
+}
+
+int sw4_search_iterative(sw4_handle* h, const char* query, int32_t query_length, int32_t max_iterations, double inclusion_evalue,
+                         double beta, int32_t* out_scores, int32_t* out_ids, int32_t* out_count, int8_t* out_pssm,
+                         int32_t* out_iterations, int32_t* out_converged, sw4_stats* stats) {
+    if (!h) return SW4_ERR_INVALID;
+    return guarded(h, [&] {
+        h->eng.searchIterative(query, query_length, max_iterations, inclusion_evalue, beta, out_scores, out_ids, out_count, out_pssm,
+                               out_iterations, out_converged, stats);
+    });
 }
 
 int sw4_last_cigars(const sw4_handle* h, const char** text, size_t* length) {

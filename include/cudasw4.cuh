@@ -69,6 +69,9 @@ struct ScoreStatistics {
     double evalue(int score) const { return K * (double)queryLength * (double)dbResidues * std::exp(-lambda * score); }
     double bitScore(int score) const { return (lambda * score - std::log(K)) / std::log(2.0); }
 };
+// Extension: what searchIterative returns (sw4_search_iterative in sw4b200.h): the last round's hits, the [length][21]
+// PSSM that round searched with, the number of rounds and whether they converged
+struct IterativeSearchResult { ScanResult result; std::vector<std::int8_t> pssm; int iterations; bool converged; };
 struct KernelTypeConfig {                                                                             // :88-93
     KernelType singlePassType = KernelType::Half2;
     KernelType manyPassType_small = KernelType::Half2;
@@ -209,6 +212,38 @@ public:
         check(sw4_last_score_histogram(handle, queryIndex, counts.data(), lensums.data(), SW4_SCORE_BINS));
     }
 
+    // Extension (sw4b200.h): the [length][21] profile of the query and the hits `ids`, aligned with the sequence or
+    // with a PSSM query form; pseudocountWeight is beta
+    std::vector<std::int8_t> buildPssm(const char* query, SequenceLengthT length, const std::vector<ReferenceIdT>& ids,
+                                       double pseudocountWeight = 10.0) {
+        return buildPssmImpl(query, nullptr, length, ids, pseudocountWeight);
+    }
+    std::vector<std::int8_t> buildPssm(const char* query, const std::int8_t* pssm, SequenceLengthT length,
+                                       const std::vector<ReferenceIdT>& ids, double pseudocountWeight = 10.0) {
+        return buildPssmImpl(query, pssm, length, ids, pseudocountWeight);
+    }
+    // Extension: rounds of scan -> hits with E <= inclusionEvalue -> buildPssm -> scan (needs setScoreStatistics(true))
+    IterativeSearchResult searchIterative(const char* query, SequenceLengthT length, int maxIterations = 3,
+                                          double inclusionEvalue = 0.002, double pseudocountWeight = 10.0) {
+        sw4_db_info info{};
+        check(sw4_get_db_info(handle, &info));
+        const size_t cap = (size_t)std::max<uint64_t>(1, std::min<uint64_t>(info.num_sequences, (uint64_t)std::max(numTop, 0)));
+        std::vector<int32_t> scores(cap), ids(cap);
+        IterativeSearchResult r{};
+        r.pssm.assign((size_t)std::max(length, 1) * 21, 0);
+        int32_t count = 0, iterations = 0, converged = 0;
+        sw4_stats st{};
+        check(sw4_search_iterative(handle, query, length, maxIterations, inclusionEvalue, pseudocountWeight, scores.data(), ids.data(),
+                                   &count, r.pssm.data(), &iterations, &converged, &st));
+        r.pssm.resize((size_t)std::max(length, 0) * 21);
+        r.result.scores.assign(scores.begin(), scores.begin() + count);
+        r.result.referenceIds.assign(ids.begin(), ids.begin() + count);
+        r.result.stats = BenchmarkStats{st.num_overflows, st.seconds, st.gcups};
+        r.iterations = iterations;
+        r.converged = converged != 0;
+        return r;
+    }
+
     void printDBInfo() const {                                                                      // :799-807
         sw4_db_info info{}; check(sw4_get_db_info(handle, &info));
         std::cout << info.num_sequences << " sequences, " << info.num_residues << " characters\n";
@@ -295,6 +330,14 @@ private:
             out[i].stats = BenchmarkStats{per[i].num_overflows, per[i].seconds, per[i].gcups};
         }
         if (total) *total = BenchmarkStats{tot.num_overflows, tot.seconds, tot.gcups};
+        return out;
+    }
+
+    std::vector<std::int8_t> buildPssmImpl(const char* query, const std::int8_t* pssm, SequenceLengthT length,
+                                           const std::vector<ReferenceIdT>& ids, double pseudocountWeight) {
+        std::vector<std::int8_t> out((size_t)std::max(length, 1) * 21, 0);
+        check(sw4_build_pssm(handle, query, pssm, length, ids.data(), (int32_t)ids.size(), pseudocountWeight, out.data(), nullptr));
+        out.resize((size_t)std::max(length, 0) * 21);
         return out;
     }
 

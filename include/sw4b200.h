@@ -317,6 +317,53 @@ int sw4_last_score_statistics(const sw4_handle* h, int32_t query_index, sw4_scor
  * and bins must be SW4_SCORE_BINS. A sharded search sums these over its ranks and calls sw4_fit_score_statistics. */
 int sw4_last_score_histogram(const sw4_handle* h, int32_t query_index, int64_t* counts, int64_t* lensums, int32_t bins);
 
+/* Iterative profile search (no reference counterpart): a PSSM built on the GPU from a search's own hits, and rounds of
+ * scan -> significant hits -> profile -> scan, in the manner of PSI-BLAST (its numbers are not reproduced).
+ *
+ * sw4_build_pssm writes out[query_length][21], the profile of the query and the hits `ids`. M is the handle's table, its
+ * gap scores apply, and `pssm` (NULL: the sequence query, scored with M) is the query form the hits are aligned with.
+ *   1. Alignments: for each id, the alignment sw4_alignment_traceback(_pssm) reports for that query form. Ids whose
+ *      score is 0 add no row.
+ *   2. Query-anchored MSA over the query's m positions (columns c): row 0 is the query, x_0c = q_c (its codes, converted
+ *      as every call converts them). Then one row per remaining id, in the order of `ids` (duplicates each add a row).
+ *      Row k covers columns qb..qe of its alignment: an = or X column puts the reference code paired with query position
+ *      c into x_kc; an I column (query position c in a gap) puts GAP there; D columns leave nothing; columns outside
+ *      [qb, qe] are empty. The symbols are codes 0..20 and GAP.
+ *   3. Henikoff position-based weights over the whole MSA: r_c = the number of distinct symbols in column c,
+ *      n_{c,s} = the number of rows with symbol s there, w_k = sum over the non-empty c of row k of 1 / (r_c n_{c,x_kc}).
+ *   4. Frequencies from the rows with x_kc in 0..19: W_c = sum w_k over those rows, f_ca = sum_{x_kc = a} w_k / W_c. If
+ *      W_c = 0 (q_c = 20 and no standard residue in the column), output row c is M[20][.].
+ *   5. Background p_a = the generated databases' frequencies (sw4_set_pseudo_database_lengths, 1/256 steps). lambda_u is
+ *      the root of sum_{a,b<20} p_a p_b e^(lambda M[a][b]) = 1, bisected in double on [1e-3, 2] until the interval
+ *      stops shrinking; q_ab = p_a p_b e^(lambda_u M[a][b]) / Z with Z that sum.
+ *   6. r'_c = the number of distinct codes 0..19 in column c; N = the mean of r'_c over the columns with r'_c >= 1 and
+ *      alpha = N - 1 (0 when there is no such column); g_ca = sum_b f_cb q_ab / p_b;
+ *      Q_ca = (alpha f_ca + beta g_ca) / (alpha + beta);
+ *      out[c][a] = clamp(floor(ln(Q_ca / p_a) / lambda_u + 1/2), -128, 127) for a < 20, and out[c][20] = M's `low`.
+ * With no hits alpha = 0 and every row is M[q_c][.]: a scan with that PSSM equals the sequence scan.
+ * The arguments, errors and chunking are those of sw4_alignment_traceback(_pssm), and sw4_last_cigars is left as it was.
+ * The MSA, (1 + rows) x query_length bytes, is allocated apart from the traceback scratch: when it alone exceeds
+ * max_temp_bytes the call is SW4_ERR_NOMEM. beta (the pseudocount weight, PSI-BLAST's default is 10) <= 0, NaN or
+ * infinite is SW4_ERR_INVALID. The same call always returns the same bytes, however the pairs are chunked. stats may be
+ * NULL: it covers every pass and kernel of the call.
+ *
+ * sw4_search_iterative runs the rounds on the query letters:
+ *   P_1 = the sequence;
+ *   round i: scan with P_i; H_i = the ids of the top-num_top list, taken before the handle's max_evalue cutoff, with
+ *   E <= inclusion_evalue; stop when i == max_iterations, H_i is empty or set(H_i) == set(H_{i-1}) (then converged = 1,
+ *   for i >= 2 and a non-empty H_i); else P_{i+1} = sw4_build_pssm(query, P_i, H_i in list order, beta).
+ * It reports the last scan's list exactly as that scan reports it (the max_evalue cutoff applies) in out_scores /
+ * out_ids / *out_count (num_top entries), the PSSM that scan searched with in out_pssm[query_length][21] (after one
+ * round: the profile without hits, the matrix rows), the number of rounds and the converged flag.
+ * sw4_last_score_statistics then describes the last scan. SW4_ERR_INVALID: statistics not enabled, a handle that does
+ * not scan the whole database (sw4_set_shard with world > 1, a partly held database), max_iterations < 1, a NaN or
+ * negative inclusion_evalue, a bad beta, or null outputs. stats may be NULL: it sums every scan, pass and kernel. */
+int sw4_build_pssm(sw4_handle* h, const char* query, const int8_t* pssm, int32_t query_length, const int32_t* ids, int32_t num_ids,
+                   double beta, int8_t* out, sw4_stats* stats);
+int sw4_search_iterative(sw4_handle* h, const char* query, int32_t query_length, int32_t max_iterations, double inclusion_evalue,
+                         double beta, int32_t* out_scores, int32_t* out_ids, int32_t* out_count, int8_t* out_pssm,
+                         int32_t* out_iterations, int32_t* out_converged, sw4_stats* stats);
+
 /* Debug / parity helper (the reference's CUDASW_DEBUG_CHECK_CORRECTNESS mode sets numTop to the whole database,
  * src/cudasw4.cuh:505-507): all scores of the last scan for this handle's shard, plus their global ids, in shard
  * order. capacity is in entries; returns the number written in *out_count. */
